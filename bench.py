@@ -19,6 +19,11 @@ work fixed as N grows, batch slices, no collective on the data path).
   fp64_peak : DFMA / DMMA throughput measured in this run (lqrb_fp64_peak_f64) — the denominator of the FP64-bound
           fractions, with its own clock record.
 
+  --steps K / --warmup W : every config runs W untimed steps (at least 3), then exactly K timed steps.
+  --dump-outputs DIR : after the timed steps, each config's outputs of its last step as DIR/<config key>_<name>.npy
+          (float64; a fixed seeded sample of instances, 60 MiB in all).  The inputs depend only on the arguments, so
+          two builds of the library can be compared output for output.
+
   --impl reference : times the reference algorithm's CPU restatement (oracle/, OpenMP over all host cores) on a
           bounded sample of the same workloads.  (LQR.jl itself is pure Julia and Julia is not installed in this
           image — see DESIGN.md.)
@@ -44,6 +49,7 @@ import numpy as np  # noqa: E402
 METRIC = "batched LQR KKT solves/sec (FP64)"
 UNIT = "solves/s"
 PARITY_INSTANCES = 64
+DUMP_BYTES = 60 << 20   # --dump-outputs: total size of the written sample, shared equally by the configs that run
 
 # key, BASELINE config, workload name, kind, n, m, N, per-GPU batch, roofline bound, parity tolerance
 CONFIGS = [
@@ -333,6 +339,7 @@ class Runner:
         self.hbm_peak, self.hbm_src = measured_peak_hbm()
         self.fp64_peak = None
         self.launches_timed = 0
+        self.dump_share = DUMP_BYTES  # main() divides it among the configs that run
 
     def handle(self):
         from lqr_b200 import _lib
@@ -380,18 +387,28 @@ class Runner:
         time.sleep(0.06)
         return total_ms, per, launches, self.sampler.window(t_w0, t_w1)
 
-    def steps_for(self, h, step, want):
-        """Secondary configs: as many steps as asked, but no more than ~1.5 s of kernel time."""
+    def dump_outputs(self, cfg, arrays):
+        """--dump-outputs: what the last timed step of a config computed.  `arrays` maps an output's name to a device
+        tensor with one row per instance; each is written as DIR/<config key>_<name>.npy in float64.  Outputs larger
+        than the config's share of DUMP_BYTES are represented by a fixed seeded sample of instances, the same on every
+        run with the same arguments; DIR/<config key>_instances.npy lists the instances written.  (The untimed steps
+        time_steps may append for the clock record repeat the last step on the same inputs, bit for bit.)"""
         torch = self.torch
-        step()
-        torch.cuda.synchronize()
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record(self.stream)
-        step()
-        e1.record(self.stream)
-        torch.cuda.synchronize()
-        est = max(e0.elapsed_time(e1), 1e-3)
-        return max(3, min(want, int(1500.0 / est)))
+        first = next(iter(arrays.values()))
+        batch = first.shape[0]
+        per_instance = 8 * (1 + sum(t[0].numel() for t in arrays.values()))
+        count = max(1, min(batch, self.dump_share // per_instance))
+        idx = (np.arange(batch) if count == batch
+               else np.sort(np.random.default_rng(0).choice(batch, size=count, replace=False)))
+        sel = torch.from_numpy(idx).to(first.device)
+        out = {"instances": idx}
+        out.update({name: t.index_select(0, sel).cpu().numpy() for name, t in arrays.items()})
+        os.makedirs(self.args.dump_outputs, exist_ok=True)
+        for name, a in out.items():
+            np.save(os.path.join(self.args.dump_outputs, f"{cfg['key']}_{name}.npy"), a.astype(np.float64))
+
+    def dumping(self):
+        return bool(self.args.dump_outputs) and self.rank == 0
 
     # ---------------------------------------------------------------- fp64 peak
     def measure_fp64_peak(self):
@@ -466,11 +483,16 @@ class Runner:
         def step():
             ops.riccati_solve_packed(h, n, m, N, batch, 0, knots, term, Zp, gains, info)
 
-        if not headline:
-            steps = self.steps_for(h, step, steps)
         total_ms, per, launches, clocks = self.time_steps(h, step, steps, warmup)
         assert int(info.abs().max().item()) == 0, "numerical failure flagged in info[]"
         kernel = h.last_kernel
+        if self.dumping():
+            Zd = torch.empty(batch, L.z_rows, dtype=torch.float64, device="cuda")
+            Kd = torch.empty(batch, N - 1, n, m, dtype=torch.float64, device="cuda")  # column-major m x n per knot
+            kffd = torch.empty(batch, N - 1, m, dtype=torch.float64, device="cuda")
+            ops.riccati_unpack(h, n, m, N, batch, Zp, gains, Zd, Kd, kffd)
+            self.dump_outputs(cfg, dict(Z=Zd, K=Kd, kff=kffd, info=info))
+            del Zd, Kd, kffd
         # parity of the timed output
         pc = prob_math["x0"].shape[0]
         Zd = torch.empty(pc, L.z_rows, dtype=torch.float64, device="cuda")
@@ -563,10 +585,15 @@ class Runner:
         def step():
             ops.kkt_solve_packed(h, n, m, N, batch, p, hm, False, 0, data, dzp, mp, None, info)
 
-        steps = self.steps_for(h, step, steps)
         total_ms, per, launches, clocks = self.time_steps(h, step, steps, warmup)
         assert int(info.abs().max().item()) == 0, "numerical failure flagged in info[]"
         kernel = h.last_kernel
+        if self.dumping():
+            dzd = torch.empty(batch, NN, dtype=torch.float64, device="cuda")
+            multd = torch.empty(batch, P, dtype=torch.float64, device="cuda")
+            ops.kkt_unpack(h, n, m, N, batch, p, hm, False, dzp, mp, None, dzd, multd, None)
+            self.dump_outputs(cfg, dict(dz=dzd, mult=multd, info=info))
+            del dzd, multd
         pc = prob_math["q"].shape[0]
         dz = torch.empty(pc, NN, dtype=torch.float64, device="cuda")
         mult = torch.empty(pc, P, dtype=torch.float64, device="cuda")
@@ -601,13 +628,14 @@ class Runner:
         def step():
             ops.kkt_solve_packed(h, n, m, N, 1, p, hm, False, 0, data, dzp, mp, None, info)
 
-        steps = max(steps, 50)
         total_ms, per, launches, clocks = self.time_steps(h, step, steps, warmup)
         kernel = h.last_kernel
         dz = torch.empty(1, NN, dtype=torch.float64, device="cuda")
         mult = torch.empty(1, P, dtype=torch.float64, device="cuda")
         ops.kkt_unpack(h, n, m, N, 1, p, hm, False, dzp, mp, None, dz, mult, None)
         torch.cuda.synchronize()
+        if self.dumping():
+            self.dump_outputs(cfg, dict(dz=dz, mult=mult, info=info))
         parity = parity_kkt(prob, dz.cpu().numpy(), mult.cpu().numpy()) if self.rank == 0 else None
         h.close()
         return dict(total_ms=total_ms, per=per, launches=launches, clocks=clocks, kernel=kernel, parity=parity,
@@ -631,9 +659,10 @@ class Runner:
             Z.copy_(Z0)          # restart from the initial guess (a 0.5-GB device copy inside the timed region)
             solves[0] = ops.sqp_dubins(h, batch, o, x0, xf, Z, fp, fd, it)
 
-        steps = self.steps_for(h, step, steps)
         total_ms, per, launches, clocks = self.time_steps(h, step, steps, warmup)
         kernel = h.last_kernel
+        if self.dumping():
+            self.dump_outputs(cfg, dict(Z=Z, feas_p=fp, feas_d=fd, iters=it))
         conv = float(((fp < 1e-5) & (fd < 2e-5)).double().mean().item())
         parity = None
         if self.rank == 0:
@@ -711,7 +740,12 @@ def main():
     ap.add_argument("--batch-scale", type=float, default=1.0, help="scale every batch (debug only)")
     ap.add_argument("--e2e-steps", type=int, default=3)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what each config's last timed step computed to DIR/<config key>_<name>.npy (float64, "
+                         "a fixed seeded sample of instances, 60 MiB in all; rank 0's instances)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -774,6 +808,7 @@ def main():
     if world > 1:
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
     runner = Runner(args, rank, local_rank, world)
+    runner.dump_share = DUMP_BYTES // len(cfgs)
     fp64_peak = runner.measure_fp64_peak()
 
     entries, head_res = [], None
