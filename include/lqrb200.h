@@ -251,11 +251,12 @@ int32_t lqrb_kkt_get_shur_f64(lqrb_handle_t handle, int32_t n, int32_t m, int32_
                               const double *C, const double *c, double *S, double *h, double *U,
                               int32_t *info);
 
-/* Diagnostic of the last lqrb_kkt_solve*_f64 launch on this handle that used one of the tuned large-size kernels
- * (which carry explicit block inverses): log2 of the worst pivot ratio met in any Schur block of each instance (of the
- * last chunk when the batch was processed in chunks; -1 = not tracked), and how many instances were found
- * ill-conditioned (>= 2^kkt_cond_bits, option, default 12) and solved again by the Cholesky-based general kernel, the
- * reference's own operation order (src/cholesky_solve.jl:47-67).  Either output may be NULL.                    */
+/* Diagnostic of the last lqrb_kkt_solve_f64 / lqrb_kkt_solve_packed_f64 call on this handle that used one of the
+ * tuned large-size kernels (which carry explicit block inverses): log2 of the worst pivot ratio met in any Schur block
+ * of each instance of the call, in instance order however the call was chunked (-1 = not tracked), and how many of
+ * its instances were found ill-conditioned (>= 2^kkt_cond_bits, option, default 6) and solved again by the
+ * Cholesky-based general kernel, the reference's own operation order (src/cholesky_solve.jl:47-67).  Either output
+ * may be NULL.                                                                                                   */
 int32_t lqrb_kkt_last_condition(lqrb_handle_t handle, int64_t count, int32_t *log2_pivot_ratio,
                                 int64_t *resolved);
 

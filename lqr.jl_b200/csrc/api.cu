@@ -337,11 +337,10 @@ int32_t lqrb_scatter_unpack(lqrb_context *h, const DevMap &map, const ArrayTable
     return 0;
 }
 
-// identity row maps: packed [rows] <-> instance-major [rows, batch]
-static std::vector<RowMap> identity_map(int64_t rows) {
+DevMap lqrb_identity_map(lqrb_context *h, int64_t rows) {
     std::vector<RowMap> m((size_t)rows);
     for (int64_t r = 0; r < rows; ++r) m[(size_t)r] = RowMap{0, (int32_t)r, 0.0};
-    return m;
+    return lqrb_get_map(h, "id" + std::to_string(rows), m);
 }
 
 extern "C" int32_t lqrb_unpack_rows_f64(lqrb_handle_t h, int64_t rows, int64_t batch, int32_t tile,
@@ -356,8 +355,7 @@ extern "C" int32_t lqrb_unpack_rows_f64(lqrb_handle_t h, int64_t rows, int64_t b
     ArrayTableOut t = {};
     t.ptr[0] = instance_major;
     t.stride[0] = rows;
-    return lqrb_scatter_unpack(h, lqrb_get_map(h, "id" + std::to_string(rows), identity_map(rows)), t,
-                               batch, tile, packed, h->stream);
+    return lqrb_scatter_unpack(h, lqrb_identity_map(h, rows), t, batch, tile, packed, h->stream);
 }
 
 extern "C" int32_t lqrb_pack_rows_f64(lqrb_handle_t h, int64_t rows, int64_t batch, int32_t tile,
@@ -372,6 +370,5 @@ extern "C" int32_t lqrb_pack_rows_f64(lqrb_handle_t h, int64_t rows, int64_t bat
     ArrayTable t = {};
     t.ptr[0] = instance_major;
     t.stride[0] = rows;
-    return lqrb_gather_pack(h, lqrb_get_map(h, "id" + std::to_string(rows), identity_map(rows)), t,
-                            batch, tile, packed, h->stream);
+    return lqrb_gather_pack(h, lqrb_identity_map(h, rows), t, batch, tile, packed, h->stream);
 }

@@ -87,8 +87,9 @@ struct lqrb_context {
     std::map<std::string, int64_t> options;
     std::map<std::string, struct DevMap> maps;  // cached device copies of row maps
     std::map<std::string, void *> blobs;        // cached device tables (cooperative KKT offsets)
-    std::vector<int32_t> last_cond;             // conditioning estimates of the last tuned KKT launch (log2 pivot ratio)
-    int64_t last_refined = 0;                   // instances of that launch re-solved by the Cholesky-based kernel
+    std::vector<int32_t> last_cond;             // conditioning estimates (log2 pivot ratio) per instance of the last
+                                                // KKT solve call that ran a tuned kernel
+    int64_t last_refined = 0;                   // instances of that call re-solved by the Cholesky-based kernel
     std::string kept_key;                       // shape + flags of the factorisation kept by lqrb_kkt_factor_f64
     int64_t kept_batch = 0;
 
@@ -149,6 +150,8 @@ struct ArrayTableOut {
 DevMap lqrb_get_map(lqrb_context *h, const std::string &key, std::vector<RowMap> (*build)(const int *),
                     const int *args);
 DevMap lqrb_get_map(lqrb_context *h, const std::string &key, const std::vector<RowMap> &map);
+// identity row map: packed [rows] <-> instance-major [rows, batch]
+DevMap lqrb_identity_map(lqrb_context *h, int64_t rows);
 // instance-major sources -> packed [tile][rows][tile_w]
 int32_t lqrb_gather_pack(lqrb_context *h, const DevMap &map, const ArrayTable &src, int64_t batch,
                          int tile_w, double *packed, cudaStream_t s);

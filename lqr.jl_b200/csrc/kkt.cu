@@ -4,7 +4,9 @@
 
 #include "kkt_dispatch.cuh"
 
-static bool kkt_has_tpi(const KktShape &s) {
+// ------------------------------------------------------------------ routing -------------------
+// Shapes each family has an instantiation for (kkt_dispatch.cuh) and whose stage pattern it handles.
+static bool tpi_has(const KktShape &s) {
     if (!s.uniform || s.d2x || s.free_final) return false;
 #define X(N_, M_, A_, B_, C_) \
     if (s.n == N_ && s.m == M_ && s.P1 == A_ && (s.N == 2 || s.PM == B_) && s.PN == C_) return true;
@@ -13,10 +15,7 @@ static bool kkt_has_tpi(const KktShape &s) {
     return false;
 }
 
-
-static bool kkt_has_hw(const lqrb_context *h, const KktShape &s, int flags) {
-    if (h->opt("kkt_variant", 0) == 2 || h->opt("kkt_variant", 0) == 5) return false;
-    (void)flags;
+static bool hw_has(const KktShape &s) {
     if (!s.uniform || s.d2x || s.hess == LQRB_HESS_DENSE || s.free_final) return false;
     if (s.N < 3 || s.P1 != s.n || s.PM != 0 || s.PN != s.n) return false;
 #define X(N_, M_) \
@@ -26,11 +25,7 @@ static bool kkt_has_hw(const lqrb_context *h, const KktShape &s, int flags) {
     return false;
 }
 
-
-// kkt_variant: 0 = default (half-warp kernel where it exists, else this one), 5 = force this kernel
-static bool kkt_has_wp(const lqrb_context *h, const KktShape &s) {
-    const int64_t v = h->opt("kkt_variant", 0);
-    if (v == 2 || v == 3 || v == 4) return false;
+static bool wp_has(const KktShape &s) {
     if (s.d2x) return false;
     if (s.N < 3 || s.P1 != s.n || s.PMAX > 4 || s.PN != s.n) return false;  // up to 4 stage rows on every interior knot
 #define X(N_, M_) \
@@ -40,10 +35,7 @@ static bool kkt_has_wp(const lqrb_context *h, const KktShape &s) {
     return false;
 }
 
-
-static bool kkt_has_cta(const lqrb_context *h, const KktShape &s, int flags) {
-    if (h->opt("kkt_variant", 0) == 2) return false;
-    (void)flags;
+static bool cta_has(const KktShape &s) {
     if (!s.uniform || s.d2x || s.hess == LQRB_HESS_DENSE) return false;
     if (s.N < 3 || s.P1 != s.n || s.PM > 4 || s.PN != s.n) return false;  // up to 4 stage rows on every interior knot
 #define X(N_, M_) \
@@ -53,10 +45,66 @@ static bool kkt_has_cta(const lqrb_context *h, const KktShape &s, int flags) {
     return false;
 }
 
+// The tuned size class (n2, m2) a shape without a tuned kernel of its own is embedded in (see kkt_pad_maps).
+static bool pad_class(const KktShape &s, int *n2, int *m2) {
+    // goal rows on the whole final state, or none at all (free final state: embedded with a zero goal block)
+    if (s.d2x || s.N < 3 || s.P1 != s.n || (s.PN != s.n && s.PN != 0) || s.PMAX > 4) return false;
+    auto fits = [&](int N2, int M2) {
+        if (N2 < s.n || M2 < s.m) return false;
+        const int np = N2 - s.n, mp = M2 - s.m;
+        if (np > 0 && mp < 1) return false;  // no pad control to drive the pad states
+        if (np > (int64_t)(s.N - 1) * std::min(mp, np)) return false;  // every pad state must be driven at some knot
+        return true;
+    };
+#define X(N_, M_) \
+    if (fits(N_, M_)) { *n2 = N_; *m2 = M_; return true; }
+    // the half-warp kernel (1.3x faster than the warp-per-instance one) exists at (8,4) and (12,4) for init + goal rows and a
+    // diagonal / block-diagonal Hessian: prefer those two targets when the problem has that form
+    if (s.hess != LQRB_HESS_DENSE && s.PMAX == 0 && s.PN == s.n) {
+        X(8, 4) X(12, 4)
+    }
+    // warp-per-instance class: any Hessian mode, any stage-row count per knot
+    X(8, 1) X(8, 2) X(8, 3) X(8, 4) X(12, 1) X(12, 2) X(12, 3) X(12, 4)
+    if (s.hess == LQRB_HESS_DENSE || !s.uniform) return false;
+    X(16, 8) X(16, 16) X(24, 8) X(24, 16) X(32, 8) X(32, 16) X(48, 16) X(64, 16)
+#undef X
+    return false;
+}
+
+namespace {
+enum class KktFamily { Pad, Cta, Wp, Hw, Tpi, Coop };
+struct KktRoute {
+    KktFamily family;
+    int n2 = 0, m2 = 0;  // Pad: the tuned size class
+};
+}  // namespace
+
+static bool is_tuned(KktFamily f) { return f == KktFamily::Cta || f == KktFamily::Wp || f == KktFamily::Hw; }
+
+// Which kernel family solves a shape: the only reader of the options that steer the choice.
+//   kkt_variant = 2: the cooperative kernel for every shape (the tests' reference); 5: the warp-per-instance kernel
+//   where the half-warp kernel also has the shape; any other value: the default.
+//   kkt_pad = 0: a shape without a tuned kernel of its own goes to the cooperative kernel instead of being padded.
+// The tuned kernels and the padded path read the packed data with 16-byte loads: misaligned data goes to kkt_tpi or
+// kkt_coop.
+static KktRoute kkt_route(const lqrb_context *h, const KktShape &s, bool data_aligned) {
+    const int64_t variant = h->opt("kkt_variant", 0);
+    if (variant == 2) return {KktFamily::Coop};
+    if (data_aligned) {
+        if (cta_has(s)) return {KktFamily::Cta};
+        // for (12,4) / (8,4) block-diagonal the half-warp kernel is the faster one (49.0 vs 65.5 ms on config 5a-K)
+        if (hw_has(s) && variant != 5) return {KktFamily::Hw};
+        if (wp_has(s)) return {KktFamily::Wp};
+    }
+    if (tpi_has(s)) return {KktFamily::Tpi};
+    int n2, m2;
+    if (data_aligned && h->opt("kkt_pad", 1) != 0 && pad_class(s, &n2, &m2)) return {KktFamily::Pad, n2, m2};
+    return {KktFamily::Coop};
+}
+
 int lqrb_kkt_tile(const lqrb_context *h, int n, int m, int N, const int32_t *p, int hess_mode,
                   int explicit_d2) {
-    if (h->opt("kkt_variant", 0) == 2) return 1;
-    return kkt_has_tpi(make_shape(n, m, N, p, hess_mode, explicit_d2)) ? LQRB_TILE : 1;
+    return kkt_route(h, make_shape(n, m, N, p, hess_mode, explicit_d2), true).family == KktFamily::Tpi ? LQRB_TILE : 1;
 }
 
 // ------------------------------------------------------------------ layout queries ------------
@@ -159,26 +207,40 @@ static int32_t check_kkt(lqrb_context *h, int n, int m, int N, int64_t batch, co
     return 0;
 }
 
-static size_t kkt_hw_scratch_doubles(const KktShape &s, int64_t batch);
+// ------------------------------------------------------------------ tuned families ------------
+// The conditioning record of one API call (lqrb_kkt_last_condition), over every chunk its tuned kernels ran in:
+// scratch chunks, padded chunks and host-buffer chunks append in instance order.
+namespace {
+struct KktRecord {
+    std::vector<int32_t> cond;  // log2 pivot ratio per instance
+    int64_t refined = 0;        // instances re-solved by the Cholesky-based kernel
+    bool tuned = false;         // a tuned kernel ran
+};
+}  // namespace
 
-// ------------------------------------------------------------------ solve (packed, device) ----
-// The tuned large-size kernels (kkt_hw2, kkt_cta) carry the block elimination with explicit SPD inverses (products
-// instead of the reference's sequential triangular solves); their error grows with cond(Sigma_k) where the reference's
-// U'U form (src/cholesky_solve.jl:47-67) does not.  Both kernels report, per instance, log2 of the worst pivot ratio
-// met in any Sigma_k (free: integer compares of the pivots' high words).  Instances above `kkt_cond_bits` are solved
-// again by the Cholesky-based general kernel — the reference's own operation order — which overwrites their outputs.
-// `kkt_refine` = 0 switches this off.  Costs one 4-byte-per-instance read-back and a stream synchronisation.
-int32_t kkt_resolve_ill_conditioned(lqrb_context *h, const KktShape &s, int64_t cb, int flags, const double *dc,
+// A call that ran no tuned kernel leaves the handle's record as it was; with kkt_refine = 0 only the count is reset.
+static void kkt_keep_record(lqrb_context *h, KktRecord &rec) {
+    if (!rec.tuned) return;
+    h->last_refined = rec.refined;
+    if (!rec.cond.empty()) h->last_cond.swap(rec.cond);
+}
+
+// The tuned large-size kernels (kkt_hw2, kkt_wp, kkt_cta) carry the block elimination with explicit SPD inverses
+// (products instead of the reference's sequential triangular solves); their error grows with cond(Sigma_k) where the
+// reference's U'U form (src/cholesky_solve.jl:47-67) does not.  The kernels report, per instance, log2 of the worst
+// pivot ratio met in any Sigma_k (free: integer compares of the pivots' high words).  Instances above `kkt_cond_bits`
+// are solved again by the Cholesky-based general kernel — the reference's own operation order — which overwrites their
+// outputs.  `kkt_refine` = 0 switches this off.  Costs one 4-byte-per-instance read-back and a stream synchronisation.
+static int32_t kkt_resolve_ill_conditioned(lqrb_context *h, const KktShape &s, int64_t cb, int flags, const double *dc,
                                            const int32_t *cinfo_dev, double *dz, double *mult, double *res, int32_t *info,
-                                           cudaStream_t st) {
-    h->last_refined = 0;
+                                           cudaStream_t st, KktRecord *record) {
     if (h->opt("kkt_refine", 1) == 0) return 0;
     const int slot = st == h->copy_stream[1] ? 1 : 0;
     int32_t *hc = (int32_t *)lqrb_pinned(h, 2 + slot, (size_t)cb * sizeof(int32_t));
     if (!hc) return 1000 + (int)cudaErrorMemoryAllocation;
     LQRB_CUDA(h, cudaMemcpyAsync(hc, cinfo_dev, (size_t)cb * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
     LQRB_CUDA(h, cudaStreamSynchronize(st));
-    h->last_cond.assign(hc, hc + cb);
+    record->cond.insert(record->cond.end(), hc, hc + cb);
     const int thr = (int)h->opt("kkt_cond_bits", LQRB_KKT_COND_BITS);
     std::vector<int32_t> list;
     for (int64_t i = 0; i < cb; ++i)
@@ -210,13 +272,12 @@ int32_t kkt_resolve_ill_conditioned(lqrb_context *h, const KktShape &s, int64_t 
         if (rc) return rc;
         LQRB_CUDA(h, cudaStreamSynchronize(st));  // `list` (pageable) must outlive the copy
     }
-    h->last_refined = (int64_t)list.size();
+    record->refined += (int64_t)list.size();
     return 0;
 }
 
-// scratch of the tuned kernels in doubles: the largest need of the families that have this (n, m) — which one runs
-// also depends on options (kkt_variant) and on the Hessian mode / stage rows
-static size_t kkt_hw_scratch_doubles(const KktShape &s, int64_t batch) {
+// scratch of the tuned kernels in doubles: the largest need of the families that have this (n, m)
+static size_t kkt_tuned_scratch_doubles(const KktShape &s, int64_t batch) {
     const size_t per = std::max(kkt_cta_scratch_per_instance(s), std::max(kkt_hw_scratch_per_instance(s), kkt_wp_scratch_per_instance(s)));
     return per == 0 ? 0 : (size_t)batch * per + 2;
 }
@@ -225,8 +286,8 @@ static size_t kkt_hw_scratch_doubles(const KktShape &s, int64_t batch) {
 // N=1001; 13.7 MB for n=64, N=101).  Batches are processed in chunks so that the scratch stays under
 // `scratch_budget_mb` (default 48 GB of the 180 GB) whatever the batch size.  A chunk is a whole number of
 // resident waves of the sequential kernel (its CTAs live for the whole horizon, so a partial wave is a tail).
-int64_t kkt_tuned_chunk(const lqrb_context *h, const KktShape &s) {
-    const size_t per = kkt_hw_scratch_doubles(s, 1);
+static int64_t kkt_tuned_chunk(const lqrb_context *h, const KktShape &s) {
+    const size_t per = kkt_tuned_scratch_doubles(s, 1);
     if (per == 0) return 0;
     const size_t budget = (size_t)h->opt("scratch_budget_mb", 49152) << 20;
     int64_t c = (int64_t)(budget / (per * 8));
@@ -234,6 +295,39 @@ int64_t kkt_tuned_chunk(const lqrb_context *h, const KktShape &s) {
     const int64_t wave = (int64_t)h->sm_count * (s.n + s.m <= 16 ? 24 : 2);
     c = std::max<int64_t>(wave, c / wave * wave);
     return c;
+}
+
+// scratch of a tuned family for `batch` instances (never less than the general kernel needs)
+static size_t kkt_tuned_scratch_bytes(const lqrb_context *h, const KktShape &s, const KktSizes &z, int64_t batch) {
+    return std::max((size_t)lqrb_padded_batch(batch) * z.rec_rows * 8,
+                    kkt_tuned_scratch_doubles(s, std::min(batch, kkt_tuned_chunk(h, s))) * 8 + 64);
+}
+
+// Runs a tuned family over the batch in chunks of kkt_tuned_chunk instances, each followed by the re-solve of its
+// ill-conditioned instances.  The kernel name counts the re-solved instances of the whole call so far.
+static int32_t kkt_solve_tuned(lqrb_context *h, KktFamily family, const KktShape &s, int64_t batch, int flags,
+                               const double *data, double *scratch, double *dz, double *mult, double *res, int32_t *info,
+                               cudaStream_t st, KktRecord *record) {
+    auto launch = family == KktFamily::Cta ? kkt_cta_chunk : family == KktFamily::Wp ? kkt_wp_chunk : kkt_hw_chunk;
+    const KktSizes z = kkt_sizes(s);
+    const int soc = (flags & LQRB_FLAG_SOC) ? 1 : 0;
+    const int64_t chunk = std::min(batch, kkt_tuned_chunk(h, s));
+    std::string name;
+    for (int64_t first = 0; first < batch; first += chunk) {
+        const int64_t cb = std::min(chunk, batch - first);
+        const double *dc = data + first * z.data_rows;
+        double *dzc = dz + first * z.NN, *mc = mult + first * z.P, *rc_ = res ? res + first * z.NN : nullptr;
+        int32_t *ic = info ? info + first : nullptr, *cinfo = nullptr;
+        int32_t rc = launch(h, s, cb, soc, dc, scratch, dzc, mc, rc_, ic, &cinfo, st);
+        if (rc) return rc;
+        name = h->kernel_name;  // (the re-solve names its own kernel)
+        rc = kkt_resolve_ill_conditioned(h, s, cb, soc ? LQRB_FLAG_SOC : 0, dc, cinfo, dzc, mc, rc_, ic, st, record);
+        if (rc) return rc;
+    }
+    record->tuned = true;
+    h->kernel_name = name;
+    if (record->refined) h->kernel_name += "+kkt_coop[" + std::to_string(record->refined) + " ill-conditioned]";
+    return 0;
 }
 
 // ------------------------------------------------------------------ padding into a tuned size class ----
@@ -245,33 +339,6 @@ int64_t kkt_tuned_chunk(const lqrb_context *h, const KktShape &s) {
 // variables and their multipliers are exactly zero at the optimum and the original variables see the same KKT system.
 // The packed data (layout of s) is expanded on the device into the layout of the padded shape, the tuned kernel runs,
 // and dz, mult, res are compacted back: two extra passes over the data, a few percent of what the padding saves.
-static bool kkt_pad_target(const lqrb_context *h, const KktShape &s, int *n2, int *m2) {
-    if (h->opt("kkt_pad", 1) == 0 || h->opt("kkt_variant", 0) == 2) return false;
-    // goal rows on the whole final state, or none at all (free final state: embedded with a zero goal block)
-    if (s.d2x || s.N < 3 || s.P1 != s.n || (s.PN != s.n && s.PN != 0) || s.PMAX > 4) return false;
-    if (kkt_has_tpi(s) || kkt_has_hw(h, s, 0) || kkt_has_wp(h, s) || kkt_has_cta(h, s, 0)) return false;
-    auto fits = [&](int N2, int M2) {
-        if (N2 < s.n || M2 < s.m) return false;
-        const int np = N2 - s.n, mp = M2 - s.m;
-        if (np > 0 && mp < 1) return false;  // no pad control to drive the pad states
-        if (np > (int64_t)(s.N - 1) * std::min(mp, np)) return false;  // every pad state must be driven at some knot
-        return true;
-    };
-#define X(N_, M_) \
-    if (fits(N_, M_)) { *n2 = N_; *m2 = M_; return true; }
-    // the half-warp kernel (1.3x faster than the warp-per-instance one) exists at (8,4) and (12,4) for init + goal rows and a
-    // diagonal / block-diagonal Hessian: prefer those two targets when the problem has that form
-    if (s.hess != LQRB_HESS_DENSE && s.PMAX == 0 && s.PN == s.n) {
-        X(8, 4) X(12, 4)
-    }
-    // warp-per-instance class: any Hessian mode, any stage-row count per knot
-    X(8, 1) X(8, 2) X(8, 3) X(8, 4) X(12, 1) X(12, 2) X(12, 3) X(12, 4)
-    if (s.hess == LQRB_HESS_DENSE || !s.uniform) return false;
-    X(16, 8) X(16, 16) X(24, 8) X(24, 16) X(32, 8) X(32, 16) X(48, 16) X(64, 16)
-#undef X
-    return false;
-}
-
 namespace {
 struct PadMaps {
     std::vector<RowMap> data, dz, mult;  // rows of the padded layout -> offset in the original one (or fill / skip)
@@ -368,10 +435,6 @@ static PadMaps kkt_pad_maps(const KktShape &s, int n2, int m2) {
     return M;
 }
 
-static size_t kkt_scratch_bytes(const lqrb_context *h, const KktShape &s, const KktSizes &z, int64_t batch);
-static int32_t kkt_solve_on(lqrb_context *h, const KktShape &s, int64_t batch, int flags, const double *data, double *scratch,
-                            double *dz, double *mult, double *res, int32_t *info, cudaStream_t st);
-
 struct PadPlan {
     std::vector<int32_t> p2;
     KktShape s2;
@@ -391,14 +454,16 @@ static void kkt_pad_plan(const lqrb_context *h, const KktShape &s, int n2, int m
     const size_t ldb = (size_t)lqrb_padded_batch(P->chunk);
     P->data_b = (ldb * P->z2.data_rows * 8 + 255) / 256 * 256;
     P->out_b = (ldb * (2 * P->z2.NN + P->z2.P) * 8 + 255) / 256 * 256;
-    P->scr_b = (kkt_scratch_bytes(h, P->s2, P->z2, P->chunk) + 255) / 256 * 256;
+    P->scr_b = (kkt_tuned_scratch_bytes(h, P->s2, P->z2, P->chunk) + 255) / 256 * 256;
 }
 
 static int32_t kkt_solve_padded(lqrb_context *h, const KktShape &s, int n2, int m2, int64_t batch, int flags,
                                 const double *data, double *scratch, double *dz, double *mult, double *res, int32_t *info,
-                                cudaStream_t st) {
+                                cudaStream_t st, KktRecord *record) {
     PadPlan P;
     kkt_pad_plan(h, s, n2, m2, batch, &P);
+    const KktFamily family = kkt_route(h, P.s2, true).family;
+    if (!is_tuned(family)) return lqrb_fail(h, 1, "padded KKT shape has no tuned kernel");
     const KktSizes z = kkt_sizes(s);
     char key[64];
     snprintf(key, sizeof key, "->%d,%d", n2, m2);
@@ -421,9 +486,6 @@ static int32_t kkt_solve_padded(lqrb_context *h, const KktShape &s, int n2, int 
     const size_t ldb = (size_t)lqrb_padded_batch(P.chunk);
     double *mult2 = dz2 + ldb * P.z2.NN, *res2 = mult2 + ldb * P.z2.P;
     double *scr2 = reinterpret_cast<double *>(base + P.data_b + P.out_b);
-    std::string name;
-    int64_t refined = 0;
-    std::vector<int32_t> cond;
     for (int64_t first = 0; first < batch; first += P.chunk) {
         const int64_t cb = std::min(P.chunk, batch - first);
         ArrayTable src = {};
@@ -431,11 +493,9 @@ static int32_t kkt_solve_padded(lqrb_context *h, const KktShape &s, int n2, int 
         src.stride[0] = z.data_rows;
         int32_t rc = lqrb_gather_pack(h, md, src, cb, 1, data2, st);
         if (rc) return rc;
-        rc = kkt_solve_on(h, P.s2, cb, flags, data2, scr2, dz2, mult2, res ? res2 : nullptr, info ? info + first : nullptr, st);
+        rc = kkt_solve_tuned(h, family, P.s2, cb, flags, data2, scr2, dz2, mult2, res ? res2 : nullptr,
+                             info ? info + first : nullptr, st, record);
         if (rc) return rc;
-        name = h->kernel_name;
-        refined += h->last_refined;
-        cond.insert(cond.end(), h->last_cond.begin(), h->last_cond.end());
         ArrayTableOut o = {};
         o.ptr[0] = dz + first * z.NN;
         o.stride[0] = z.NN;
@@ -453,53 +513,39 @@ static int32_t kkt_solve_padded(lqrb_context *h, const KktShape &s, int n2, int 
     }
     char nm[64];
     snprintf(nm, sizeof nm, " <- (%d,%d)%s padded", s.n, s.m, s.PN == 0 ? " free final state" : "");
-    h->kernel_name = name + nm;
-    h->last_refined = refined;
-    h->last_cond = cond;
+    h->kernel_name += nm;
     return 0;
 }
 
+// scratch of one call, sized for 16-byte aligned data (misaligned data runs the general kernel, which needs less)
 static size_t kkt_scratch_bytes(const lqrb_context *h, const KktShape &s, const KktSizes &z, int64_t batch) {
-    {
-        int n2, m2;
-        if (kkt_pad_target(h, s, &n2, &m2)) {
-            PadPlan P;
-            kkt_pad_plan(h, s, n2, m2, batch, &P);
-            // (never less than the general kernel needs: it is what runs if the padded path is not taken after all)
-            return std::max(P.data_b + P.out_b + P.scr_b, (size_t)lqrb_padded_batch(batch) * z.rec_rows * 8);
-        }
+    const KktRoute r = kkt_route(h, s, true);
+    const size_t general = (size_t)lqrb_padded_batch(batch) * z.rec_rows * 8;
+    if (r.family == KktFamily::Pad) {
+        PadPlan P;
+        kkt_pad_plan(h, s, r.n2, r.m2, batch, &P);
+        return std::max(P.data_b + P.out_b + P.scr_b, general);
     }
-    size_t bytes = (size_t)lqrb_padded_batch(batch) * z.rec_rows * 8;
-    // the tuned kernels' records only when one of them will actually run for this shape (a dense Hessian, an
-    // irregular stage pattern, explicit D2 or kkt_variant = 2 route the same (n, m) to the cooperative kernel)
-    if (!kkt_has_hw(h, s, 0) && !kkt_has_cta(h, s, 0) && !kkt_has_wp(h, s)) return bytes;
-    const int64_t chunk = kkt_tuned_chunk(h, s);
-    if (chunk > 0) bytes = std::max(bytes, kkt_hw_scratch_doubles(s, std::min(batch, chunk)) * 8 + 64);
-    return bytes;
+    return is_tuned(r.family) ? kkt_tuned_scratch_bytes(h, s, z, batch) : general;
 }
 
 static int32_t kkt_solve_on(lqrb_context *h, const KktShape &s, int64_t batch, int flags,
                             const double *data, double *scratch, double *dz, double *mult, double *res,
-                            int32_t *info, cudaStream_t st) {
+                            int32_t *info, cudaStream_t st, KktRecord *record) {
     if (batch == 0) return 0;
-    {
-        int n2, m2;
-        if (((uintptr_t)data & 15) == 0 && ((uintptr_t)scratch & 255) == 0 && kkt_pad_target(h, s, &n2, &m2))
-            return kkt_solve_padded(h, s, n2, m2, batch, flags, data, scratch, dz, mult, res, info, st);
+    const KktRoute r = kkt_route(h, s, ((uintptr_t)data & 15) == 0);
+    switch (r.family) {
+    case KktFamily::Pad:
+        return kkt_solve_padded(h, s, r.n2, r.m2, batch, flags, data, scratch, dz, mult, res, info, st, record);
+    case KktFamily::Cta:
+    case KktFamily::Wp:
+    case KktFamily::Hw:
+        return kkt_solve_tuned(h, r.family, s, batch, flags, data, scratch, dz, mult, res, info, st, record);
+    case KktFamily::Tpi:
+        return kkt_launch_tpi(h, s, batch, flags, data, scratch, dz, mult, res, info, st);
+    case KktFamily::Coop:
+        break;
     }
-    int32_t rc = LQRB_NO_KERNEL;
-    if (kkt_has_cta(h, s, flags) && ((uintptr_t)data & 15) == 0 && ((uintptr_t)scratch & 15) == 0)
-        rc = kkt_launch_cta(h, s, batch, flags, data, scratch, dz, mult, res, info, st);
-    // The warp-per-instance tensor-core kernel takes the shapes the half-warp kernel does not have (m < 4, dense
-    // Hessian, stage rows); for (12,4) / (8,4) block-diagonal it is the slower one (65.5 vs 49.0 ms on config 5a-K) and
-    // runs only when forced (kkt_variant = 5; 3 = the column layout of the half-warp kernel).
-    else if (kkt_has_wp(h, s) && ((uintptr_t)data & 15) == 0 && (h->opt("kkt_variant", 0) == 5 || !kkt_has_hw(h, s, flags)))
-        rc = kkt_launch_wp(h, s, batch, flags, data, scratch, dz, mult, res, info, st);
-    else if (kkt_has_hw(h, s, flags) && ((uintptr_t)data & 15) == 0)
-        rc = kkt_launch_hw(h, s, batch, flags, data, scratch, dz, mult, res, info, st);
-    else if (lqrb_kkt_tile(h, s.n, s.m, s.N, s.p, s.hess, s.d2x) == LQRB_TILE)
-        rc = kkt_launch_tpi(h, s, batch, flags, data, scratch, dz, mult, res, info, st);
-    if (rc != LQRB_NO_KERNEL) return rc;
     return launch_kkt_coop(h, s.n, s.m, s.N, s.p, s.hess, s.d2x, flags, batch, data, scratch, dz, mult, res,
                            info, st);
 }
@@ -518,7 +564,11 @@ extern "C" int32_t lqrb_kkt_solve_packed_f64(lqrb_handle_t h, int32_t n, int32_t
     const KktSizes z = kkt_sizes(s);
     double *scratch = (double *)lqrb_scratch(h, SCR_FACT, kkt_scratch_bytes(h, s, z, batch));
     if (!scratch) return 1000 + (int)cudaErrorMemoryAllocation;
-    return kkt_solve_on(h, s, batch, flags, data, scratch, dz, mult, res, info, h->stream);
+    KktRecord record;
+    rc = kkt_solve_on(h, s, batch, flags, data, scratch, dz, mult, res, info, h->stream, &record);
+    if (rc) return rc;
+    kkt_keep_record(h, record);
+    return 0;
 }
 
 // ------------------------------------------------------------------ pack / unpack -------------
@@ -633,8 +683,10 @@ extern "C" int32_t lqrb_kkt_solve_f64(lqrb_handle_t h, int32_t n, int32_t m, int
         if (!data || !dzp || !mp || !scr || (res && !rp)) return 1000 + (int)cudaErrorMemoryAllocation;
         rc = kkt_pack_on(h, s, z, batch, src, data, h->stream);
         if (rc) return rc;
-        rc = kkt_solve_on(h, s, batch, flags, data, scr, dzp, mp, rp, info, h->stream);
+        KktRecord record;
+        rc = kkt_solve_on(h, s, batch, flags, data, scr, dzp, mp, rp, info, h->stream, &record);
         if (rc) return rc;
+        kkt_keep_record(h, record);
         return kkt_unpack_on(h, s, z, batch, dzp, mp, rp, dz, mult, res, h->stream);
     }
 
@@ -659,6 +711,7 @@ extern "C" int32_t lqrb_kkt_solve_f64(lqrb_handle_t h, int32_t n, int32_t m, int
 
     LQRB_CUDA(h, cudaEventRecord(h->ev[0], h->stream));
     for (int i = 0; i < 2; ++i) LQRB_CUDA(h, cudaStreamWaitEvent(h->copy_stream[i], h->ev[0], 0));
+    KktRecord record;
     int which = 0;
     for (int64_t first = 0; first < batch; first += chunk, which ^= 1) {
         const int64_t cb = std::min(chunk, batch - first);
@@ -681,7 +734,7 @@ extern "C" int32_t lqrb_kkt_solve_f64(lqrb_handle_t h, int32_t n, int32_t m, int
         int32_t *di = dinfo + which * chunk;
         rc = kkt_pack_on(h, s, z, cb, dsrc, data, st);
         if (rc) return rc;
-        rc = kkt_solve_on(h, s, cb, flags, data, scr, dzp, mp, res ? rp : nullptr, di, st);
+        rc = kkt_solve_on(h, s, cb, flags, data, scr, dzp, mp, res ? rp : nullptr, di, st, &record);
         if (rc) return rc;
         double *so = (double *)(stage_out + which * out_bytes);
         double *odz = so, *om = odz + cb * z.NN, *ores = om + cb * z.P;
@@ -695,6 +748,7 @@ extern "C" int32_t lqrb_kkt_solve_f64(lqrb_handle_t h, int32_t n, int32_t m, int
             LQRB_CUDA(h, cudaMemcpyAsync(info + first, di, (size_t)cb * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
     }
     for (int i = 0; i < 2; ++i) LQRB_CUDA(h, cudaStreamSynchronize(h->copy_stream[i]));
+    kkt_keep_record(h, record);
     return 0;
 }
 

@@ -3,8 +3,8 @@
 #include "kkt_cta_kernels.cuh"
 
 template <int n, int m, int HESS>
-static int32_t launch_kkt_cta(lqrb_context *h, const KktShape &s, int64_t batch, int soc, const double *data,
-                              double *scratch, double *dz, double *mult, double *res, int32_t *info,
+static int32_t launch_kkt_cta(lqrb_context *h, const KktShape &s, int64_t cb, int soc, const double *data,
+                              double *scratch, double *dz, double *mult, double *res, int32_t *info, int32_t **cinfo_out,
                               cudaStream_t st) {
     using L = kcta::Lay<n, m, HESS>;
     const int N = s.N, ps = s.PM;
@@ -15,49 +15,34 @@ static int32_t launch_kkt_cta(lqrb_context *h, const KktShape &s, int64_t batch,
     auto mk = ps ? kcta::kkt_cta_kernel<n, m, HESS, true> : kcta::kkt_cta_kernel<n, m, HESS, false>;
     LQRB_CUDA(h, cudaFuncSetAttribute(pk, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)psm));
     LQRB_CUDA(h, cudaFuncSetAttribute(mk, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msm));
-    const int64_t chunk = std::min(batch, kkt_tuned_chunk(h, s));
-    const int64_t drows = L::data_rows(N, ps), zrows = L::z_rows(N), mrows = L::mult_rows(N, ps);
-    int64_t refined = 0;
-    for (int64_t first = 0; first < batch; first += chunk) {
-        const int64_t cb = std::min(chunk, batch - first);
-        // scratch (reused by every chunk): [records: cb x N x REC] [pre-pass slots: cb x prep_rows] [hinfo: cb] [cinfo: cb]
-        double *recs = scratch;
-        double *prep = recs + (size_t)cb * N * L::rec(ps);
-        int32_t *hinfo = reinterpret_cast<int32_t *>(prep + (size_t)cb * L::prep_rows(N, ps));
-        int32_t *cinfo = hinfo + cb;  // conditioning estimates (the "+ 1" double per instance holds both)
-        const double *dc = data + first * drows;
-        LQRB_CUDA(h, cudaMemsetAsync(hinfo, 0x7f, (size_t)cb * sizeof(int32_t), st));
-        LQRB_CUDA(h, cudaMemsetAsync(cinfo, 0, (size_t)cb * sizeof(int32_t), st));
-        kcta::kkt_cta_ri_kernel<n, m, HESS><<<(unsigned)((cb * (N - 1) + 7) / 8), 128, 0, st>>>(dc, prep, hinfo, N, cb, soc, ps);
-        LQRB_LAUNCH_CHECK(h, "kkt_cta_ri_kernel");
-        pk<<<(unsigned)(cb * N), L::THREADS, psm, st>>>(dc, prep, hinfo, cinfo, N, cb, soc, ps);
-        LQRB_LAUNCH_CHECK(h, "kkt_cta_prep_kernel");
-        mk<<<(unsigned)cb, L::THREADS, msm, st>>>(dc, prep, hinfo, recs, dz + first * zrows, mult + first * mrows,
-                                                  res ? res + first * zrows : nullptr,
-                                                  info ? info + first : nullptr, cinfo, N, cb, soc, ps, s.free_final ? 1 : 0);
-        LQRB_LAUNCH_CHECK(h, "kkt_cta_kernel");
-        int32_t rc = kkt_resolve_ill_conditioned(h, s, cb, soc ? LQRB_FLAG_SOC : 0, dc, cinfo, dz + first * zrows,
-                                                 mult + first * mrows, res ? res + first * zrows : nullptr,
-                                                 info ? info + first : nullptr, st);
-        if (rc) return rc;
-        refined += h->last_refined;
-    }
+    // scratch: [records: cb x N x REC] [pre-pass slots: cb x prep_rows] [hinfo: cb] [cinfo: cb]
+    double *recs = scratch;
+    double *prep = recs + (size_t)cb * N * L::rec(ps);
+    int32_t *hinfo = reinterpret_cast<int32_t *>(prep + (size_t)cb * L::prep_rows(N, ps));
+    int32_t *cinfo = hinfo + cb;  // conditioning estimates (the "+ 1" double per instance holds both)
+    LQRB_CUDA(h, cudaMemsetAsync(hinfo, 0x7f, (size_t)cb * sizeof(int32_t), st));
+    LQRB_CUDA(h, cudaMemsetAsync(cinfo, 0, (size_t)cb * sizeof(int32_t), st));
+    kcta::kkt_cta_ri_kernel<n, m, HESS><<<(unsigned)((cb * (N - 1) + 7) / 8), 128, 0, st>>>(data, prep, hinfo, N, cb, soc, ps);
+    LQRB_LAUNCH_CHECK(h, "kkt_cta_ri_kernel");
+    pk<<<(unsigned)(cb * N), L::THREADS, psm, st>>>(data, prep, hinfo, cinfo, N, cb, soc, ps);
+    LQRB_LAUNCH_CHECK(h, "kkt_cta_prep_kernel");
+    mk<<<(unsigned)cb, L::THREADS, msm, st>>>(data, prep, hinfo, recs, dz, mult, res, info, cinfo, N, cb, soc, ps,
+                                              s.free_final ? 1 : 0);
+    LQRB_LAUNCH_CHECK(h, "kkt_cta_kernel");
+    *cinfo_out = cinfo;
     char nm[128];
     snprintf(nm, sizeof nm, "kkt_cta_dmma<%d,%d,p=%d/%d/%d,hess=%d%s>", n, m, n, ps, n, HESS, soc ? ",soc" : "");
     h->kernel_name = nm;
-    if (refined) h->kernel_name += "+kkt_coop[" + std::to_string(refined) + " ill-conditioned]";
-    h->last_refined = refined;
     return 0;
 }
 
-int32_t kkt_launch_cta(lqrb_context *h, const KktShape &s, int64_t batch, int flags, const double *data, double *scratch,
-                       double *dz, double *mult, double *res, int32_t *info, cudaStream_t st) {
-    const int soc = (flags & LQRB_FLAG_SOC) ? 1 : 0;
-#define X(N_, M_)                                                                                                     \
-    if (s.n == N_ && s.m == M_)                                                                                       \
-        return s.hess == LQRB_HESS_DIAG                                                                               \
-                   ? launch_kkt_cta<N_, M_, LQRB_HESS_DIAG>(h, s, batch, soc, data, scratch, dz, mult, res, info, st) \
-                   : launch_kkt_cta<N_, M_, LQRB_HESS_BLOCKDIAG>(h, s, batch, soc, data, scratch, dz, mult, res, info, st);
+int32_t kkt_cta_chunk(lqrb_context *h, const KktShape &s, int64_t cb, int soc, const double *data, double *scratch,
+                      double *dz, double *mult, double *res, int32_t *info, int32_t **cinfo, cudaStream_t st) {
+#define X(N_, M_)                                                                                                    \
+    if (s.n == N_ && s.m == M_)                                                                                      \
+        return s.hess == LQRB_HESS_DIAG                                                                              \
+                   ? launch_kkt_cta<N_, M_, LQRB_HESS_DIAG>(h, s, cb, soc, data, scratch, dz, mult, res, info, cinfo, st) \
+                   : launch_kkt_cta<N_, M_, LQRB_HESS_BLOCKDIAG>(h, s, cb, soc, data, scratch, dz, mult, res, info, cinfo, st);
     KKT_CTA_SIZES(X)
 #undef X
     return LQRB_NO_KERNEL;

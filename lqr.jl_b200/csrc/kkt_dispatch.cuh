@@ -87,23 +87,20 @@ inline KktSizes kkt_sizes(const KktShape &s) {
 }
 
 
-// kkt.cu
-int64_t kkt_tuned_chunk(const lqrb_context *h, const KktShape &s);
-int32_t kkt_resolve_ill_conditioned(lqrb_context *h, const KktShape &s, int64_t cb, int flags, const double *dc,
-                                    const int32_t *cinfo_dev, double *dz, double *mult, double *res, int32_t *info,
-                                    cudaStream_t st);
-
-// Family launchers: the caller has checked the size list and the stage pattern (kkt_has_*); LQRB_NO_KERNEL if no
-// instantiation matches.  *_scratch_per_instance: doubles of scratch one instance needs (0: not in the size list).
+// Family launchers.  kkt_launch_tpi runs a whole batch.  The tuned families (kkt_*_chunk) launch one chunk of `cb`
+// instances (every pointer at the chunk's first instance, scratch reused by every chunk), name the kernel in
+// h->kernel_name and return in *cinfo the chunk's conditioning estimates (device memory inside scratch); the chunk loop
+// and the re-solve of ill-conditioned instances are in kkt.cu.  LQRB_NO_KERNEL if no instantiation matches.
+// *_scratch_per_instance: doubles of scratch one instance needs (0: not in the size list).
 #define LQRB_NO_KERNEL (-12345)
 int32_t kkt_launch_tpi(lqrb_context *h, const KktShape &s, int64_t batch, int flags, const double *data, double *scratch,
                        double *dz, double *mult, double *res, int32_t *info, cudaStream_t st);
-int32_t kkt_launch_hw(lqrb_context *h, const KktShape &s, int64_t batch, int flags, const double *data, double *scratch,
-                      double *dz, double *mult, double *res, int32_t *info, cudaStream_t st);
-int32_t kkt_launch_wp(lqrb_context *h, const KktShape &s, int64_t batch, int flags, const double *data, double *scratch,
-                      double *dz, double *mult, double *res, int32_t *info, cudaStream_t st);
-int32_t kkt_launch_cta(lqrb_context *h, const KktShape &s, int64_t batch, int flags, const double *data, double *scratch,
-                       double *dz, double *mult, double *res, int32_t *info, cudaStream_t st);
+int32_t kkt_hw_chunk(lqrb_context *h, const KktShape &s, int64_t cb, int soc, const double *data, double *scratch,
+                     double *dz, double *mult, double *res, int32_t *info, int32_t **cinfo, cudaStream_t st);
+int32_t kkt_wp_chunk(lqrb_context *h, const KktShape &s, int64_t cb, int soc, const double *data, double *scratch,
+                     double *dz, double *mult, double *res, int32_t *info, int32_t **cinfo, cudaStream_t st);
+int32_t kkt_cta_chunk(lqrb_context *h, const KktShape &s, int64_t cb, int soc, const double *data, double *scratch,
+                      double *dz, double *mult, double *res, int32_t *info, int32_t **cinfo, cudaStream_t st);
 size_t kkt_hw_scratch_per_instance(const KktShape &s);
 size_t kkt_wp_scratch_per_instance(const KktShape &s);
 size_t kkt_cta_scratch_per_instance(const KktShape &s);

@@ -1,62 +1,46 @@
-// kkt_hw.cu — launcher of the half-warp-per-instance KKT kernels (kkt_hw_kernels.cuh); size list in kkt_dispatch.cuh.
+// kkt_hw.cu — launcher of the half-warp-per-instance KKT kernel (kkt_hw_kernels.cuh); size list in kkt_dispatch.cuh.
 #include "kkt_dispatch.cuh"
 #include "kkt_hw_kernels.cuh"
 
 template <int n, int m, int HESS>
-static int32_t launch_kkt_hw(lqrb_context *h, const KktShape &s, int64_t batch, int soc, const double *data,
-                             double *scratch, double *dz, double *mult, double *res, int32_t *info,
+static int32_t launch_kkt_hw(lqrb_context *h, const KktShape &s, int64_t cb, int soc, const double *data,
+                             double *scratch, double *dz, double *mult, double *res, int32_t *info, int32_t **cinfo_out,
                              cudaStream_t st) {
     using L = khw::Lay<n, m, HESS>;
     const int N = s.N;
-    // default: the block-layout kernel (4 x 4 lane grid per instance); kkt_variant = 3 keeps the column-per-lane one.
     // Three 4-warp CTAs per SM at 168 registers: eight 2-warp CTAs at 128 registers (16 warps, a few spills) were
     // 3.5 % slower in an A/B on one box (48.95 vs 47.2 ms) — the kernel is not latency-bound.
     constexpr int WARPS = 4, MINB = 3;
-    const bool blocks = h->opt("kkt_variant", 0) != 3;
-    const size_t smem = (size_t)WARPS * (2 * (blocks ? L::INST2 : L::INST) + 4) * sizeof(double);
-    auto kern = blocks ? khw::kkt_hw2_kernel<n, m, HESS, WARPS, MINB> : khw::kkt_hw_kernel<n, m, HESS, WARPS, MINB>;
+    const size_t smem = (size_t)WARPS * (2 * L::INST2 + 4) * sizeof(double);
+    auto kern = khw::kkt_hw2_kernel<n, m, HESS, WARPS, MINB>;
     LQRB_CUDA(h, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    const int64_t chunk = std::min(batch, kkt_tuned_chunk(h, s));
-    int64_t refined = 0;
-    for (int64_t first = 0; first < batch; first += chunk) {
-        const int64_t cb = std::min(chunk, batch - first);
-        // scratch (reused by every chunk): [records: cb x N x REC] [Hi: cb x N x HI] [hinfo: cb] [cinfo: cb]
-        double *recs = scratch;
-        double *hinv = recs + (size_t)cb * N * L::REC;
-        int32_t *hinfo = reinterpret_cast<int32_t *>(hinv + (size_t)cb * N * L::HI);
-        int32_t *cinfo = hinfo + cb;  // conditioning estimates (the "+ 1" double per instance holds both)
-        const double *dc = data + first * L::data_rows(N);
-        LQRB_CUDA(h, cudaMemsetAsync(hinfo, 0x7f, (size_t)cb * sizeof(int32_t), st));
-        const int64_t total = cb * N;
-        khw::kkt_hinv_kernel<n, m, HESS><<<(unsigned)((total + 127) / 128), 128, 0, st>>>(dc, hinv, hinfo, N, cb, soc);
-        LQRB_LAUNCH_CHECK(h, "kkt_hinv_kernel");
-        const int64_t pairs = (cb + 1) / 2;
-        kern<<<(unsigned)((pairs + WARPS - 1) / WARPS), WARPS * 32, smem, st>>>(
-            dc, hinv, hinfo, recs, dz + first * L::z_rows(N), mult + first * L::mult_rows(N),
-            res ? res + first * L::z_rows(N) : nullptr, info ? info + first : nullptr, cinfo, N, cb, soc);
-        LQRB_LAUNCH_CHECK(h, "kkt_hw_kernel");
-        int32_t rc = kkt_resolve_ill_conditioned(h, s, cb, soc ? LQRB_FLAG_SOC : 0, dc, cinfo, dz + first * L::z_rows(N),
-                                                 mult + first * L::mult_rows(N), res ? res + first * L::z_rows(N) : nullptr,
-                                                 info ? info + first : nullptr, st);
-        if (rc) return rc;
-        refined += h->last_refined;
-    }
+    // scratch: [records: cb x N x REC] [Hi: cb x N x HI] [hinfo: cb] [cinfo: cb]
+    double *recs = scratch;
+    double *hinv = recs + (size_t)cb * N * L::REC;
+    int32_t *hinfo = reinterpret_cast<int32_t *>(hinv + (size_t)cb * N * L::HI);
+    int32_t *cinfo = hinfo + cb;  // conditioning estimates (the "+ 1" double per instance holds both)
+    LQRB_CUDA(h, cudaMemsetAsync(hinfo, 0x7f, (size_t)cb * sizeof(int32_t), st));
+    const int64_t total = cb * N;
+    khw::kkt_hinv_kernel<n, m, HESS><<<(unsigned)((total + 127) / 128), 128, 0, st>>>(data, hinv, hinfo, N, cb, soc);
+    LQRB_LAUNCH_CHECK(h, "kkt_hinv_kernel");
+    const int64_t pairs = (cb + 1) / 2;
+    kern<<<(unsigned)((pairs + WARPS - 1) / WARPS), WARPS * 32, smem, st>>>(data, hinv, hinfo, recs, dz, mult, res, info,
+                                                                            cinfo, N, cb, soc);
+    LQRB_LAUNCH_CHECK(h, "kkt_hw_kernel");
+    *cinfo_out = cinfo;
     char nm[128];
-    snprintf(nm, sizeof nm, "kkt_hw<%d,%d,p=%d/0/%d,hess=%d%s%s>", n, m, n, n, HESS, soc ? ",soc" : "", blocks ? "" : ",cols");
+    snprintf(nm, sizeof nm, "kkt_hw<%d,%d,p=%d/0/%d,hess=%d%s>", n, m, n, n, HESS, soc ? ",soc" : "");
     h->kernel_name = nm;
-    if (refined) h->kernel_name += "+kkt_coop[" + std::to_string(refined) + " ill-conditioned]";
-    h->last_refined = refined;
     return 0;
 }
 
-int32_t kkt_launch_hw(lqrb_context *h, const KktShape &s, int64_t batch, int flags, const double *data, double *scratch,
-                      double *dz, double *mult, double *res, int32_t *info, cudaStream_t st) {
-    const int soc = (flags & LQRB_FLAG_SOC) ? 1 : 0;
-#define X(N_, M_)                                                                                                    \
-    if (s.n == N_ && s.m == M_)                                                                                      \
-        return s.hess == LQRB_HESS_DIAG                                                                              \
-                   ? launch_kkt_hw<N_, M_, LQRB_HESS_DIAG>(h, s, batch, soc, data, scratch, dz, mult, res, info, st) \
-                   : launch_kkt_hw<N_, M_, LQRB_HESS_BLOCKDIAG>(h, s, batch, soc, data, scratch, dz, mult, res, info, st);
+int32_t kkt_hw_chunk(lqrb_context *h, const KktShape &s, int64_t cb, int soc, const double *data, double *scratch,
+                     double *dz, double *mult, double *res, int32_t *info, int32_t **cinfo, cudaStream_t st) {
+#define X(N_, M_)                                                                                                   \
+    if (s.n == N_ && s.m == M_)                                                                                     \
+        return s.hess == LQRB_HESS_DIAG                                                                             \
+                   ? launch_kkt_hw<N_, M_, LQRB_HESS_DIAG>(h, s, cb, soc, data, scratch, dz, mult, res, info, cinfo, st) \
+                   : launch_kkt_hw<N_, M_, LQRB_HESS_BLOCKDIAG>(h, s, cb, soc, data, scratch, dz, mult, res, info, cinfo, st);
     KKT_HW_SIZES(X)
 #undef X
     return LQRB_NO_KERNEL;

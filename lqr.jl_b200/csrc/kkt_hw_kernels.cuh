@@ -1,5 +1,5 @@
 // kkt_hw_kernels.cuh — constrained KKT solve for the "quadrotor-sized" class (n + m <= 16): half a warp
-// per instance, one lane per column.
+// per instance.
 //
 // Replaces _solve!(::CholeskySolver) : src/cholesky_solver.jl:166-182 for the stage pattern of the
 // reference's own fixtures (test/problems.jl:58-88: initial condition + dynamics + goal constraint, i.e.
@@ -13,14 +13,13 @@
 // elimination is carried in block-LDL' form with explicit inverses so that everything of order n^3 is a
 // product:  with  Hi = H_k^-1 (a fully parallel pre-pass, one thread per knot),  W = Qi A',  F_k = -W,
 //   Sigma_{k-1} = Cp + Qi_k            (pending Schur complement of row k-1, A_k = C_{k-1} aliasing :165-167)
-//   Si = Sigma^-1 (Gauss-Jordan, one lane per column),  U = Si F_k,  v = Si y_{k-1}      -> record (U, v)
+//   Si = Sigma^-1 (Gauss-Jordan),  U = Si F_k,  v = Si y_{k-1}                            -> record (U, v)
 //   Cp <- A W + B Ri B' - F_k' U,      dp <- (D1 Hi g - d) - F_k' v
 // and the backward sweep is  x_{k-1} = v_k - U_k x_k,  Lambda = -x,  res_k, dz_k = -Hi res_k.
 // The first knot (general C_1: B = C Hi C', E = C Hi D1') and the last knot (C_N, no controls) run the same
-// step with other operands.  Two instances share a warp; lane j of a half-warp owns column j of every n x n
-// block (registers) and the operand that must be seen by all lanes sits in shared memory and is read with
-// broadcast 16-byte loads.  Knot data and Hi are staged by cp.async.bulk + mbarrier, re-issued as soon as
-// their last reader in the current knot is done.
+// step with other operands.  Two instances share a warp (the lane layout of a half-warp is described at
+// kkt_hw2_kernel).  Knot data and Hi are staged by cp.async.bulk + mbarrier, re-issued as soon as their last
+// reader in the current knot is done.
 #pragma once
 #include "riccati_dmma_kernels.cuh"
 
@@ -50,15 +49,13 @@ struct Lay {
     __host__ __device__ static constexpr int64_t knot_off(int k) { return k == 0 ? 0 : FIRST + (int64_t)(k - 1) * MID; }
     __host__ __device__ static constexpr int64_t mult_rows(int N) { return 2 * n + (int64_t)(N - 1) * n; }
     __host__ __device__ static constexpr int64_t z_rows(int N) { return (int64_t)N * n + (int64_t)(N - 1) * m; }
-    // shared memory per instance (doubles): core | hi | MA | MB | vectors
-    static constexpr int sHi = CORE, sMA = sHi + HI, sMB = sMA + n * n, sVec = sMB + n * n, INST = sVec + 128;
-    // block-layout kernel (kkt_hw2_kernel): g | D1 | d of the knot (H is only read by the pre-pass), Hi, three
+    // shared memory per instance (doubles): g | D1 | d of the knot (H is only read by the pre-pass), Hi, three
     // n x n operand buffers, 64 doubles of vectors.  7,008 bytes per instance for n = 12, m = 4: eight 2-warp
     // CTAs = 16 warps per SM (the kernel is bound by the latency of its serial chains: warps are throughput).
     static constexpr int sCore2 = CORE - og, sHi2 = sCore2, s2A = sHi2 + HI, s2B = s2A + n * n, s2C = s2B + n * n,
                          sVec2 = s2C + n * n, INST2 = sVec2 + 64;
     static_assert(INST2 % 2 == 0 && og % 2 == 0, "16-byte alignment of the per-instance buffers");
-    static_assert(2 * n * n >= n * w, "first knot stages C Hi (n x w) in MA|MB");
+    static_assert(2 * n * n >= n * w, "first knot stages C Hi (n x w) in WC|SI");
 };
 
 // In-place inverse of an SPD matrix from its packed upper Cholesky factor (LAPACK potri = trtri + lauum):
@@ -271,343 +268,12 @@ __device__ __forceinline__ int gj_inverse(double (&a)[n], double *colb, int hl) 
     return bad;
 }
 
-// ------------------------------------------------------------------ main kernel -----------------------
-template <int n, int m, int HESS, int WARPS, int MINB>
-__global__ void __launch_bounds__(WARPS * 32, MINB)
-    kkt_hw_kernel(const double *__restrict__ data, const double *__restrict__ hinv, const int32_t *__restrict__ hinfo,
-                  double *__restrict__ recs, double *__restrict__ dz, double *__restrict__ mult,
-                  double *__restrict__ res, int32_t *__restrict__ info, int32_t *__restrict__ cinfo, int N,
-                   int64_t batch, int soc) {
-    using L = Lay<n, m, HESS>;
-    const double gsc = soc ? 0.0 : 1.0;  // second-order correction: g = 0
-    constexpr int w = L::w;
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, hh = lane >> 4, hl = lane & 15;
-    const int64_t inst_raw = ((int64_t)blockIdx.x * WARPS + warp) * 2 + hh;
-    if (((int64_t)blockIdx.x * WARPS + warp) * 2 >= batch) return;  // whole warp leaves
-    const bool active = inst_raw < batch;
-    const int64_t inst = active ? inst_raw : batch - 1;  // an odd tail shadows the last instance (no stores)
-
-    double *wb = reinterpret_cast<double *>(smem_raw) + (size_t)warp * (2 * L::INST + 4);
-    double *S = wb + hh * L::INST;
-    double *core = S, *hi = S + L::sHi, *MA = S + L::sMA, *MB = S + L::sMB, *vec = S + L::sVec;
-    double *ys = vec, *vs = vec + 16, *hgs = vec + 32, *xs = vec + 48, *rs_ = vec + 64, *colb = vec + 80;  // colb: 2n <= 32
-    uint64_t *bars = reinterpret_cast<uint64_t *>(wb + 2 * L::INST);  // [0] core, [1] Hi
-    if (lane == 0) {
-        mbar_init(bars, 1);
-        mbar_init(bars + 1, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncwarp();
-    uint32_t phC = 0, phH = 0;
-
-    const double *db = data + inst * L::data_rows(N);
-    const double *hb = hinv + inst * (int64_t)N * L::HI;
-    double *rb = recs + inst * (int64_t)N * L::REC;
-    double *zb = dz + inst * L::z_rows(N);
-    double *mb = mult + inst * L::mult_rows(N);
-    double *resb = res ? res + inst * L::z_rows(N) : nullptr;
-
-    // one lane per half-warp streams its instance's knot; both halves complete on the warp's barriers
-    auto issue_core = [&](int k) {
-        // only g | D1 | d of a record is read here (H went through the pre-pass)
-        if (lane == 0) mbar_expect_tx(bars, 2u * (uint32_t)((k < N - 1 ? L::CORE - L::og : n + n * n + n) * 8));
-        __syncwarp();
-        if (hl == 0) {
-            const double *src = db + L::knot_off(k);
-            if (k < N - 1) {
-                bulk_g2s(core + L::og, src + L::og, (L::CORE - L::og) * 8, bars);
-            } else {  // last knot: Q | g | C_N | c_N land where Q | g(x) | A | d live
-                bulk_g2s(core + L::og, src + L::HQ, n * 8, bars);
-                bulk_g2s(core + L::oD1, src + L::oCl, n * n * 8, bars);
-                bulk_g2s(core + L::od, src + L::oCl + n * n, n * 8, bars);
-            }
-        }
-    };
-    auto issue_hi = [&](int k) {
-        if (lane == 0) mbar_expect_tx(bars + 1, 2u * (uint32_t)(L::HI * 8));
-        __syncwarp();
-        if (hl == 0) bulk_g2s(hi, hb + (int64_t)k * L::HI, L::HI * 8, bars + 1);
-    };
-    issue_hi(0);
-    issue_core(0);
-
-    int st_all = 0;
-    double Cp[n], dp = 0.0;  // pending Schur complement (column hl) and right-hand side (entry hl)
-    SM_UNROLL
-    for (int i = 0; i < n; ++i) Cp[i] = 0.0;
-
-    // ---------------- forward sweep: k = 0 .. N-1
-    for (int k = 0; k < N; ++k) {
-        const bool first = k == 0, last = k == N - 1;
-        const int mk = last ? 0 : m;
-        mbar_wait(bars + 1, phH);
-        phH ^= 1;
-        mbar_wait(bars, phC);
-        phC ^= 1;
-        const double *Xs = core + L::oD1;          // A_k, or C_N at the last knot (n x n, column-major)
-        const double *Bs = core + L::oD1 + n * n;  // B_k
-        // hg = Hi g
-        double hgj = 0.0;
-        if (hl < n) {
-            double gq[n];
-            SM_UNROLL
-            for (int l = 0; l < n; l += 2) {
-                const double2 v = *reinterpret_cast<const double2 *>(core + L::og + l);
-                gq[l] = gsc * v.x;
-                gq[l + 1] = gsc * v.y;
-            }
-            hgj = dot_col<n>(hi + n * hl, gq);
-        } else if (hl < n + mk) {
-            SM_UNROLL
-            for (int s = 0; s < m; ++s) hgj = fma(hi[n * n + m * (hl - n) + s], gsc * core[L::og + n + s], hgj);
-        }
-        hgs[hl] = hgj;
-
-        // X row hl (the lane's row of A_k / C_N) and W[:, hl] = Qi X[hl, :]'
-        double xrow[n], Wc[n];
-        SM_UNROLL
-        for (int l = 0; l < n; ++l) xrow[l] = hl < n ? Xs[hl + n * l] : 0.0;
-        SM_UNROLL
-        for (int i = 0; i < n; ++i) Wc[i] = 0.0;
-        acc_cols<n, n>(Wc, hi, xrow, 1.0);
-        // V[:, hl] = Ri B[hl, :]'   (B Ri B' = sum_t B[:, t] V[t, hl])
-        double Vc[m];
-        SM_UNROLL
-        for (int t = 0; t < m; ++t) Vc[t] = 0.0;
-        if (!last) {
-            double brow[m];
-            SM_UNROLL
-            for (int t = 0; t < m; ++t) brow[t] = hl < n ? Bs[hl + n * t] : 0.0;
-            SM_UNROLL
-            for (int s = 0; s < m; ++s)
-                SM_UNROLL
-                for (int t = 0; t < m; ++t) Vc[t] = fma(hi[n * n + t + m * s], brow[s], Vc[t]);
-        }
-
-        // Sigma column, right-hand side, coupling block F (column hl)
-        double a[n], Fc[n], y;
-        if (!first) {
-            SM_UNROLL
-            for (int i = 0; i < n; ++i) {
-                a[i] = Cp[i] + (hl < n ? hi[n * hl + i] : (i == 0 ? 1.0 : 0.0));  // res.A .+= YYt[ip1,ip1]
-                Fc[i] = -Wc[i];                                                  // F = D2 Hi D1' = -Qi A'
-            }
-            y = dp - hgj;  // d += next.r_[1]
-        } else {
-            // first knot: T0 = C Hi (n x w) staged in MA|MB, then B = T0 C', E = T0 D1', y = C hg - c
-            const double *C0 = db + L::oC0;
-            double t0[n];
-            SM_UNROLL
-            for (int i = 0; i < n; ++i) t0[i] = 0.0;
-            if (hl < n) {
-                SM_UNROLL
-                for (int l = 0; l < n; ++l) {
-                    const double c = hi[n * hl + l];
-                    SM_UNROLL
-                    for (int i = 0; i < n; ++i) t0[i] = fma(C0[i + n * l], c, t0[i]);
-                }
-            } else if (hl < w) {
-                SM_UNROLL
-                for (int s = 0; s < m; ++s) {
-                    const double c = hi[n * n + m * (hl - n) + s];
-                    SM_UNROLL
-                    for (int i = 0; i < n; ++i) t0[i] = fma(C0[i + n * (n + s)], c, t0[i]);
-                }
-            }
-            if (hl < w) store_col<n>(MA + n * hl, t0);
-            __syncwarp();
-            SM_UNROLL
-            for (int i = 0; i < n; ++i) a[i] = Fc[i] = 0.0;
-            double yy = 0.0;
-            if (hl < n) {
-                double crow[w], drow[w];
-                SM_UNROLL
-                for (int j = 0; j < w; ++j) {
-                    crow[j] = C0[hl + n * j];
-                    drow[j] = core[L::oD1 + hl + n * j];
-                    yy = fma(crow[j], hgs[j], yy);
-                }
-                acc_cols<n, w>(a, MA, crow, 1.0);
-                acc_cols<n, w>(Fc, MA, drow, 1.0);
-                yy -= C0[n * w + hl];
-            } else {
-                a[0] = 1.0;
-            }
-            y = yy;
-            __syncwarp();  // T0 is consumed before MA|MB are reused
-        }
-        {
-            const int bad = gj_inverse<n>(a, colb, hl);
-            if (bad != 0 && st_all == 0) st_all = first ? 1000 + 100 + bad : k * 1000 + 200 + bad;
-        }
-        if (hl < n) {
-            store_col<n>(MA + n * hl, a);   // Si
-            store_col<n>(MB + n * hl, Fc);  // F
-        }
-        ys[hl] = y;
-        __syncwarp();
-        if (k + 1 < N) issue_hi(k + 1);  // Hi_k is no longer read
-        // v = Si y  (Si symmetric: row hl = the lane's column)
-        const double v = dot_vec<n>(a, ys);
-        vs[hl] = v;
-        // U = Si F
-        double Uc[n];
-        SM_UNROLL
-        for (int i = 0; i < n; ++i) Uc[i] = 0.0;
-        acc_cols<n, n>(Uc, MA, Fc, 1.0);
-        if (active && hl < n) {
-            double *rk = rb + (int64_t)k * L::REC;
-            store_col<n>(rk + n * hl, Uc);
-            rk[n * n + hl] = v;
-        }
-        // G22 = X W + B V ; rho2 = X hg_x + B hg_u - d
-        double G[n];
-        SM_UNROLL
-        for (int i = 0; i < n; ++i) G[i] = 0.0;
-        acc_cols<n, n>(G, Xs, Wc, 1.0);
-        if (!last) acc_cols<n, m>(G, Bs, Vc, 1.0);
-        double rho = 0.0;
-        if (hl < n) {
-            rho = -core[L::od + hl];
-            SM_UNROLL
-            for (int l = 0; l < n; ++l) rho = fma(xrow[l], hgs[l], rho);
-            if (!last) {
-                SM_UNROLL
-                for (int t = 0; t < m; ++t) rho = fma(Bs[hl + n * t], hgs[n + t], rho);
-            }
-        }
-        __syncwarp();  // every lane is done with the knot data, Si (MA) and has published vs
-        if (k + 1 < N) issue_core(k + 1);
-        // Cp' = G22 - F'U ; dp' = rho2 - F'v
-        double Cn[n];
-        SM_UNROLL
-        for (int i = 0; i < n; ++i) Cn[i] = G[i] - dot_col<n>(MB + n * i, Uc);
-        dp = rho - dot_vec<n>(Fc, vs);
-        // exact symmetrisation (an antisymmetric rounding residue is amplified by |A|^2 per knot)
-        if (hl < n) store_col<n>(MA + n * hl, Cn);
-        __syncwarp();
-        SM_UNROLL
-        for (int i = 0; i < n; ++i) Cp[i] = hl < n ? 0.5 * (Cn[i] + MA[hl + n * i]) : 0.0;
-        __syncwarp();
-    }
-    // ---------------- last block: mu_N' = Bl'^-1 y_mu  (Cp, dp hold Bl' and y_mu)
-    double xcur;
-    {
-        double a[n];
-        SM_UNROLL
-        for (int i = 0; i < n; ++i) a[i] = hl < n ? Cp[i] : (i == 0 ? 1.0 : 0.0);
-        const int bad = gj_inverse<n>(a, colb, hl);
-        if (bad != 0 && st_all == 0) st_all = N * 1000 + 100 + bad;
-        ys[hl] = dp;
-        __syncwarp();
-        xcur = dot_vec<n>(a, ys);
-        __syncwarp();
-    }
-    if (info && active && hl == 0) {
-        const int hcode = hinfo[inst];
-        info[inst] = hcode != 0x7f7f7f7f ? hcode : st_all;
-    }
-    if (active && hl == 0) cinfo[inst] = -1;  // the column-per-lane variant does not track conditioning
-    if (active && hl < n) __stcs(mb + L::mult_rows(N) - n + hl, -xcur);  // mu_N
-
-    // ---------------- backward sweep: k = N-1 .. 0     x_{k-1} = v_k - U_k x_k,  Lambda = -x
-    issue_hi(N - 1);
-    issue_core(N - 1);
-    for (int k = N - 1; k >= 0; --k) {
-        const bool first = k == 0, last = k == N - 1;
-        const int mk = last ? 0 : m, wk = n + mk;
-        const double *rk = rb + (int64_t)k * L::REC;
-        // record loads (written by this half-warp in the forward sweep)
-        double ucol[n];  // row hl of U_k: U[hl][j] = rk[n*j + hl]
-        SM_UNROLL
-        for (int j = 0; j < n; ++j) ucol[j] = hl < n ? rk[n * j + hl] : 0.0;
-        const double vk = hl < n ? rk[n * n + hl] : 0.0;
-        xs[hl] = xcur;  // x of the block after this record: mu_N' (k = N-1) or lam_k'
-        __syncwarp();
-        double xprev = vk - dot_vec<n>(ucol, xs);  // k >= 1: lam_{k-1}' ; k = 0: mu_1'
-        mbar_wait(bars + 1, phH);
-        phH ^= 1;
-        mbar_wait(bars, phC);
-        phC ^= 1;
-        // res_k = D1' lam_k + C' mu_k + D2' lam_{k-1} + g_k  with Lambda = -x   (calc_residual! :201-236)
-        double r = 0.0;
-        if (hl < wk) {
-            r = gsc * core[L::og + hl];
-            if (!last) {  // D1' lam_k : column hl of [A B] dotted with lam_k = -x_k
-                double xv[n];
-                SM_UNROLL
-                for (int l = 0; l < n; l += 2) {
-                    const double2 t = *reinterpret_cast<const double2 *>(xs + l);
-                    xv[l] = t.x;
-                    xv[l + 1] = t.y;
-                }
-                r -= dot_col<n>(core + L::oD1 + n * hl, xv);
-            } else {  // C_N' mu_N
-                double xv[n];
-                SM_UNROLL
-                for (int l = 0; l < n; l += 2) {
-                    const double2 t = *reinterpret_cast<const double2 *>(xs + l);
-                    xv[l] = t.x;
-                    xv[l + 1] = t.y;
-                }
-                r -= dot_col<n>(core + L::oD1 + n * hl, xv);
-            }
-            if (!first && hl < n) r += xprev;  // D2' lam_{k-1} = -lam_{k-1} = +x_{k-1}
-        }
-        if (first) {  // C_1' mu_1 with mu_1 = -xprev
-            ys[hl] = xprev;
-            __syncwarp();
-            if (hl < wk) {
-                const double *C0 = db + L::oC0;
-                double s = 0.0;
-                SM_UNROLL
-                for (int i = 0; i < n; ++i) s = fma(C0[i + n * hl], ys[i], s);
-                r -= s;
-            }
-        }
-        rs_[hl] = r;
-        __syncwarp();
-        // dz_k = -Hi res_k   (calc_primals! :195-199)
-        double z = 0.0;
-        if (hl < n) {
-            double rv[n];
-            SM_UNROLL
-            for (int l = 0; l < n; l += 2) {
-                const double2 t = *reinterpret_cast<const double2 *>(rs_ + l);
-                rv[l] = t.x;
-                rv[l + 1] = t.y;
-            }
-            z = -dot_col<n>(hi + n * hl, rv);
-        } else if (hl < wk) {
-            SM_UNROLL
-            for (int s = 0; s < m; ++s) z = fma(-hi[n * n + m * (hl - n) + s], rs_[n + s], z);
-        }
-        if (active && hl < wk) {
-            __stcs(zb + (int64_t)k * w + hl, z);
-            if (resb) __stcs(resb + (int64_t)k * w + hl, r);
-        }
-        if (active && hl < n) {
-            // multipliers: [mu_1 (n); lam_1 (n); ...; lam_{N-1}; mu_N]; this knot produces lam_{k-1} (k>=1) or mu_1
-            __stcs(mb + (int64_t)k * n + hl, -xprev);
-        }
-        __syncwarp();  // knot data, Hi, xs, ys, rs_ are free
-        if (k > 0) {
-            issue_hi(k - 1);
-            issue_core(k - 1);
-        }
-        xcur = xprev;
-    }
-}
-
-
-// ------------------------------------------------------------------ block-layout variant --------------
-// Same algorithm and records as kkt_hw_kernel, but every n x n block is spread over the 16 lanes of the
-// half-warp as a 4 x 4 grid of (n/4) x (n/4) register blocks instead of one column per lane.  A product
-// C = X Y' then needs only the lane's n/4 rows of X and n/4 rows of Y from shared memory (2 n^2 / 4 doubles per
-// lane instead of n^2 broadcast to every lane), which halves the shared-memory wavefronts the column
-// version is bound by; Gauss-Jordan exchanges the pivot row / column with 7 shuffles per pivot and the exact
-// symmetrisation is a block transpose by shuffle.  Vectors stay one entry per lane.
+// ------------------------------------------------------------------ block layout ----------------------
+// Every n x n block is spread over the 16 lanes of the half-warp as a 4 x 4 grid of (n/4) x (n/4) register blocks.
+// A product C = X Y' then needs only the lane's n/4 rows of X and n/4 rows of Y from shared memory (2 n^2 / 4
+// doubles per lane instead of n^2 broadcast to every lane with one column per lane, which halves the shared-memory
+// wavefronts); Gauss-Jordan exchanges the pivot row / column with 7 shuffles per pivot and the exact symmetrisation
+// is a block transpose by shuffle.  Vectors stay one entry per lane.
 template <int n, int bs>
 __device__ __forceinline__ void gemm_rr(double (&acc)[bs][bs], const double *X, const double *Y, double sign) {
     // acc[r][c] += sign * sum_l X[r*n + l] * Y[c*n + l]

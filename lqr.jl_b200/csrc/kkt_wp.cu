@@ -2,12 +2,12 @@
 #include "kkt_dispatch.cuh"
 #include "kkt_wp_kernels.cuh"
 
-// warp-per-instance FP64 tensor-core kernel (kkt_wp_kernels.cuh): the default for the half-warp size list; H^-1 is
-// formed in the kernel, so there is no pre-pass and no Hi array (scratch: the records and the two info arrays)
+// warp-per-instance FP64 tensor-core kernel (kkt_wp_kernels.cuh): H^-1 is formed in the kernel, so there is no
+// pre-pass and no Hi array (scratch: the records and the conditioning estimates)
 template <int n, int m, int HESS>
-static int32_t launch_kkt_wp(lqrb_context *h, const KktShape &s, int64_t batch, int soc, const double *data,
-                             double *scratch, double *dz, double *mult, double *res, int32_t *info, cudaStream_t st) {
-    using L = kwp::Lay<n, m, HESS>;
+static int32_t launch_kkt_wp(lqrb_context *h, const KktShape &s, int64_t cb, int soc, const double *data,
+                             double *scratch, double *dz, double *mult, double *res, int32_t *info, int32_t **cinfo_out,
+                             cudaStream_t st) {
     using RW = kwp::RecW<n>;
     const int N = s.N;
     constexpr int WARPS = 4, MINB = 3;  // 168 registers: 12 warps per SM
@@ -19,49 +19,34 @@ static int32_t launch_kkt_wp(lqrb_context *h, const KktShape &s, int64_t batch, 
         int32_t trc = lqrb_kkt_tables(h, n, m, N, s.p, HESS, 0, &tb);
         if (trc) return trc;
     }
-    const int64_t drows = lqrb_kkt_data_rows(n, m, N, s.p, HESS, 0), zrows = L::z_rows(N), mrows = lqrb_num_cons(n, N, s.p);
     auto kern = kwp::kkt_wp_kernel<n, m, HESS, WARPS, MINB>;
     LQRB_CUDA(h, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    const int64_t chunk = std::min(batch, kkt_tuned_chunk(h, s));
-    int64_t refined = 0;
-    for (int64_t first = 0; first < batch; first += chunk) {
-        const int64_t cb = std::min(chunk, batch - first);
-        // scratch (reused by every chunk): [records: cb x N x REC] [cinfo: cb]
-        double *recs = scratch;
-        int32_t *cinfo = reinterpret_cast<int32_t *>(recs + (size_t)cb * N * RW::rec(ps));
-        const double *dc = data + first * drows;
-        kern<<<(unsigned)((cb + WARPS - 1) / WARPS), WARPS * 32, smem, st>>>(
-            dc, recs, dz + first * zrows, mult + first * mrows, res ? res + first * zrows : nullptr,
-            info ? info + first : nullptr, cinfo, N, cb, soc, ps, s.uniform ? nullptr : tb.p,
-            s.uniform ? nullptr : tb.knot_off, s.uniform ? nullptr : tb.mult_off, s.free_final ? 1 : 0);
-        LQRB_LAUNCH_CHECK(h, "kkt_wp_kernel");
-        int32_t rc = kkt_resolve_ill_conditioned(h, s, cb, soc ? LQRB_FLAG_SOC : 0, dc, cinfo, dz + first * zrows,
-                                                 mult + first * mrows, res ? res + first * zrows : nullptr,
-                                                 info ? info + first : nullptr, st);
-        if (rc) return rc;
-        refined += h->last_refined;
-    }
+    // scratch: [records: cb x N x REC] [cinfo: cb]
+    double *recs = scratch;
+    int32_t *cinfo = reinterpret_cast<int32_t *>(recs + (size_t)cb * N * RW::rec(ps));
+    kern<<<(unsigned)((cb + WARPS - 1) / WARPS), WARPS * 32, smem, st>>>(
+        data, recs, dz, mult, res, info, cinfo, N, cb, soc, ps, s.uniform ? nullptr : tb.p,
+        s.uniform ? nullptr : tb.knot_off, s.uniform ? nullptr : tb.mult_off, s.free_final ? 1 : 0);
+    LQRB_LAUNCH_CHECK(h, "kkt_wp_kernel");
+    *cinfo_out = cinfo;
     char nm[128];
     if (s.uniform)
         snprintf(nm, sizeof nm, "kkt_wp_dmma<%d,%d,p=%d/%d/%d,hess=%d%s>", n, m, n, ps, n, HESS, soc ? ",soc" : "");
     else
         snprintf(nm, sizeof nm, "kkt_wp_dmma<%d,%d,p=%d/per-knot<=%d/%d,hess=%d%s>", n, m, n, ps, n, HESS, soc ? ",soc" : "");
     h->kernel_name = nm;
-    if (refined) h->kernel_name += "+kkt_coop[" + std::to_string(refined) + " ill-conditioned]";
-    h->last_refined = refined;
     return 0;
 }
 
-int32_t kkt_launch_wp(lqrb_context *h, const KktShape &s, int64_t batch, int flags, const double *data, double *scratch,
-                      double *dz, double *mult, double *res, int32_t *info, cudaStream_t st) {
-    const int soc = (flags & LQRB_FLAG_SOC) ? 1 : 0;
-#define X(N_, M_)                                                                                                        \
-    if (s.n == N_ && s.m == M_) {                                                                                        \
-        if (s.hess == LQRB_HESS_DIAG)                                                                                    \
-            return launch_kkt_wp<N_, M_, LQRB_HESS_DIAG>(h, s, batch, soc, data, scratch, dz, mult, res, info, st);      \
-        if (s.hess == LQRB_HESS_BLOCKDIAG)                                                                               \
-            return launch_kkt_wp<N_, M_, LQRB_HESS_BLOCKDIAG>(h, s, batch, soc, data, scratch, dz, mult, res, info, st); \
-        return launch_kkt_wp<N_, M_, LQRB_HESS_DENSE>(h, s, batch, soc, data, scratch, dz, mult, res, info, st);         \
+int32_t kkt_wp_chunk(lqrb_context *h, const KktShape &s, int64_t cb, int soc, const double *data, double *scratch,
+                     double *dz, double *mult, double *res, int32_t *info, int32_t **cinfo, cudaStream_t st) {
+#define X(N_, M_)                                                                                                          \
+    if (s.n == N_ && s.m == M_) {                                                                                          \
+        if (s.hess == LQRB_HESS_DIAG)                                                                                      \
+            return launch_kkt_wp<N_, M_, LQRB_HESS_DIAG>(h, s, cb, soc, data, scratch, dz, mult, res, info, cinfo, st);      \
+        if (s.hess == LQRB_HESS_BLOCKDIAG)                                                                                 \
+            return launch_kkt_wp<N_, M_, LQRB_HESS_BLOCKDIAG>(h, s, cb, soc, data, scratch, dz, mult, res, info, cinfo, st); \
+        return launch_kkt_wp<N_, M_, LQRB_HESS_DENSE>(h, s, cb, soc, data, scratch, dz, mult, res, info, cinfo, st);         \
     }
     KKT_WP_SIZES(X)
 #undef X

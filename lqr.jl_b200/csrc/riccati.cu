@@ -42,7 +42,7 @@ static bool riccati_has_cta(int n, int m) {
 }
 
 int lqrb_riccati_tile(const lqrb_context *h, int n, int m) {
-    const int64_t force = h->opt("riccati_variant", 0);  // 1 = tpi, 2 = coop
+    const int64_t force = h->opt("riccati_variant", 0);  // 2 = coop
     if (force == 2) return 1;
     return riccati_has_tpi(n, m) ? LQRB_TILE : 1;
 }
@@ -83,12 +83,6 @@ static std::vector<RowMap> riccati_gain_map(int n, int m, int N) {
         for (int e = 0; e < m * n; ++e) map.push_back({0, k * m * n + e, 0.0});
         for (int e = 0; e < m; ++e) map.push_back({1, k * m + e, 0.0});
     }
-    return map;
-}
-
-static std::vector<RowMap> identity_rows(int64_t rows) {
-    std::vector<RowMap> map((size_t)rows);
-    for (int64_t r = 0; r < rows; ++r) map[(size_t)r] = RowMap{0, (int32_t)r, 0.0};
     return map;
 }
 
@@ -428,8 +422,7 @@ static int32_t riccati_unpack_on(lqrb_context *h, int n, int m, int N, int64_t b
     ArrayTableOut t = {};
     t.ptr[0] = Z;
     t.stride[0] = NN;
-    int32_t rc = lqrb_scatter_unpack(h, lqrb_get_map(h, "id" + std::to_string(NN), identity_rows(NN)), t,
-                                     batch, tile, Zp, s);
+    int32_t rc = lqrb_scatter_unpack(h, lqrb_identity_map(h, NN), t, batch, tile, Zp, s);
     if (rc) return rc;
     if (K || kff) {
         ArrayTableOut g = {};

@@ -881,20 +881,15 @@ extern "C" int32_t lqrb_sqp_dubins_f64(lqrb_handle_t h, int64_t batch, const lqr
         dx0 = stage + batch * NN;
         dxf = stage + batch * (NN + n);
     }
-    auto idmap = [&](int64_t rows) {
-        std::vector<RowMap> mp((size_t)rows);
-        for (int64_t r = 0; r < rows; ++r) mp[(size_t)r] = RowMap{0, (int32_t)r, 0.0};
-        return lqrb_get_map(h, "id" + std::to_string(rows), mp);
-    };
     ArrayTable t = {};
     t.ptr[0] = dZ; t.stride[0] = NN;
-    int32_t rc = lqrb_gather_pack(h, idmap(NN), t, batch, LQRB_TILE, Zp, s);
+    int32_t rc = lqrb_gather_pack(h, lqrb_identity_map(h, NN), t, batch, LQRB_TILE, Zp, s);
     if (rc) return rc;
     t.ptr[0] = dx0; t.stride[0] = n;
-    rc = lqrb_gather_pack(h, idmap(n), t, batch, LQRB_TILE, x0p, s);
+    rc = lqrb_gather_pack(h, lqrb_identity_map(h, n), t, batch, LQRB_TILE, x0p, s);
     if (rc) return rc;
     t.ptr[0] = dxf;
-    rc = lqrb_gather_pack(h, idmap(n), t, batch, LQRB_TILE, xfp, s);
+    rc = lqrb_gather_pack(h, lqrb_identity_map(h, n), t, batch, LQRB_TILE, xfp, s);
     if (rc) return rc;
     LQRB_CUDA(h, cudaMemsetAsync(multk, 0, (size_t)ldb * P * 8, s));
 
@@ -979,7 +974,7 @@ extern "C" int32_t lqrb_sqp_dubins_f64(lqrb_handle_t h, int64_t batch, const lqr
     }
     ArrayTableOut to = {};
     to.ptr[0] = oZ; to.stride[0] = NN;
-    rc = lqrb_scatter_unpack(h, idmap(NN), to, batch, LQRB_TILE, Zp, s);
+    rc = lqrb_scatter_unpack(h, lqrb_identity_map(h, NN), to, batch, LQRB_TILE, Zp, s);
     if (rc) return rc;
     stats_export_kernel<<<grid, 64, 0, s>>>(stats, (feas_p || !dev) ? ofp : nullptr, (feas_d || !dev) ? ofd : nullptr,
                                             (iters_done || !dev) ? oit : nullptr, batch);
