@@ -7,8 +7,12 @@
  * lqr.jl_b200/julia/LQRB200.jl, and INTEGRATION.md shows the binding a maintainer would add.
  *
  * Conventions
- *   - plain C types only; every array is caller-owned (host OR device pointer, detected with
- *     cudaPointerGetAttributes); the library owns only its handle and internal scratch.
+ *   - plain C types only; every array is caller-owned; the library owns only its handle and internal scratch.
+ *   - instance-major arrays may be host or device memory.  A call is device-resident when every non-NULL
+ *     array it is given, inputs and outputs alike, is device or managed memory (cudaPointerGetAttributes):
+ *     it then runs on the handle's stream and returns without synchronising.  Any other call is staged:
+ *     its arrays are copied through device buffers in chunks over two internal streams (each copy
+ *     cudaMemcpyDefault, so device arrays in a staged call are fine), and it returns when done.
  *   - every function returns int32: 0 ok; -i = argument i (1-based) invalid (LAPACK style);
  *     >0 = 1000 + cudaError_t.  Nothing throws across the ABI.  lqrb_last_error_string() explains.
  *   - numerical failure never aborts a batch: per-instance `info[batch]` mirrors the potrf `info`
@@ -115,7 +119,7 @@ int64_t lqrb_kkt_knot_offset(int32_t n, int32_t m, int32_t N, const int32_t *p, 
  * compute_ctg! :48-52, chol_solve! :28-31) and the rollout of src/least_squares.jl:195-202,
  * generalised to per-knot (LTV) data and affine cost terms (SURVEY Appendix A).
  *
- * Instance-major arrays (host or device; all the same kind):
+ * Instance-major arrays (host or device):
  *   A[n,n,Kn,batch] B[n,m,Kn,batch] Q[n,n,Kn,batch] R[m,m,Kn,batch] q[n,Kn,batch] r[m,Kn,batch]
  *   Qf[n,n,batch] qf[n,batch] x0[n,batch]       Kn = (flags & LTI) ? 1 : N-1; q, r, qf may be NULL
  * Outputs: Z[NN,batch] (Primals order), optional K[m,n,N-1,batch], kff[m,N-1,batch], info[batch].

@@ -15,14 +15,16 @@ int32_t lqrb_cuda_fail(lqrb_context *h, cudaError_t e, const char *what) {
     return 1000 + (int32_t)e;
 }
 
-void *lqrb_scratch(lqrb_context *h, int slot, size_t bytes) {
+void *lqrb_scratch(lqrb_context *h, int slot, size_t bytes, int lane) {
     if (bytes == 0) bytes = 16;
-    if (h->scratch_bytes[slot] >= bytes) return h->scratch[slot];
-    if (h->scratch[slot]) {
-        cudaDeviceSynchronize();  // the slot may still be in use on the handle's copy streams
-        cudaFree(h->scratch[slot]);
-        h->scratch[slot] = nullptr;
-        h->scratch_bytes[slot] = 0;
+    void *&cur = h->scratch[slot][lane];
+    size_t &have = h->scratch_bytes[slot][lane];
+    if (have >= bytes) return cur;
+    if (cur) {
+        cudaDeviceSynchronize();  // the slot may still be in use on the handle's streams
+        cudaFree(cur);
+        cur = nullptr;
+        have = 0;
     }
     void *p = nullptr;
     cudaError_t e = cudaMalloc(&p, bytes);
@@ -30,19 +32,19 @@ void *lqrb_scratch(lqrb_context *h, int slot, size_t bytes) {
         lqrb_cuda_fail(h, e, "cudaMalloc(scratch)");
         return nullptr;
     }
-    h->scratch[slot] = p;
-    h->scratch_bytes[slot] = bytes;
+    cur = p;
+    have = bytes;
     return p;
 }
 
-void *lqrb_pinned(lqrb_context *h, int slot, size_t bytes) {
+void *lqrb_pinned(lqrb_context *h, int lane, size_t bytes) {
     if (bytes == 0) bytes = 16;
-    if (h->pinned_bytes[slot] >= bytes) return h->pinned[slot];
-    if (h->pinned[slot]) {
+    if (h->pinned_bytes[lane] >= bytes) return h->pinned[lane];
+    if (h->pinned[lane]) {
         cudaStreamSynchronize(h->stream);
-        cudaFreeHost(h->pinned[slot]);
-        h->pinned[slot] = nullptr;
-        h->pinned_bytes[slot] = 0;
+        cudaFreeHost(h->pinned[lane]);
+        h->pinned[lane] = nullptr;
+        h->pinned_bytes[lane] = 0;
     }
     void *p = nullptr;
     cudaError_t e = cudaMallocHost(&p, bytes);
@@ -50,20 +52,9 @@ void *lqrb_pinned(lqrb_context *h, int slot, size_t bytes) {
         lqrb_cuda_fail(h, e, "cudaMallocHost");
         return nullptr;
     }
-    h->pinned[slot] = p;
-    h->pinned_bytes[slot] = bytes;
+    h->pinned[lane] = p;
+    h->pinned_bytes[lane] = bytes;
     return p;
-}
-
-bool lqrb_is_device_ptr(const void *p) {
-    if (!p) return false;
-    cudaPointerAttributes a;
-    cudaError_t e = cudaPointerGetAttributes(&a, p);
-    if (e != cudaSuccess) {
-        cudaGetLastError();
-        return false;
-    }
-    return a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged;
 }
 
 // ------------------------------------------------------------------ library / handle ----------
@@ -122,10 +113,11 @@ extern "C" int32_t lqrb_destroy(lqrb_handle_t h) {
     if (!h) return -1;
     cudaSetDevice(h->device);
     cudaDeviceSynchronize();
-    for (int i = 0; i < SCR_COUNT; ++i)
-        if (h->scratch[i]) cudaFree(h->scratch[i]);
-    for (int i = 0; i < 4; ++i)
-        if (h->pinned[i]) cudaFreeHost(h->pinned[i]);
+    for (auto &slot : h->scratch)
+        for (void *p : slot)
+            if (p) cudaFree(p);
+    for (void *p : h->pinned)
+        if (p) cudaFreeHost(p);
     for (auto &kv : h->maps)
         if (kv.second.dev) cudaFree((void *)kv.second.dev);
     for (auto &kv : h->blobs)

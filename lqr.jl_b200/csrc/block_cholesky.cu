@@ -89,29 +89,6 @@ __global__ void block_ldiv_kernel(const double *__restrict__ M, double *__restri
     }
 }
 
-// copies host arrays to a staging scratch when needed; returns device pointers
-static int32_t stage_in(lqrb_context *h, int slot, const void *const *src, const size_t *bytes, int count,
-                        const void **dev, bool on_device) {
-    if (on_device) {
-        for (int i = 0; i < count; ++i) dev[i] = src[i];
-        return 0;
-    }
-    size_t tot = 0;
-    for (int i = 0; i < count; ++i) tot += round_up((int64_t)(src[i] ? bytes[i] : 0), 256);
-    char *buf = (char *)lqrb_scratch(h, slot, tot);
-    if (!buf) return 1000 + (int)cudaErrorMemoryAllocation;
-    for (int i = 0; i < count; ++i) {
-        if (!src[i]) {
-            dev[i] = nullptr;
-            continue;
-        }
-        LQRB_CUDA(h, cudaMemcpyAsync(buf, src[i], bytes[i], cudaMemcpyHostToDevice, h->stream));
-        dev[i] = buf;
-        buf += round_up((int64_t)bytes[i], 256);
-    }
-    return 0;
-}
-
 extern "C" int32_t lqrb_block_cholesky_f64(lqrb_handle_t h, int32_t n, int32_t m, int64_t batch,
                                            int32_t mode, const double *A, const double *B,
                                            const double *C, double *M, int32_t *info) {
@@ -125,30 +102,18 @@ extern "C" int32_t lqrb_block_cholesky_f64(lqrb_handle_t h, int32_t n, int32_t m
     if (!M) return lqrb_fail(h, -9, "M is NULL");
     if (batch == 0) return 0;
     LQRB_CUDA(h, cudaSetDevice(h->device));
-    const bool dev = lqrb_is_device_ptr(A);
     const int w = n + m;
-    const void *src[3] = {A, B, C};
-    const size_t bytes[3] = {(size_t)batch * n * n * 8, (size_t)batch * m * m * 8, (size_t)batch * m * n * 8};
-    const void *d[3];
-    int32_t rc = stage_in(h, SCR_STAGE_A, src, bytes, 3, d, dev);
-    if (rc) return rc;
-    double *dM = M;
-    int32_t *dinfo = info;
-    if (!dev) {
-        dM = (double *)lqrb_scratch(h, SCR_STAGE_B, (size_t)batch * w * w * 8);
-        dinfo = (int32_t *)lqrb_scratch(h, SCR_INFO, (size_t)batch * 4);
-        if (!dM || !dinfo) return 1000 + (int)cudaErrorMemoryAllocation;
-    }
-    block_cholesky_kernel<<<(unsigned)((batch + 63) / 64), 64, 0, h->stream>>>(
-        (const double *)d[0], (const double *)d[1], (const double *)d[2], dM, dinfo, n, m, mode, batch);
-    h->kernel_name = "block_cholesky";
-    LQRB_LAUNCH_CHECK(h, "block_cholesky_kernel");
-    if (!dev) {
-        LQRB_CUDA(h, cudaMemcpyAsync(M, dM, (size_t)batch * w * w * 8, cudaMemcpyDeviceToHost, h->stream));
-        if (info) LQRB_CUDA(h, cudaMemcpyAsync(info, dinfo, (size_t)batch * 4, cudaMemcpyDeviceToHost, h->stream));
-        LQRB_CUDA(h, cudaStreamSynchronize(h->stream));
-    }
-    return 0;
+    return lqrb_for_chunks(
+        h, batch, batch, {{A, (int64_t)n * n * 8}, {B, (int64_t)m * m * 8}, {C, (int64_t)m * n * 8}},
+        {{M, (int64_t)w * w * 8}, {info, 4}},
+        [&](Lane lane, int64_t cb, const void *const *in, void *const *out) -> int32_t {
+            block_cholesky_kernel<<<(unsigned)((cb + 63) / 64), 64, 0, lane.stream>>>(
+                (const double *)in[0], (const double *)in[1], (const double *)in[2], (double *)out[0], (int32_t *)out[1],
+                n, m, mode, cb);
+            h->kernel_name = "block_cholesky";
+            LQRB_LAUNCH_CHECK(h, "block_cholesky_kernel");
+            return 0;
+        });
 }
 
 extern "C" int32_t lqrb_block_ldiv_f64(lqrb_handle_t h, int32_t n, int32_t m, int64_t batch,
@@ -163,21 +128,16 @@ extern "C" int32_t lqrb_block_ldiv_f64(lqrb_handle_t h, int32_t n, int32_t m, in
     if (!b) return lqrb_fail(h, -8, "b is NULL");
     if (batch == 0 || nrhs == 0) return 0;
     LQRB_CUDA(h, cudaSetDevice(h->device));
-    const bool dev = lqrb_is_device_ptr(M);
     const int w = n + m;
-    const void *src[2] = {M, b};
-    const size_t bytes[2] = {(size_t)batch * w * w * 8, (size_t)batch * w * nrhs * 8};
-    const void *d[2];
-    int32_t rc = stage_in(h, SCR_STAGE_A, src, bytes, 2, d, dev);
-    if (rc) return rc;
-    const int64_t tot = batch * nrhs;
-    block_ldiv_kernel<<<(unsigned)((tot + 63) / 64), 64, 0, h->stream>>>((const double *)d[0], (double *)d[1], n, m,
-                                                                         mode, nrhs, batch);
-    h->kernel_name = "block_ldiv";
-    LQRB_LAUNCH_CHECK(h, "block_ldiv_kernel");
-    if (!dev) {
-        LQRB_CUDA(h, cudaMemcpyAsync(b, d[1], bytes[1], cudaMemcpyDeviceToHost, h->stream));
-        LQRB_CUDA(h, cudaStreamSynchronize(h->stream));
-    }
-    return 0;
+    const int64_t bb = (int64_t)w * nrhs * 8;
+    // b is updated in place
+    return lqrb_for_chunks(h, batch, batch, {{M, (int64_t)w * w * 8}, {b, bb}}, {{b, bb}},
+                           [&](Lane lane, int64_t cb, const void *const *in, void *const *out) -> int32_t {
+                               const int64_t tot = cb * nrhs;
+                               block_ldiv_kernel<<<(unsigned)((tot + 63) / 64), 64, 0, lane.stream>>>(
+                                   (const double *)in[0], (double *)out[0], n, m, mode, nrhs, cb);
+                               h->kernel_name = "block_ldiv";
+                               LQRB_LAUNCH_CHECK(h, "block_ldiv_kernel");
+                               return 0;
+                           });
 }

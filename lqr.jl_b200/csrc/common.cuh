@@ -4,6 +4,7 @@
 #include <stdint.h>
 
 #include <algorithm>
+#include <functional>
 #include <map>
 #include <string>
 #include <vector>
@@ -34,34 +35,37 @@ __host__ __device__ constexpr int hess_rows(int n, int mk, int hess) {
 }
 
 // ------------------------------------------------------------------ context -------------------
+// Device scratch: one grow-only allocation per (slot, lane); see `Lane`.
 enum ScratchSlot {
     SCR_GAINS = 0,
     SCR_FACT,
-    SCR_STAGE_A,
-    SCR_STAGE_B,
+    SCR_STAGE_A,  // lqrb_for_chunks: staged inputs of a chunk
+    SCR_STAGE_B,  //                  staged outputs of a chunk
     SCR_PACK_IN,
     SCR_PACK_IN2,
     SCR_PACK_OUT,
     SCR_PACK_OUT2,
     SCR_PACK_OUT3,
-    SCR_INFO,
-    SCR_MAP,
     SCR_MISC,
     SCR_SQP0,
     SCR_SQP1,
     SCR_SQP2,
     SCR_SQP3,
-    SCR_KEEP_DATA,  // lqrb_kkt_factor_f64: packed matrices of the kept factorisation
-    SCR_KEEP_REC,   //                      block rows of U (BlockUpperTriangular3 records)
-    // one slot per stream for everything the host-buffer paths use from inside a chunk (two chunks are in flight, and
-    // chunk sizes differ: slices of one allocation at a size-dependent offset could overlap)
+    SCR_KEEP_DATA,    // lqrb_kkt_factor_f64: packed matrices of the kept factorisation
+    SCR_KEEP_REC,     //                      block rows of U (BlockUpperTriangular3 records)
     SCR_REFINE,       // records of the instances re-solved by the Cholesky-based kernel (ill-conditioned blocks)
-    SCR_REFINE_B,
     SCR_REFINE_LIST,  // their indices
-    SCR_REFINE_LIST_B,
     SCR_RICCATI_PAD,  // Riccati problems embedded in a tuned size class: padded knots, term, Z, gains
-    SCR_RICCATI_PAD_B,
     SCR_COUNT
+};
+
+// Where a piece of work runs: its stream and which per-lane scratch it owns.  A staged call (lqrb_for_chunks) runs its
+// chunks alternately on lanes {copy_stream[0], 0} and {copy_stream[1], 1}; a device-resident call runs on
+// {h->stream, 0}.  Sharing lane 0 between h->stream and copy stream 0 is safe: a staged call waits for h->stream before
+// its first chunk and synchronises both copy streams before it returns, so work of two calls never overlaps on it.
+struct Lane {
+    cudaStream_t stream;
+    int index;  // 0 or 1
 };
 
 struct RowMap;
@@ -80,10 +84,10 @@ struct lqrb_context {
     std::string err;
     std::string kernel_name;
     int64_t launches = 0;
-    void *scratch[SCR_COUNT] = {};
-    size_t scratch_bytes[SCR_COUNT] = {};
-    void *pinned[4] = {};
-    size_t pinned_bytes[4] = {};
+    void *scratch[SCR_COUNT][2] = {};
+    size_t scratch_bytes[SCR_COUNT][2] = {};
+    void *pinned[2] = {};
+    size_t pinned_bytes[2] = {};
     std::map<std::string, int64_t> options;
     std::map<std::string, struct DevMap> maps;  // cached device copies of row maps
     std::map<std::string, void *> blobs;        // cached device tables (cooperative KKT offsets)
@@ -101,10 +105,28 @@ struct lqrb_context {
 
 int32_t lqrb_fail(lqrb_context *h, int32_t code, const std::string &msg);
 int32_t lqrb_cuda_fail(lqrb_context *h, cudaError_t e, const char *what);
-// grow-only scratch; returns nullptr and records the error on failure
-void *lqrb_scratch(lqrb_context *h, int slot, size_t bytes);
-void *lqrb_pinned(lqrb_context *h, int slot, size_t bytes);
-bool lqrb_is_device_ptr(const void *p);
+// grow-only scratch of one lane; returns nullptr and records the error on failure
+void *lqrb_scratch(lqrb_context *h, int slot, size_t bytes, int lane = 0);
+void *lqrb_pinned(lqrb_context *h, int lane, size_t bytes);
+
+// ------------------------------------------------------------------ host / device staging (host_io.cu) ----
+// One instance-major caller array: its pointer (NULL: absent) and its bytes per instance (0: absent).
+struct HostArray {
+    const void *ptr;
+    int64_t bytes;
+};
+// Runs one chunk of `cb` instances (chunks run in instance order).  `in` / `out` hold device pointers to the chunk's
+// part of every listed array, in list order; absent arrays are NULL.
+using ChunkBody = std::function<int32_t(Lane lane, int64_t cb, const void *const *in, void *const *out)>;
+// Runs `body` over the batch.  A call is device-resident when every present array, inputs and outputs alike, is device
+// or managed memory: then `body` runs once on {h->stream, 0} with the caller's own pointers, without synchronising.
+// Otherwise the call is staged: chunks of `chunk` instances alternate over the two copy streams; each copies its part
+// of every present input into the lane's staging scratch, runs `body`, and copies every present output back; the call
+// returns when both streams are done.  An output with the same pointer as an input is updated in place (in/out arrays).
+// chunk = 0 picks the size: the `host_chunk` option if set, otherwise about 64 MB of input (counting every listed
+// input, present or not), rounded up to LQRB_TILE.
+int32_t lqrb_for_chunks(lqrb_context *h, int64_t batch, int64_t chunk, const std::vector<HostArray> &inputs,
+                        const std::vector<HostArray> &outputs, const ChunkBody &body);
 
 #define LQRB_CUDA(h, call)                                              \
     do {                                                                \
@@ -163,4 +185,8 @@ int32_t lqrb_scatter_unpack(lqrb_context *h, const DevMap &map, const ArrayTable
 int lqrb_riccati_tile(const lqrb_context *h, int n, int m);
 int lqrb_kkt_tile(const lqrb_context *h, int n, int m, int N, const int32_t *p, int hess_mode,
                   int explicit_d2);
+// lqrb_kkt_solve_packed_f64 on a given lane (the SQP driver calls it from inside its own staged call)
+int32_t lqrb_kkt_solve_packed_on(lqrb_context *h, int n, int m, int N, int64_t batch, const int32_t *p, int hess_mode,
+                                 int explicit_d2, int flags, const double *data, double *dz, double *mult, double *res,
+                                 int32_t *info, Lane lane);
 

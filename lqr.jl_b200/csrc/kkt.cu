@@ -233,10 +233,10 @@ static void kkt_keep_record(lqrb_context *h, KktRecord &rec) {
 // outputs.  `kkt_refine` = 0 switches this off.  Costs one 4-byte-per-instance read-back and a stream synchronisation.
 static int32_t kkt_resolve_ill_conditioned(lqrb_context *h, const KktShape &s, int64_t cb, int flags, const double *dc,
                                            const int32_t *cinfo_dev, double *dz, double *mult, double *res, int32_t *info,
-                                           cudaStream_t st, KktRecord *record) {
+                                           Lane lane, KktRecord *record) {
     if (h->opt("kkt_refine", 1) == 0) return 0;
-    const int slot = st == h->copy_stream[1] ? 1 : 0;
-    int32_t *hc = (int32_t *)lqrb_pinned(h, 2 + slot, (size_t)cb * sizeof(int32_t));
+    const cudaStream_t st = lane.stream;
+    int32_t *hc = (int32_t *)lqrb_pinned(h, lane.index, (size_t)cb * sizeof(int32_t));
     if (!hc) return 1000 + (int)cudaErrorMemoryAllocation;
     LQRB_CUDA(h, cudaMemcpyAsync(hc, cinfo_dev, (size_t)cb * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
     LQRB_CUDA(h, cudaStreamSynchronize(st));
@@ -252,9 +252,8 @@ static int32_t kkt_resolve_ill_conditioned(lqrb_context *h, const KktShape &s, i
     const int64_t piece = std::max<int64_t>(1, (int64_t)(((size_t)h->opt("scratch_budget_mb", 49152) << 20) / 4 / per));
     for (size_t first = 0; first < list.size(); first += (size_t)piece) {
         const int64_t cnt = std::min<int64_t>(piece, (int64_t)(list.size() - first));
-        // separate allocations per stream: the host-buffer path has two of these in flight
-        int32_t *dl = (int32_t *)lqrb_scratch(h, slot ? SCR_REFINE_LIST_B : SCR_REFINE_LIST, (size_t)cb * sizeof(int32_t));
-        double *rec = (double *)lqrb_scratch(h, slot ? SCR_REFINE_B : SCR_REFINE, (size_t)std::min<int64_t>(piece, cb) * per);
+        int32_t *dl = (int32_t *)lqrb_scratch(h, SCR_REFINE_LIST, (size_t)cb * sizeof(int32_t), lane.index);
+        double *rec = (double *)lqrb_scratch(h, SCR_REFINE, (size_t)std::min<int64_t>(piece, cb) * per, lane.index);
         if (!dl || !rec) return 1000 + (int)cudaErrorMemoryAllocation;
         LQRB_CUDA(h, cudaMemcpyAsync(dl, list.data() + first, (size_t)cnt * sizeof(int32_t), cudaMemcpyHostToDevice, st));
         KktCoopExtra ex;
@@ -268,7 +267,7 @@ static int32_t kkt_resolve_ill_conditioned(lqrb_context *h, const KktShape &s, i
             ex.data_stride = z.data_rows;
             ex.mult_stride = z.P;
         }
-        int32_t rc = launch_kkt_coop(h, s.n, s.m, s.N, pp, s.hess, s.d2x, flags, cnt, dc, rec, dz, mult, res, info, st, &ex);
+        int32_t rc = launch_kkt_coop(h, s.n, s.m, s.N, pp, s.hess, s.d2x, flags, cnt, dc, rec, dz, mult, res, info, lane, &ex);
         if (rc) return rc;
         LQRB_CUDA(h, cudaStreamSynchronize(st));  // `list` (pageable) must outlive the copy
     }
@@ -307,7 +306,7 @@ static size_t kkt_tuned_scratch_bytes(const lqrb_context *h, const KktShape &s, 
 // ill-conditioned instances.  The kernel name counts the re-solved instances of the whole call so far.
 static int32_t kkt_solve_tuned(lqrb_context *h, KktFamily family, const KktShape &s, int64_t batch, int flags,
                                const double *data, double *scratch, double *dz, double *mult, double *res, int32_t *info,
-                               cudaStream_t st, KktRecord *record) {
+                               Lane lane, KktRecord *record) {
     auto launch = family == KktFamily::Cta ? kkt_cta_chunk : family == KktFamily::Wp ? kkt_wp_chunk : kkt_hw_chunk;
     const KktSizes z = kkt_sizes(s);
     const int soc = (flags & LQRB_FLAG_SOC) ? 1 : 0;
@@ -318,10 +317,10 @@ static int32_t kkt_solve_tuned(lqrb_context *h, KktFamily family, const KktShape
         const double *dc = data + first * z.data_rows;
         double *dzc = dz + first * z.NN, *mc = mult + first * z.P, *rc_ = res ? res + first * z.NN : nullptr;
         int32_t *ic = info ? info + first : nullptr, *cinfo = nullptr;
-        int32_t rc = launch(h, s, cb, soc, dc, scratch, dzc, mc, rc_, ic, &cinfo, st);
+        int32_t rc = launch(h, s, cb, soc, dc, scratch, dzc, mc, rc_, ic, &cinfo, lane.stream);
         if (rc) return rc;
         name = h->kernel_name;  // (the re-solve names its own kernel)
-        rc = kkt_resolve_ill_conditioned(h, s, cb, soc ? LQRB_FLAG_SOC : 0, dc, cinfo, dzc, mc, rc_, ic, st, record);
+        rc = kkt_resolve_ill_conditioned(h, s, cb, soc ? LQRB_FLAG_SOC : 0, dc, cinfo, dzc, mc, rc_, ic, lane, record);
         if (rc) return rc;
     }
     record->tuned = true;
@@ -459,7 +458,8 @@ static void kkt_pad_plan(const lqrb_context *h, const KktShape &s, int n2, int m
 
 static int32_t kkt_solve_padded(lqrb_context *h, const KktShape &s, int n2, int m2, int64_t batch, int flags,
                                 const double *data, double *scratch, double *dz, double *mult, double *res, int32_t *info,
-                                cudaStream_t st, KktRecord *record) {
+                                Lane lane, KktRecord *record) {
+    const cudaStream_t st = lane.stream;
     PadPlan P;
     kkt_pad_plan(h, s, n2, m2, batch, &P);
     const KktFamily family = kkt_route(h, P.s2, true).family;
@@ -494,7 +494,7 @@ static int32_t kkt_solve_padded(lqrb_context *h, const KktShape &s, int n2, int 
         int32_t rc = lqrb_gather_pack(h, md, src, cb, 1, data2, st);
         if (rc) return rc;
         rc = kkt_solve_tuned(h, family, P.s2, cb, flags, data2, scr2, dz2, mult2, res ? res2 : nullptr,
-                             info ? info + first : nullptr, st, record);
+                             info ? info + first : nullptr, lane, record);
         if (rc) return rc;
         ArrayTableOut o = {};
         o.ptr[0] = dz + first * z.NN;
@@ -531,23 +531,37 @@ static size_t kkt_scratch_bytes(const lqrb_context *h, const KktShape &s, const 
 
 static int32_t kkt_solve_on(lqrb_context *h, const KktShape &s, int64_t batch, int flags,
                             const double *data, double *scratch, double *dz, double *mult, double *res,
-                            int32_t *info, cudaStream_t st, KktRecord *record) {
+                            int32_t *info, Lane lane, KktRecord *record) {
     if (batch == 0) return 0;
     const KktRoute r = kkt_route(h, s, ((uintptr_t)data & 15) == 0);
     switch (r.family) {
     case KktFamily::Pad:
-        return kkt_solve_padded(h, s, r.n2, r.m2, batch, flags, data, scratch, dz, mult, res, info, st, record);
+        return kkt_solve_padded(h, s, r.n2, r.m2, batch, flags, data, scratch, dz, mult, res, info, lane, record);
     case KktFamily::Cta:
     case KktFamily::Wp:
     case KktFamily::Hw:
-        return kkt_solve_tuned(h, r.family, s, batch, flags, data, scratch, dz, mult, res, info, st, record);
+        return kkt_solve_tuned(h, r.family, s, batch, flags, data, scratch, dz, mult, res, info, lane, record);
     case KktFamily::Tpi:
-        return kkt_launch_tpi(h, s, batch, flags, data, scratch, dz, mult, res, info, st);
+        return kkt_launch_tpi(h, s, batch, flags, data, scratch, dz, mult, res, info, lane.stream);
     case KktFamily::Coop:
         break;
     }
     return launch_kkt_coop(h, s.n, s.m, s.N, s.p, s.hess, s.d2x, flags, batch, data, scratch, dz, mult, res,
-                           info, st);
+                           info, lane);
+}
+
+int32_t lqrb_kkt_solve_packed_on(lqrb_context *h, int n, int m, int N, int64_t batch, const int32_t *p, int hess_mode,
+                                 int explicit_d2, int flags, const double *data, double *dz, double *mult, double *res,
+                                 int32_t *info, Lane lane) {
+    const KktShape s = make_shape(n, m, N, p, hess_mode, explicit_d2);
+    const KktSizes z = kkt_sizes(s);
+    double *scratch = (double *)lqrb_scratch(h, SCR_FACT, kkt_scratch_bytes(h, s, z, batch), lane.index);
+    if (!scratch) return 1000 + (int)cudaErrorMemoryAllocation;
+    KktRecord record;
+    int32_t rc = kkt_solve_on(h, s, batch, flags, data, scratch, dz, mult, res, info, lane, &record);
+    if (rc) return rc;
+    kkt_keep_record(h, record);
+    return 0;
 }
 
 extern "C" int32_t lqrb_kkt_solve_packed_f64(lqrb_handle_t h, int32_t n, int32_t m, int32_t N,
@@ -560,15 +574,8 @@ extern "C" int32_t lqrb_kkt_solve_packed_f64(lqrb_handle_t h, int32_t n, int32_t
     if (!dz) return lqrb_fail(h, -12, "dz is NULL");
     if (!mult) return lqrb_fail(h, -13, "mult is NULL");
     LQRB_CUDA(h, cudaSetDevice(h->device));
-    const KktShape s = make_shape(n, m, N, p, hess_mode, explicit_d2);
-    const KktSizes z = kkt_sizes(s);
-    double *scratch = (double *)lqrb_scratch(h, SCR_FACT, kkt_scratch_bytes(h, s, z, batch));
-    if (!scratch) return 1000 + (int)cudaErrorMemoryAllocation;
-    KktRecord record;
-    rc = kkt_solve_on(h, s, batch, flags, data, scratch, dz, mult, res, info, h->stream, &record);
-    if (rc) return rc;
-    kkt_keep_record(h, record);
-    return 0;
+    return lqrb_kkt_solve_packed_on(h, n, m, N, batch, p, hess_mode, explicit_d2, flags, data, dz, mult, res, info,
+                                    Lane{h->stream, 0});
 }
 
 // ------------------------------------------------------------------ pack / unpack -------------
@@ -649,6 +656,27 @@ extern "C" int32_t lqrb_kkt_unpack_f64(lqrb_handle_t h, int32_t n, int32_t m, in
 }
 
 // ------------------------------------------------------------------ full call -----------------
+// The instance-major inputs of a KKT call (sources of kkt_data_map, NULL where absent) with their bytes per instance;
+// an absent Hux or D2 counts as 0 bytes.
+static std::vector<HostArray> kkt_inputs(const KktShape &s, const KktSizes &z, const double *const src[11]) {
+    const int64_t n = s.n, m = s.m, N = s.N, K1 = N - 1;
+    const int64_t per[11] = {n * n * N, m * m * K1, src[2] ? m * n * K1 : 0, n * N,  m * K1, n * n * K1,
+                             n * m * K1, n * K1,     src[8] ? z.sD2 : 0,     z.sC,   z.sc};
+    std::vector<HostArray> v(11);
+    for (int i = 0; i < 11; ++i) v[i] = {src[i], per[i] * 8};
+    return v;
+}
+
+// gather sources of one chunk: the driver's device pointers with the listed arrays' strides
+static ArrayTable kkt_array_table(const std::vector<HostArray> &inputs, const void *const *in) {
+    ArrayTable t = {};
+    for (size_t i = 0; i < inputs.size(); ++i) {
+        t.ptr[i] = (const double *)in[i];
+        t.stride[i] = inputs[i].bytes / 8;
+    }
+    return t;
+}
+
 extern "C" int32_t lqrb_kkt_solve_f64(lqrb_handle_t h, int32_t n, int32_t m, int32_t N, int64_t batch,
                                       const int32_t *p, int32_t hess_mode, int32_t flags,
                                       const double *Q, const double *R, const double *Hux,
@@ -666,88 +694,26 @@ extern "C" int32_t lqrb_kkt_solve_f64(lqrb_handle_t h, int32_t n, int32_t m, int
     const KktShape s = make_shape(n, m, N, p, hess_mode, D2 != nullptr);
     const KktSizes z = kkt_sizes(s);
     if (z.sC > 0 && (!C || !c)) return lqrb_fail(h, -18, "C/c is NULL but p has non-zero entries");
-    const int64_t K1 = N - 1;
-    const int64_t per[11] = {(int64_t)n * n * N, (int64_t)m * m * K1, Hux ? (int64_t)m * n * K1 : 0,
-                             (int64_t)n * N,     (int64_t)m * K1,     (int64_t)n * n * K1,
-                             (int64_t)n * m * K1, (int64_t)n * K1,    D2 ? z.sD2 : 0, z.sC, z.sc};
     const double *src[11] = {Q, R, Hux, q, r, A, B, d, D2, C, c};
-    const bool on_device = lqrb_is_device_ptr(Q);
-
-    if (on_device) {
-        const int64_t ldb = lqrb_padded_batch(batch);
-        double *data = (double *)lqrb_scratch(h, SCR_PACK_IN, (size_t)ldb * z.data_rows * 8);
-        double *dzp = (double *)lqrb_scratch(h, SCR_PACK_OUT, (size_t)ldb * z.NN * 8);
-        double *mp = (double *)lqrb_scratch(h, SCR_PACK_OUT2, (size_t)ldb * z.P * 8);
-        double *rp = res ? (double *)lqrb_scratch(h, SCR_PACK_OUT3, (size_t)ldb * z.NN * 8) : nullptr;
-        double *scr = (double *)lqrb_scratch(h, SCR_FACT, kkt_scratch_bytes(h, s, z, batch));
-        if (!data || !dzp || !mp || !scr || (res && !rp)) return 1000 + (int)cudaErrorMemoryAllocation;
-        rc = kkt_pack_on(h, s, z, batch, src, data, h->stream);
-        if (rc) return rc;
-        KktRecord record;
-        rc = kkt_solve_on(h, s, batch, flags, data, scr, dzp, mp, rp, info, h->stream, &record);
-        if (rc) return rc;
-        kkt_keep_record(h, record);
-        return kkt_unpack_on(h, s, z, batch, dzp, mp, rp, dz, mult, res, h->stream);
-    }
-
-    // ---- host buffers: chunked over two streams ----
-    int64_t in_per = 0;
-    for (int i = 0; i < 11; ++i) in_per += per[i];
-    int64_t chunk = h->opt("host_chunk", 0);
-    if (chunk <= 0) chunk = std::max<int64_t>(LQRB_TILE, (64ll << 20) / (in_per * 8) / LQRB_TILE * LQRB_TILE);
-    chunk = std::min<int64_t>(round_up(chunk, LQRB_TILE), lqrb_padded_batch(batch));
-    const int64_t out_per = z.NN + z.P + (res ? z.NN : 0);
-    const size_t in_bytes = (size_t)chunk * in_per * 8, out_bytes = (size_t)chunk * out_per * 8;
-    const size_t pk_bytes = (size_t)chunk * z.data_rows * 8;
-    const size_t po_bytes = (size_t)chunk * (2 * z.NN + z.P) * 8;
-    const size_t sc_bytes = (kkt_scratch_bytes(h, s, z, chunk) + 255) / 256 * 256;
-    char *stage_in = (char *)lqrb_scratch(h, SCR_STAGE_A, 2 * in_bytes);
-    char *stage_out = (char *)lqrb_scratch(h, SCR_STAGE_B, 2 * out_bytes);
-    char *pk = (char *)lqrb_scratch(h, SCR_PACK_IN, 2 * pk_bytes);
-    char *po = (char *)lqrb_scratch(h, SCR_PACK_OUT, 2 * po_bytes);
-    char *sc = (char *)lqrb_scratch(h, SCR_FACT, 2 * sc_bytes);
-    int32_t *dinfo = (int32_t *)lqrb_scratch(h, SCR_INFO, 2 * (size_t)chunk * sizeof(int32_t));
-    if (!stage_in || !stage_out || !pk || !po || !sc || !dinfo) return 1000 + (int)cudaErrorMemoryAllocation;
-
-    LQRB_CUDA(h, cudaEventRecord(h->ev[0], h->stream));
-    for (int i = 0; i < 2; ++i) LQRB_CUDA(h, cudaStreamWaitEvent(h->copy_stream[i], h->ev[0], 0));
     KktRecord record;
-    int which = 0;
-    for (int64_t first = 0; first < batch; first += chunk, which ^= 1) {
-        const int64_t cb = std::min(chunk, batch - first);
-        cudaStream_t st = h->copy_stream[which];
-        double *cur = (double *)(stage_in + which * in_bytes);
-        const double *dsrc[11];
-        for (int i = 0; i < 11; ++i) {
-            if (!src[i] || per[i] == 0) {
-                dsrc[i] = nullptr;
-                continue;
-            }
-            LQRB_CUDA(h, cudaMemcpyAsync(cur, src[i] + first * per[i], (size_t)cb * per[i] * 8,
-                                         cudaMemcpyHostToDevice, st));
-            dsrc[i] = cur;
-            cur += cb * per[i];
-        }
-        double *data = (double *)(pk + which * pk_bytes);
-        double *dzp = (double *)(po + which * po_bytes), *mp = dzp + chunk * z.NN, *rp = mp + chunk * z.P;
-        double *scr = (double *)(sc + which * sc_bytes);
-        int32_t *di = dinfo + which * chunk;
-        rc = kkt_pack_on(h, s, z, cb, dsrc, data, st);
-        if (rc) return rc;
-        rc = kkt_solve_on(h, s, cb, flags, data, scr, dzp, mp, res ? rp : nullptr, di, st, &record);
-        if (rc) return rc;
-        double *so = (double *)(stage_out + which * out_bytes);
-        double *odz = so, *om = odz + cb * z.NN, *ores = om + cb * z.P;
-        rc = kkt_unpack_on(h, s, z, cb, dzp, mp, rp, odz, om, res ? ores : nullptr, st);
-        if (rc) return rc;
-        LQRB_CUDA(h, cudaMemcpyAsync(dz + first * z.NN, odz, (size_t)cb * z.NN * 8, cudaMemcpyDeviceToHost, st));
-        LQRB_CUDA(h, cudaMemcpyAsync(mult + first * z.P, om, (size_t)cb * z.P * 8, cudaMemcpyDeviceToHost, st));
-        if (res)
-            LQRB_CUDA(h, cudaMemcpyAsync(res + first * z.NN, ores, (size_t)cb * z.NN * 8, cudaMemcpyDeviceToHost, st));
-        if (info)
-            LQRB_CUDA(h, cudaMemcpyAsync(info + first, di, (size_t)cb * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-    }
-    for (int i = 0; i < 2; ++i) LQRB_CUDA(h, cudaStreamSynchronize(h->copy_stream[i]));
+    rc = lqrb_for_chunks(
+        h, batch, 0, kkt_inputs(s, z, src), {{dz, z.NN * 8}, {mult, z.P * 8}, {res, z.NN * 8}, {info, 4}},
+        [&](Lane lane, int64_t cb, const void *const *in, void *const *out) -> int32_t {
+            const int64_t ldb = lqrb_padded_batch(cb);
+            double *data = (double *)lqrb_scratch(h, SCR_PACK_IN, (size_t)ldb * z.data_rows * 8, lane.index);
+            double *dzp = (double *)lqrb_scratch(h, SCR_PACK_OUT, (size_t)ldb * z.NN * 8, lane.index);
+            double *mp = (double *)lqrb_scratch(h, SCR_PACK_OUT2, (size_t)ldb * z.P * 8, lane.index);
+            double *rp = out[2] ? (double *)lqrb_scratch(h, SCR_PACK_OUT3, (size_t)ldb * z.NN * 8, lane.index) : nullptr;
+            double *scr = (double *)lqrb_scratch(h, SCR_FACT, kkt_scratch_bytes(h, s, z, cb), lane.index);
+            if (!data || !dzp || !mp || !scr || (out[2] && !rp)) return 1000 + (int)cudaErrorMemoryAllocation;
+            int32_t rc = kkt_pack_on(h, s, z, cb, (const double *const *)in, data, lane.stream);
+            if (rc) return rc;
+            rc = kkt_solve_on(h, s, cb, flags, data, scr, dzp, mp, rp, (int32_t *)out[3], lane, &record);
+            if (rc) return rc;
+            return kkt_unpack_on(h, s, z, cb, dzp, mp, rp, (double *)out[0], (double *)out[1], (double *)out[2],
+                                 lane.stream);
+        });
+    if (rc) return rc;
     kkt_keep_record(h, record);
     return 0;
 }
@@ -758,41 +724,6 @@ extern "C" int32_t lqrb_kkt_solve_f64(lqrb_handle_t h, int32_t n, int32_t m, int
 // runs the five steps of _solve! one by one (test/cholesky_solve.jl:14-35), re-using the factor for further
 // right-hand sides.  Here the handle owns ONE kept factorisation (packed matrices + the block rows of U in the
 // cooperative kernel's record layout, tile width 1); the fused kernels of lqrb_kkt_solve_f64 never touch it.
-
-// stage instance-major arrays on the device when they are host pointers; returns device pointers
-static int32_t stage_inputs(lqrb_context *h, int slot, int cnt, const double *const *src, const int64_t *per,
-                            int64_t batch, const double **dev, cudaStream_t st) {
-    bool host = false;
-    size_t total = 0;
-    for (int i = 0; i < cnt; ++i)
-        if (src[i] && per[i] > 0) {
-            if (!lqrb_is_device_ptr(src[i])) host = true;
-            total += (size_t)per[i] * batch;
-        }
-    if (!host) {
-        for (int i = 0; i < cnt; ++i) dev[i] = (src[i] && per[i] > 0) ? src[i] : nullptr;
-        return 0;
-    }
-    double *cur = (double *)lqrb_scratch(h, slot, total * 8);
-    if (!cur) return 1000 + (int)cudaErrorMemoryAllocation;
-    for (int i = 0; i < cnt; ++i) {
-        if (!src[i] || per[i] == 0) {
-            dev[i] = nullptr;
-            continue;
-        }
-        LQRB_CUDA(h, cudaMemcpyAsync(cur, src[i], (size_t)per[i] * batch * 8, cudaMemcpyDefault, st));
-        dev[i] = cur;
-        cur += per[i] * batch;
-    }
-    return 0;
-}
-
-static void kkt_per_instance(const KktShape &s, const KktSizes &z, bool has_hux, bool has_d2, int64_t per[11]) {
-    const int64_t n = s.n, m = s.m, N = s.N, K1 = N - 1;
-    const int64_t v[11] = {n * n * N, m * m * K1, has_hux ? m * n * K1 : 0, n * N,  m * K1, n * n * K1,
-                           n * m * K1, n * K1,     has_d2 ? z.sD2 : 0,     z.sC,   z.sc};
-    for (int i = 0; i < 11; ++i) per[i] = v[i];
-}
 
 // row map of the right-hand-side array of phase 2: per knot g (w) | d (p2) | c (ps); sources 0 q, 1 r, 2 d, 3 c
 static std::vector<RowMap> kkt_rhs_map(const KktShape &s) {
@@ -827,35 +758,24 @@ extern "C" int32_t lqrb_kkt_factor_f64(lqrb_handle_t h, int32_t n, int32_t m, in
     h->kept_key.clear();
     h->kept_batch = 0;
     if (batch == 0) return 0;
-    cudaStream_t st = h->stream;
-    int64_t per[11];
-    kkt_per_instance(s, z, Hux != nullptr, D2 != nullptr, per);
     // sources in kkt_data_map order: Q R Hux q r A B d D2 C c — the right-hand-side rows are filled with zeros
     const double *src[11] = {Q, R, Hux, nullptr, nullptr, A, B, nullptr, D2, C, nullptr};
-    const double *dev[11];
-    rc = stage_inputs(h, SCR_STAGE_A, 11, src, per, batch, dev, st);
+    const std::vector<HostArray> inputs = kkt_inputs(s, z, src);
+    rc = lqrb_for_chunks(h, batch, batch, inputs, {{info, 4}},
+                         [&](Lane lane, int64_t cb, const void *const *in, void *const *out) -> int32_t {
+                             double *data = (double *)lqrb_scratch(h, SCR_KEEP_DATA, (size_t)cb * z.data_rows * 8);
+                             double *rec = (double *)lqrb_scratch(h, SCR_KEEP_REC, (size_t)cb * z.rec_rows * 8);
+                             if (!data || !rec) return 1000 + (int)cudaErrorMemoryAllocation;
+                             const ArrayTable t = kkt_array_table(inputs, in);
+                             int32_t rc = lqrb_gather_pack(h, lqrb_get_map(h, shape_key("kd", s), kkt_data_map(s)), t,
+                                                           cb, 1, data, lane.stream);
+                             if (rc) return rc;
+                             KktCoopExtra ex;
+                             ex.phase = 1;
+                             return launch_kkt_coop(h, n, m, N, p, hess_mode, s.d2x, flags, cb, data, rec, nullptr,
+                                                    nullptr, nullptr, (int32_t *)out[0], lane, &ex);
+                         });
     if (rc) return rc;
-    double *data = (double *)lqrb_scratch(h, SCR_KEEP_DATA, (size_t)batch * z.data_rows * 8);
-    double *rec = (double *)lqrb_scratch(h, SCR_KEEP_REC, (size_t)batch * z.rec_rows * 8);
-    int32_t *dinfo = (int32_t *)lqrb_scratch(h, SCR_INFO, (size_t)batch * sizeof(int32_t));
-    if (!data || !rec || !dinfo) return 1000 + (int)cudaErrorMemoryAllocation;
-    ArrayTable t = {};
-    for (int i = 0; i < 11; ++i) {
-        t.ptr[i] = dev[i];
-        t.stride[i] = per[i];
-    }
-    rc = lqrb_gather_pack(h, lqrb_get_map(h, shape_key("kd", s), kkt_data_map(s)), t, batch, 1, data, st);
-    if (rc) return rc;
-    KktCoopExtra ex;
-    ex.phase = 1;
-    const bool info_dev = info && lqrb_is_device_ptr(info);
-    rc = launch_kkt_coop(h, n, m, N, p, hess_mode, s.d2x, flags, batch, data, rec, nullptr, nullptr, nullptr,
-                         info_dev ? info : dinfo, st, &ex);
-    if (rc) return rc;
-    if (info && !info_dev) {
-        LQRB_CUDA(h, cudaMemcpyAsync(info, dinfo, (size_t)batch * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-        LQRB_CUDA(h, cudaStreamSynchronize(st));
-    }
     h->kept_key = kept_key_of(s, flags);
     h->kept_batch = batch;
     return 0;
@@ -880,48 +800,25 @@ extern "C" int32_t lqrb_kkt_solve_factored_f64(lqrb_handle_t h, int32_t n, int32
     if (h->kept_key.empty() || h->kept_key != kept_key_of(s, flags) || h->kept_batch != batch)
         return lqrb_fail(h, -1, "no kept factorisation of this shape / batch / flags: call lqrb_kkt_factor_f64 first");
     if (batch == 0) return 0;
-    cudaStream_t st = h->stream;
-    const int64_t per[4] = {(int64_t)n * N, (int64_t)m * (N - 1), (int64_t)n * (N - 1), z.sc};
-    const double *src[4] = {q, r, d, c};
-    const double *dev[4];
-    rc = stage_inputs(h, SCR_STAGE_A, 4, src, per, batch, dev, st);
-    if (rc) return rc;
-    const int64_t rhs_rows = z.NN + z.P;
-    double *rhs = (double *)lqrb_scratch(h, SCR_PACK_IN2, (size_t)batch * rhs_rows * 8);
-    if (!rhs) return 1000 + (int)cudaErrorMemoryAllocation;
-    ArrayTable t = {};
-    for (int i = 0; i < 4; ++i) {
-        t.ptr[i] = dev[i];
-        t.stride[i] = per[i];
-    }
-    rc = lqrb_gather_pack(h, lqrb_get_map(h, shape_key("krhs", s), kkt_rhs_map(s)), t, batch, 1, rhs, st);
-    if (rc) return rc;
-    // tile width 1: the packed outputs ARE the instance-major arrays; host outputs go through a staging buffer
-    const bool out_dev = lqrb_is_device_ptr(dz);
-    double *odz = dz, *om = mult, *ores = res;
-    int32_t *oi = info;
-    if (!out_dev) {
-        odz = (double *)lqrb_scratch(h, SCR_STAGE_B, (size_t)batch * (2 * z.NN + z.P) * 8 + (size_t)batch * 4);
-        if (!odz) return 1000 + (int)cudaErrorMemoryAllocation;
-        om = odz + batch * z.NN;
-        ores = om + batch * z.P;
-        oi = reinterpret_cast<int32_t *>(ores + batch * z.NN);
-    }
-    KktCoopExtra ex;
-    ex.phase = 2;
-    ex.rhs = rhs;
-    rc = launch_kkt_coop(h, n, m, N, p, hess_mode, s.d2x, flags, batch, (const double *)h->scratch[SCR_KEEP_DATA],
-                         (double *)h->scratch[SCR_KEEP_REC], odz, om, (res || !out_dev) ? ores : nullptr,
-                         (info || !out_dev) ? oi : nullptr, st, &ex);
-    if (rc) return rc;
-    if (!out_dev) {
-        LQRB_CUDA(h, cudaMemcpyAsync(dz, odz, (size_t)batch * z.NN * 8, cudaMemcpyDeviceToHost, st));
-        LQRB_CUDA(h, cudaMemcpyAsync(mult, om, (size_t)batch * z.P * 8, cudaMemcpyDeviceToHost, st));
-        if (res) LQRB_CUDA(h, cudaMemcpyAsync(res, ores, (size_t)batch * z.NN * 8, cudaMemcpyDeviceToHost, st));
-        if (info) LQRB_CUDA(h, cudaMemcpyAsync(info, oi, (size_t)batch * 4, cudaMemcpyDeviceToHost, st));
-        LQRB_CUDA(h, cudaStreamSynchronize(st));
-    }
-    return 0;
+    const std::vector<HostArray> inputs = {
+        {q, (int64_t)n * N * 8}, {r, (int64_t)m * (N - 1) * 8}, {d, (int64_t)n * (N - 1) * 8}, {c, z.sc * 8}};
+    return lqrb_for_chunks(
+        h, batch, batch, inputs, {{dz, z.NN * 8}, {mult, z.P * 8}, {res, z.NN * 8}, {info, 4}},
+        [&](Lane lane, int64_t cb, const void *const *in, void *const *out) -> int32_t {
+            double *rhs = (double *)lqrb_scratch(h, SCR_PACK_IN2, (size_t)cb * (z.NN + z.P) * 8, lane.index);
+            if (!rhs) return 1000 + (int)cudaErrorMemoryAllocation;
+            const ArrayTable t = kkt_array_table(inputs, in);
+            int32_t rc = lqrb_gather_pack(h, lqrb_get_map(h, shape_key("krhs", s), kkt_rhs_map(s)), t, cb, 1, rhs,
+                                          lane.stream);
+            if (rc) return rc;
+            // tile width 1: the packed outputs ARE the instance-major arrays
+            KktCoopExtra ex;
+            ex.phase = 2;
+            ex.rhs = rhs;
+            return launch_kkt_coop(h, n, m, N, p, hess_mode, s.d2x, flags, cb, (const double *)h->scratch[SCR_KEEP_DATA][0],
+                                   (double *)h->scratch[SCR_KEEP_REC][0], (double *)out[0], (double *)out[1],
+                                   (double *)out[2], (int32_t *)out[3], lane, &ex);
+        });
 }
 
 // dense P x P image of the block rows (copy_shur_factors! / copy_block!, src/jacobian_blocks.jl:173-211):
@@ -972,54 +869,48 @@ extern "C" int32_t lqrb_kkt_get_shur_f64(lqrb_handle_t h, int32_t n, int32_t m, 
     const KktSizes z = kkt_sizes(s);
     if (z.sC > 0 && (!C || !c)) return lqrb_fail(h, -18, "C/c is NULL but p has non-zero entries");
     if (batch == 0) return 0;
-    cudaStream_t st = h->stream;
-    int64_t per[11];
-    kkt_per_instance(s, z, Hux != nullptr, D2 != nullptr, per);
     const double *src[11] = {Q, R, Hux, q, r, A, B, d, D2, C, c};
-    const double *dev[11];
-    rc = stage_inputs(h, SCR_STAGE_A, 11, src, per, batch, dev, st);
-    if (rc) return rc;
-    double *data = (double *)lqrb_scratch(h, SCR_PACK_IN, (size_t)batch * z.data_rows * 8);
-    double *rec = (double *)lqrb_scratch(h, SCR_FACT, (size_t)batch * z.rec_rows * 8);
-    double *sd = (double *)lqrb_scratch(h, SCR_PACK_OUT, (size_t)batch * z.rec_rows * 8);
-    double *out = (double *)lqrb_scratch(h, SCR_PACK_OUT2, (size_t)batch * (z.NN + z.P) * 8);
-    int32_t *dinfo = (int32_t *)lqrb_scratch(h, SCR_INFO, (size_t)batch * sizeof(int32_t));
-    if (!data || !rec || !sd || !out || !dinfo) return 1000 + (int)cudaErrorMemoryAllocation;
-    ArrayTable t = {};
-    for (int i = 0; i < 11; ++i) {
-        t.ptr[i] = dev[i];
-        t.stride[i] = per[i];
-    }
-    rc = lqrb_gather_pack(h, lqrb_get_map(h, shape_key("kd", s), kkt_data_map(s)), t, batch, 1, data, st);
-    if (rc) return rc;
-    LQRB_CUDA(h, cudaMemsetAsync(sd, 0, (size_t)batch * z.rec_rows * 8, st));
-    KktCoopExtra ex;
-    ex.phase = 0;
-    ex.sdump = sd;
-    rc = launch_kkt_coop(h, n, m, N, p, hess_mode, s.d2x, flags, batch, data, rec, out, out + batch * z.NN, nullptr,
-                         dinfo, st, &ex);
-    if (rc) return rc;
-    std::vector<double> hrec((size_t)z.rec_rows), hsd((size_t)z.rec_rows), dense((size_t)z.P * z.P), hv((size_t)z.P);
-    if (info) LQRB_CUDA(h, cudaMemcpyAsync(info, dinfo, (size_t)batch * 4, cudaMemcpyDefault, st));
-    for (int64_t i = 0; i < batch; ++i) {
-        LQRB_CUDA(h, cudaMemcpyAsync(hrec.data(), rec + i * z.rec_rows, (size_t)z.rec_rows * 8, cudaMemcpyDeviceToHost, st));
-        LQRB_CUDA(h, cudaMemcpyAsync(hsd.data(), sd + i * z.rec_rows, (size_t)z.rec_rows * 8, cudaMemcpyDeviceToHost, st));
-        LQRB_CUDA(h, cudaStreamSynchronize(st));
-        if (S || hvec) {
-            std::fill(dense.begin(), dense.end(), 0.0);
-            assemble_block_rows(s, hsd.data(), z.P, false, dense.data(), hv.data());
-            if (S) LQRB_CUDA(h, cudaMemcpy(S + i * z.P * z.P, dense.data(), (size_t)z.P * z.P * 8, cudaMemcpyDefault));
-            if (hvec) LQRB_CUDA(h, cudaMemcpy(hvec + i * z.P, hv.data(), (size_t)z.P * 8, cudaMemcpyDefault));
-        }
-        if (U) {
-            std::fill(dense.begin(), dense.end(), 0.0);
-            assemble_block_rows(s, hrec.data(), z.P, true, dense.data(), nullptr);
-            LQRB_CUDA(h, cudaMemcpy(U + i * z.P * z.P, dense.data(), (size_t)z.P * z.P * 8, cudaMemcpyDefault));
-        }
-    }
-    return 0;
+    const std::vector<HostArray> inputs = kkt_inputs(s, z, src);
+    // S, h and U are assembled on the host and written with cudaMemcpyDefault, whatever memory they are in
+    return lqrb_for_chunks(
+        h, batch, batch, inputs, {{info, 4}},
+        [&](Lane lane, int64_t cb, const void *const *in, void *const *out) -> int32_t {
+            const cudaStream_t st = lane.stream;
+            double *data = (double *)lqrb_scratch(h, SCR_PACK_IN, (size_t)cb * z.data_rows * 8, lane.index);
+            double *rec = (double *)lqrb_scratch(h, SCR_FACT, (size_t)cb * z.rec_rows * 8, lane.index);
+            double *sd = (double *)lqrb_scratch(h, SCR_PACK_OUT, (size_t)cb * z.rec_rows * 8, lane.index);
+            double *sol = (double *)lqrb_scratch(h, SCR_PACK_OUT2, (size_t)cb * (z.NN + z.P) * 8, lane.index);
+            if (!data || !rec || !sd || !sol) return 1000 + (int)cudaErrorMemoryAllocation;
+            const ArrayTable t = kkt_array_table(inputs, in);
+            int32_t rc = lqrb_gather_pack(h, lqrb_get_map(h, shape_key("kd", s), kkt_data_map(s)), t, cb, 1, data, st);
+            if (rc) return rc;
+            LQRB_CUDA(h, cudaMemsetAsync(sd, 0, (size_t)cb * z.rec_rows * 8, st));
+            KktCoopExtra ex;
+            ex.phase = 0;
+            ex.sdump = sd;
+            rc = launch_kkt_coop(h, n, m, N, p, hess_mode, s.d2x, flags, cb, data, rec, sol, sol + cb * z.NN, nullptr,
+                                 (int32_t *)out[0], lane, &ex);
+            if (rc) return rc;
+            std::vector<double> hrec((size_t)z.rec_rows), hsd((size_t)z.rec_rows), dense((size_t)z.P * z.P), hv((size_t)z.P);
+            for (int64_t i = 0; i < cb; ++i) {
+                LQRB_CUDA(h, cudaMemcpyAsync(hrec.data(), rec + i * z.rec_rows, (size_t)z.rec_rows * 8, cudaMemcpyDeviceToHost, st));
+                LQRB_CUDA(h, cudaMemcpyAsync(hsd.data(), sd + i * z.rec_rows, (size_t)z.rec_rows * 8, cudaMemcpyDeviceToHost, st));
+                LQRB_CUDA(h, cudaStreamSynchronize(st));
+                if (S || hvec) {
+                    std::fill(dense.begin(), dense.end(), 0.0);
+                    assemble_block_rows(s, hsd.data(), z.P, false, dense.data(), hv.data());
+                    if (S) LQRB_CUDA(h, cudaMemcpy(S + i * z.P * z.P, dense.data(), (size_t)z.P * z.P * 8, cudaMemcpyDefault));
+                    if (hvec) LQRB_CUDA(h, cudaMemcpy(hvec + i * z.P, hv.data(), (size_t)z.P * 8, cudaMemcpyDefault));
+                }
+                if (U) {
+                    std::fill(dense.begin(), dense.end(), 0.0);
+                    assemble_block_rows(s, hrec.data(), z.P, true, dense.data(), nullptr);
+                    LQRB_CUDA(h, cudaMemcpy(U + i * z.P * z.P, dense.data(), (size_t)z.P * z.P * 8, cudaMemcpyDefault));
+                }
+            }
+            return 0;
+        });
 }
-
 
 extern "C" int32_t lqrb_kkt_last_condition(lqrb_handle_t h, int64_t count, int32_t *log2_pivot_ratio, int64_t *resolved) {
     if (!h) return -1;

@@ -407,20 +407,9 @@ static int32_t get_tables(lqrb_context *h, int n, int m, int N, const int32_t *p
     return 0;
 }
 
-// Global-memory workspace of the cooperative kernel (used when the per-instance workspace does not fit in shared
-// memory).  The host-buffer path of lqrb_kkt_solve_f64 alternates chunks over the handle's two copy streams, so two
-// of these kernels can be in flight at once: every stream gets its own slice, sized for the largest grid the
-// launcher ever uses so that it never has to grow (= be freed) while the other stream's kernel is running.
-static double *coop_global_ws(lqrb_context *h, cudaStream_t st, size_t bytes_per_stream) {
-    bytes_per_stream = (bytes_per_stream + 255) / 256 * 256;
-    const int which = st == h->copy_stream[1] ? 2 : st == h->copy_stream[0] ? 1 : 0;
-    char *base = (char *)lqrb_scratch(h, SCR_MISC, 3 * bytes_per_stream);
-    return base ? (double *)(base + which * bytes_per_stream) : nullptr;
-}
-
 int32_t launch_kkt_coop(lqrb_context *h, int n, int m, int N, const int32_t *p, int hess, int d2x,
                         int flags, int64_t batch, const double *data, double *scratch, double *dz,
-                        double *mult, double *res, int32_t *info, cudaStream_t st, const KktCoopExtra *extra) {
+                        double *mult, double *res, int32_t *info, Lane lane, const KktCoopExtra *extra) {
     CoopTables tb;
     int32_t rc = get_tables(h, n, m, N, p, hess, d2x, &tb);
     if (rc) return rc;
@@ -454,13 +443,13 @@ int32_t launch_kkt_coop(lqrb_context *h, int n, int m, int N, const int32_t *p, 
                            : (G == 8 ? kkt_coop_kernel<8, THREADS> : (G == 16 ? kkt_coop_kernel<16, THREADS> : kkt_coop_kernel<32, THREADS>));
         if (smem > smem_cap) {
             grid = std::min<unsigned>(grid, (unsigned)h->sm_count * 8);  // instances are strided over the grid
-            a.gws = coop_global_ws(h, st, (size_t)h->sm_count * 8 * IPC * wsd * 8);
+            a.gws = (double *)lqrb_scratch(h, SCR_MISC, (size_t)h->sm_count * 8 * IPC * wsd * 8, lane.index);
             if (!a.gws) return 1000 + (int)cudaErrorMemoryAllocation;
             smem = 0;
         } else {
             LQRB_CUDA(h, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         }
-        kern<<<grid, THREADS, smem, st>>>(a);
+        kern<<<grid, THREADS, smem, lane.stream>>>(a);
         snprintf(nm, sizeof nm, "kkt_coop<G=%d>(n=%d,m=%d,%s)", G, n, m, a.gws ? "gmem-ws" : "smem-ws");
     } else {
         constexpr int G = 256, THREADS = 256;
@@ -468,13 +457,13 @@ int32_t launch_kkt_coop(lqrb_context *h, int n, int m, int N, const int32_t *p, 
         unsigned grid = (unsigned)std::min<int64_t>(batch, (int64_t)h->sm_count * 4);
         auto kern = kkt_coop_kernel<G, THREADS>;
         if (smem > smem_cap) {
-            a.gws = coop_global_ws(h, st, (size_t)h->sm_count * 4 * wsd * 8);
+            a.gws = (double *)lqrb_scratch(h, SCR_MISC, (size_t)h->sm_count * 4 * wsd * 8, lane.index);
             if (!a.gws) return 1000 + (int)cudaErrorMemoryAllocation;
             smem = 0;
         } else {
             LQRB_CUDA(h, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         }
-        kern<<<grid, THREADS, smem, st>>>(a);
+        kern<<<grid, THREADS, smem, lane.stream>>>(a);
         snprintf(nm, sizeof nm, "kkt_coop<G=256>(n=%d,m=%d,%s)", n, m, a.gws ? "gmem-ws" : "smem-ws");
     }
     h->kernel_name = nm;

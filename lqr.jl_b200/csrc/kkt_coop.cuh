@@ -35,7 +35,7 @@ struct KktCoopExtra {
 
 int32_t launch_kkt_coop(lqrb_context *h, int n, int m, int N, const int32_t *p, int hess, int d2x,
                         int flags, int64_t batch, const double *data, double *scratch, double *dz,
-                        double *mult, double *res, int32_t *info, cudaStream_t st,
+                        double *mult, double *res, int32_t *info, Lane lane,
                         const KktCoopExtra *extra = nullptr);
 
 // device copies of the per-shape tables (cached on the handle): p[N], and N + 1 prefix offsets of the knot records in the

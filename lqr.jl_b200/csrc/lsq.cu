@@ -107,44 +107,21 @@ extern "C" int32_t lqrb_lsq_solve_f64(lqrb_handle_t h, int32_t n, int32_t m, int
     if (!Z) return lqrb_fail(h, -12, "Z is NULL");
     if (batch == 0) return 0;
     LQRB_CUDA(h, cudaSetDevice(h->device));
-    cudaStream_t st = h->stream;
     const int64_t NN = lqrb_num_vars(n, m, N);
-    const int64_t per[6] = {(int64_t)n * n, (int64_t)n * m, (int64_t)n * n, (int64_t)m * m, (int64_t)n * n, n};
-    const double *src[6] = {A, B, Q, R, Qf, x0};
-    const double *dev[6];
-    const bool on_dev = lqrb_is_device_ptr(A);
-    if (on_dev) {
-        for (int i = 0; i < 6; ++i) dev[i] = src[i];
-    } else {
-        int64_t tot = 0;
-        for (int i = 0; i < 6; ++i) tot += per[i];
-        double *cur = (double *)lqrb_scratch(h, SCR_STAGE_A, (size_t)tot * batch * 8);
-        if (!cur) return 1000 + (int)cudaErrorMemoryAllocation;
-        for (int i = 0; i < 6; ++i) {
-            LQRB_CUDA(h, cudaMemcpyAsync(cur, src[i], (size_t)per[i] * batch * 8, cudaMemcpyHostToDevice, st));
-            dev[i] = cur;
-            cur += per[i] * batch;
-        }
-    }
-    double *dZ = Z;
-    int32_t *dinfo = info;
-    if (!on_dev) {
-        dZ = (double *)lqrb_scratch(h, SCR_STAGE_B, (size_t)batch * NN * 8 + (size_t)batch * 4);
-        if (!dZ) return 1000 + (int)cudaErrorMemoryAllocation;
-        dinfo = reinterpret_cast<int32_t *>(dZ + batch * NN);
-    }
-    constexpr int THREADS = 256;
-    const unsigned grid = (unsigned)std::min<int64_t>(batch, (int64_t)h->sm_count * 2);
-    double *ws = (double *)lqrb_scratch(h, SCR_MISC, (size_t)grid * lsq_ws_doubles(n, m, N) * 8);
-    if (!ws) return 1000 + (int)cudaErrorMemoryAllocation;
-    lsq_solve_kernel<THREADS><<<grid, THREADS, 0, st>>>(dev[0], dev[1], dev[2], dev[3], dev[4], dev[5], dZ,
-                                                       (info || !on_dev) ? dinfo : nullptr, ws, n, m, N, batch);
-    h->kernel_name = "lsq_solve(condensed least squares)";
-    LQRB_LAUNCH_CHECK(h, "lsq_solve_kernel");
-    if (!on_dev) {
-        LQRB_CUDA(h, cudaMemcpyAsync(Z, dZ, (size_t)batch * NN * 8, cudaMemcpyDeviceToHost, st));
-        if (info) LQRB_CUDA(h, cudaMemcpyAsync(info, dinfo, (size_t)batch * 4, cudaMemcpyDeviceToHost, st));
-        LQRB_CUDA(h, cudaStreamSynchronize(st));
-    }
-    return 0;
+    const int64_t nn = (int64_t)n * n * 8, nm = (int64_t)n * m * 8, mm = (int64_t)m * m * 8;
+    return lqrb_for_chunks(
+        h, batch, batch, {{A, nn}, {B, nm}, {Q, nn}, {R, mm}, {Qf, nn}, {x0, (int64_t)n * 8}}, {{Z, NN * 8}, {info, 4}},
+        [&](Lane lane, int64_t cb, const void *const *in, void *const *out) -> int32_t {
+            constexpr int THREADS = 256;
+            const unsigned grid = (unsigned)std::min<int64_t>(cb, (int64_t)h->sm_count * 2);
+            double *ws = (double *)lqrb_scratch(h, SCR_MISC, (size_t)grid * lsq_ws_doubles(n, m, N) * 8, lane.index);
+            if (!ws) return 1000 + (int)cudaErrorMemoryAllocation;
+            const double *const *a = (const double *const *)in;
+            lsq_solve_kernel<THREADS><<<grid, THREADS, 0, lane.stream>>>(a[0], a[1], a[2], a[3], a[4], a[5],
+                                                                         (double *)out[0], (int32_t *)out[1], ws, n, m, N,
+                                                                         cb);
+            h->kernel_name = "lsq_solve(condensed least squares)";
+            LQRB_LAUNCH_CHECK(h, "lsq_solve_kernel");
+            return 0;
+        });
 }

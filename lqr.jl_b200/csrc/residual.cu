@@ -140,55 +140,29 @@ extern "C" int32_t lqrb_kkt_residual_f64(lqrb_handle_t h, int32_t n, int32_t m, 
     a.p = (const int32_t *)(blob + 2 * off_bytes);
     a.n = n; a.m = m; a.N = N; a.grad = grad ? 1 : 0;
     a.NN = NN; a.P = P; a.sC = sC; a.sD2 = sD2;
-    constexpr int THREADS = 128;
-
-    if (lqrb_is_device_ptr(A)) {
-        a.q = q; a.r = r; a.A = A; a.B = B; a.D2 = D2; a.C = sC > 0 ? C : nullptr; a.mult = mult;
-        a.res = res; a.norms = norms; a.batch = batch;
-        kkt_residual_kernel<THREADS><<<(unsigned)batch, THREADS, 0, h->stream>>>(a);
-        LQRB_LAUNCH_CHECK(h, "kkt_residual_kernel");
-        h->kernel_name = "kkt_residual";
-        return 0;
-    }
-
-    // ---- host buffers: staged in instance chunks (a diagnostic path: synchronous) ----
-    const int64_t per[7] = {grad ? (int64_t)n * N : 0, grad ? (int64_t)m * K1 : 0, (int64_t)n * n * K1,
-                            (int64_t)n * m * K1,       D2 ? sD2 : 0,               sC, P};
+    // bytes per instance; the staged chunks hold about 256 MB of input plus output (or `host_chunk` instances)
+    const int64_t per[7] = {grad ? (int64_t)n * N * 8 : 0, grad ? (int64_t)m * K1 * 8 : 0, (int64_t)n * n * K1 * 8,
+                            (int64_t)n * m * K1 * 8,       D2 ? sD2 * 8 : 0,               sC * 8, P * 8};
     const double *src[7] = {q, r, A, B, D2, C, mult};
-    int64_t in_per = 0;
-    for (int i = 0; i < 7; ++i) in_per += per[i];
-    const int64_t out_per = NN + 1;
-    int64_t chunk = std::max<int64_t>(1, (256ll << 20) / ((in_per + out_per) * 8));
-    chunk = std::min(chunk, batch);
-    double *stage = (double *)lqrb_scratch(h, SCR_STAGE_A, (size_t)chunk * in_per * 8);
-    double *outb = (double *)lqrb_scratch(h, SCR_STAGE_B, (size_t)chunk * out_per * 8);
-    if (!stage || !outb) return 1000 + (int)cudaErrorMemoryAllocation;
-    for (int64_t first = 0; first < batch; first += chunk) {
-        const int64_t cb = std::min(chunk, batch - first);
-        double *cur = stage;
-        const double *dsrc[7];
-        for (int i = 0; i < 7; ++i) {
-            if (!src[i] || per[i] == 0) {
-                dsrc[i] = nullptr;
-                continue;
-            }
-            LQRB_CUDA(h, cudaMemcpyAsync(cur, src[i] + first * per[i], (size_t)cb * per[i] * 8,
-                                         cudaMemcpyHostToDevice, h->stream));
-            dsrc[i] = cur;
-            cur += cb * per[i];
-        }
-        a.q = dsrc[0]; a.r = dsrc[1]; a.A = dsrc[2]; a.B = dsrc[3]; a.D2 = dsrc[4]; a.C = dsrc[5]; a.mult = dsrc[6];
-        a.res = outb;
-        a.norms = outb + cb * NN;
-        a.batch = cb;
-        kkt_residual_kernel<THREADS><<<(unsigned)cb, THREADS, 0, h->stream>>>(a);
-        LQRB_LAUNCH_CHECK(h, "kkt_residual_kernel");
-        if (res)
-            LQRB_CUDA(h, cudaMemcpyAsync(res + first * NN, outb, (size_t)cb * NN * 8, cudaMemcpyDeviceToHost, h->stream));
-        if (norms)
-            LQRB_CUDA(h, cudaMemcpyAsync(norms + first, outb + cb * NN, (size_t)cb * 8, cudaMemcpyDeviceToHost, h->stream));
-        LQRB_CUDA(h, cudaStreamSynchronize(h->stream));
+    std::vector<HostArray> inputs(7);
+    int64_t io_bytes = (NN + 1) * 8;
+    for (int i = 0; i < 7; ++i) {
+        inputs[i] = {src[i], per[i]};
+        io_bytes += per[i];
     }
-    h->kernel_name = "kkt_residual";
-    return 0;
+    int64_t chunk = h->opt("host_chunk", 0);
+    if (chunk <= 0) chunk = std::max<int64_t>(1, (256ll << 20) / io_bytes);
+    return lqrb_for_chunks(h, batch, chunk, inputs, {{res, NN * 8}, {norms, 8}},
+                           [&](Lane lane, int64_t cb, const void *const *in, void *const *out) -> int32_t {
+                               constexpr int THREADS = 128;
+                               const double *const *d = (const double *const *)in;
+                               a.q = d[0]; a.r = d[1]; a.A = d[2]; a.B = d[3]; a.D2 = d[4]; a.C = d[5]; a.mult = d[6];
+                               a.res = (double *)out[0];
+                               a.norms = (double *)out[1];
+                               a.batch = cb;
+                               kkt_residual_kernel<THREADS><<<(unsigned)cb, THREADS, 0, lane.stream>>>(a);
+                               LQRB_LAUNCH_CHECK(h, "kkt_residual_kernel");
+                               h->kernel_name = "kkt_residual";
+                               return 0;
+                           });
 }

@@ -255,11 +255,11 @@ static RiccatiPadMaps riccati_pad_maps(int n, int m, int N, int Kn, int n2, int 
 }
 
 static int32_t riccati_solve_on(lqrb_context *h, int n, int m, int N, int64_t batch, int flags, const double *knots,
-                                const double *term, double *Z, double *gains, int32_t *info, cudaStream_t s);
+                                const double *term, double *Z, double *gains, int32_t *info, Lane lane);
 
 static int32_t riccati_solve_padded(lqrb_context *h, int n, int m, int N, int n2, int m2, int64_t batch, int flags,
                                     const double *knots, const double *term, double *Z, double *gains, int32_t *info,
-                                    cudaStream_t st) {
+                                    Lane lane) {
     const int Kn = (flags & LQRB_FLAG_LTI) ? 1 : N - 1;
     const int64_t F = lqrb_riccati_knot_rows(n, m), F2 = lqrb_riccati_knot_rows(n2, m2);
     const int64_t TR = tri(n) + 2 * n, TR2 = tri(n2) + 2 * n2;
@@ -280,12 +280,12 @@ static int32_t riccati_solve_padded(lqrb_context *h, int n, int m, int N, int n2
         mg = h->maps[k0 + ":g"];
     }
     if (mk.rows != Kn * F2 || mt.rows != TR2 || mz.rows != ZR2 || mg.rows != GR2) return lqrb_fail(h, 1, "pad map size mismatch");
-    // chunks of at most ~2 GB of padded arrays; one allocation per stream (the host path has two in flight)
+    // chunks of at most ~2 GB of padded arrays
     const int64_t per = Kn * F2 + TR2 + ZR2 + GR2;
     int64_t chunk = std::max<int64_t>(LQRB_TILE, ((int64_t)2 << 30) / (per * 8) / LQRB_TILE * LQRB_TILE);
     chunk = std::min(chunk, lqrb_padded_batch(batch));
     const size_t slice = ((size_t)chunk * per * 8 + 255) / 256 * 256;
-    char *base = (char *)lqrb_scratch(h, st == h->copy_stream[1] ? SCR_RICCATI_PAD_B : SCR_RICCATI_PAD, slice);
+    char *base = (char *)lqrb_scratch(h, SCR_RICCATI_PAD, slice, lane.index);
     if (!base) return 1000 + (int)cudaErrorMemoryAllocation;
     double *knots2 = (double *)base, *term2 = knots2 + chunk * Kn * F2, *Z2 = term2 + chunk * TR2, *gains2 = Z2 + chunk * ZR2;
     std::string name;
@@ -294,23 +294,23 @@ static int32_t riccati_solve_padded(lqrb_context *h, int n, int m, int N, int n2
         ArrayTable src = {};
         src.ptr[0] = knots + first * Kn * F;
         src.stride[0] = Kn * F;
-        int32_t rc = lqrb_gather_pack(h, mk, src, cb, 1, knots2, st);
+        int32_t rc = lqrb_gather_pack(h, mk, src, cb, 1, knots2, lane.stream);
         if (rc) return rc;
         src.ptr[0] = term + first * TR;
         src.stride[0] = TR;
-        rc = lqrb_gather_pack(h, mt, src, cb, 1, term2, st);
+        rc = lqrb_gather_pack(h, mt, src, cb, 1, term2, lane.stream);
         if (rc) return rc;
-        rc = riccati_solve_on(h, n2, m2, N, cb, flags, knots2, term2, Z2, gains2, info ? info + first : nullptr, st);
+        rc = riccati_solve_on(h, n2, m2, N, cb, flags, knots2, term2, Z2, gains2, info ? info + first : nullptr, lane);
         if (rc) return rc;
         name = h->kernel_name;
         ArrayTableOut o = {};
         o.ptr[0] = Z + first * ZR;
         o.stride[0] = ZR;
-        rc = lqrb_scatter_unpack(h, mz, o, cb, 1, Z2, st);
+        rc = lqrb_scatter_unpack(h, mz, o, cb, 1, Z2, lane.stream);
         if (rc) return rc;
         o.ptr[0] = gains + first * GR;
         o.stride[0] = GR;
-        rc = lqrb_scatter_unpack(h, mg, o, cb, 1, gains2, st);
+        rc = lqrb_scatter_unpack(h, mg, o, cb, 1, gains2, lane.stream);
         if (rc) return rc;
     }
     char nm[64];
@@ -321,13 +321,14 @@ static int32_t riccati_solve_padded(lqrb_context *h, int n, int m, int N, int n2
 
 static int32_t riccati_solve_on(lqrb_context *h, int n, int m, int N, int64_t batch, int flags,
                                 const double *knots, const double *term, double *Z, double *gains,
-                                int32_t *info, cudaStream_t s) {
+                                int32_t *info, Lane lane) {
     if (batch == 0) return 0;
     {
         int n2, m2;
         if (((uintptr_t)knots & 15) == 0 && riccati_pad_target(h, n, m, &n2, &m2))
-            return riccati_solve_padded(h, n, m, N, n2, m2, batch, flags, knots, term, Z, gains, info, s);
+            return riccati_solve_padded(h, n, m, N, n2, m2, batch, flags, knots, term, Z, gains, info, lane);
     }
+    const cudaStream_t s = lane.stream;
     const int lti = (flags & LQRB_FLAG_LTI) ? 1 : 0;
     const int tile = lqrb_riccati_tile(h, n, m);
     if (tile == LQRB_TILE) {
@@ -367,7 +368,7 @@ extern "C" int32_t lqrb_riccati_solve_packed_f64(lqrb_handle_t h, int32_t n, int
         gains = (double *)lqrb_scratch(h, SCR_GAINS, bytes);
         if (!gains) return 1000 + (int)cudaErrorMemoryAllocation;
     }
-    return riccati_solve_on(h, n, m, N, batch, flags, knots, term, Z, gains, info, h->stream);
+    return riccati_solve_on(h, n, m, N, batch, flags, knots, term, Z, gains, info, Lane{h->stream, 0});
 }
 
 // ------------------------------------------------------------------ pack (device) -------------
@@ -475,98 +476,29 @@ extern "C" int32_t lqrb_riccati_f64(lqrb_handle_t h, int32_t n, int32_t m, int32
 
     lqrb_riccati_layout_t L;
     lqrb_riccati_layout(n, m, N, flags, &L);
-    const int64_t Kn = L.knot_count;
-    const bool on_device = lqrb_is_device_ptr(A);
-
-    // per-instance record lengths of the instance-major arrays
-    const int64_t sA = Kn * n * n, sB = Kn * n * m, sQ = Kn * n * n, sR = Kn * m * m, sq = Kn * n,
-                  sr = Kn * m, sQf = (int64_t)n * n;
-    const int64_t in_per = sA + sB + sQ + sR + sq + sr + sQf + 2 * n;
-    const int64_t NN = L.z_rows, GRN = L.gain_rows;
-
-    if (on_device) {
-        const int64_t ldb = lqrb_padded_batch(batch);
-        double *knots = (double *)lqrb_scratch(h, SCR_PACK_IN, (size_t)ldb * Kn * L.rows_per_knot * 8);
-        double *term = (double *)lqrb_scratch(h, SCR_PACK_IN2, (size_t)ldb * L.term_rows * 8);
-        double *Zp = (double *)lqrb_scratch(h, SCR_PACK_OUT, (size_t)ldb * NN * 8);
-        double *gains = (double *)lqrb_scratch(h, SCR_GAINS, (size_t)ldb * GRN * 8);
-        if (!knots || !term || !Zp || !gains) return 1000 + (int)cudaErrorMemoryAllocation;
-        rc = riccati_pack_on(h, n, m, N, batch, flags, A, B, Q, R, q, r, Qf, qf, x0, knots, term, h->stream);
-        if (rc) return rc;
-        rc = riccati_solve_on(h, n, m, N, batch, flags, knots, term, Zp, gains, info, h->stream);
-        if (rc) return rc;
-        return riccati_unpack_on(h, n, m, N, batch, Zp, gains, Z, K, kff, h->stream);
-    }
-
-    // ---- host buffers: chunked H2D -> pack -> solve -> unpack -> D2H over two streams ----
-    int64_t chunk = h->opt("host_chunk", 0);
-    if (chunk <= 0) {
-        // ~64 MB of input per chunk keeps both copy engines and the SMs busy
-        chunk = std::max<int64_t>(LQRB_TILE, (64ll << 20) / (in_per * 8) / LQRB_TILE * LQRB_TILE);
-    }
-    chunk = std::min<int64_t>(round_up(chunk, LQRB_TILE), lqrb_padded_batch(batch));
-    const int64_t out_per = NN + ((K || kff) ? GRN : 0);
-    const size_t in_bytes = (size_t)chunk * in_per * 8, out_bytes = (size_t)chunk * out_per * 8;
-    const size_t pk_bytes = (size_t)chunk * (Kn * L.rows_per_knot + L.term_rows) * 8;
-    const size_t po_bytes = (size_t)chunk * (NN + GRN) * 8;
-    char *stage_in = (char *)lqrb_scratch(h, SCR_STAGE_A, 2 * in_bytes);
-    char *stage_out = (char *)lqrb_scratch(h, SCR_STAGE_B, 2 * out_bytes);
-    char *pk = (char *)lqrb_scratch(h, SCR_PACK_IN, 2 * pk_bytes);
-    char *po = (char *)lqrb_scratch(h, SCR_PACK_OUT, 2 * po_bytes);
-    int32_t *dinfo = (int32_t *)lqrb_scratch(h, SCR_INFO, 2 * (size_t)chunk * sizeof(int32_t));
-    if (!stage_in || !stage_out || !pk || !po || !dinfo) return 1000 + (int)cudaErrorMemoryAllocation;
-
-    LQRB_CUDA(h, cudaEventRecord(h->ev[0], h->stream));
-    for (int i = 0; i < 2; ++i) LQRB_CUDA(h, cudaStreamWaitEvent(h->copy_stream[i], h->ev[0], 0));
-
-    int which = 0;
-    for (int64_t first = 0; first < batch; first += chunk, which ^= 1) {
-        const int64_t cb = std::min(chunk, batch - first);
-        cudaStream_t s = h->copy_stream[which];
-        double *si = (double *)(stage_in + which * in_bytes);
-        // carve the instance-major stage
-        double *dA = si, *dB = dA + cb * sA, *dQ = dB + cb * sB, *dR = dQ + cb * sQ,
-               *dq = dR + cb * sR, *dr = dq + cb * sq, *dQf = dr + cb * sr, *dqf = dQf + cb * sQf,
-               *dx0 = dqf + cb * n;
-        auto h2d = [&](double *dst, const double *src, int64_t per) -> cudaError_t {
-            if (!src) return cudaMemsetAsync(dst, 0, (size_t)cb * per * 8, s);
-            return cudaMemcpyAsync(dst, src + first * per, (size_t)cb * per * 8, cudaMemcpyHostToDevice, s);
-        };
-        LQRB_CUDA(h, h2d(dA, A, sA));
-        LQRB_CUDA(h, h2d(dB, B, sB));
-        LQRB_CUDA(h, h2d(dQ, Q, sQ));
-        LQRB_CUDA(h, h2d(dR, R, sR));
-        LQRB_CUDA(h, h2d(dq, q, sq));
-        LQRB_CUDA(h, h2d(dr, r, sr));
-        LQRB_CUDA(h, h2d(dQf, Qf, sQf));
-        LQRB_CUDA(h, h2d(dqf, qf, n));
-        LQRB_CUDA(h, h2d(dx0, x0, n));
-        double *knots = (double *)(pk + which * pk_bytes);
-        double *term = knots + chunk * Kn * L.rows_per_knot;
-        double *Zp = (double *)(po + which * po_bytes);
-        double *gains = Zp + chunk * NN;
-        int32_t *di = dinfo + which * chunk;
-        rc = riccati_pack_on(h, n, m, N, cb, flags, dA, dB, dQ, dR, dq, dr, dQf, dqf, dx0, knots, term, s);
-        if (rc) return rc;
-        rc = riccati_solve_on(h, n, m, N, cb, flags, knots, term, Zp, gains, di, s);
-        if (rc) return rc;
-        double *so = (double *)(stage_out + which * out_bytes);
-        double *oZ = so, *oK = so + cb * NN, *okff = oK + cb * (int64_t)(N - 1) * m * n;
-        rc = riccati_unpack_on(h, n, m, N, cb, Zp, gains, oZ, K ? oK : nullptr, kff ? okff : nullptr, s);
-        if (rc) return rc;
-        LQRB_CUDA(h, cudaMemcpyAsync(Z + first * NN, oZ, (size_t)cb * NN * 8, cudaMemcpyDeviceToHost, s));
-        if (K)
-            LQRB_CUDA(h, cudaMemcpyAsync(K + first * (int64_t)(N - 1) * m * n, oK,
-                                         (size_t)cb * (N - 1) * m * n * 8, cudaMemcpyDeviceToHost, s));
-        if (kff)
-            LQRB_CUDA(h, cudaMemcpyAsync(kff + first * (int64_t)(N - 1) * m, okff,
-                                         (size_t)cb * (N - 1) * m * 8, cudaMemcpyDeviceToHost, s));
-        if (info)
-            LQRB_CUDA(h, cudaMemcpyAsync(info + first, di, (size_t)cb * sizeof(int32_t),
-                                         cudaMemcpyDeviceToHost, s));
-    }
-    for (int i = 0; i < 2; ++i) LQRB_CUDA(h, cudaStreamSynchronize(h->copy_stream[i]));
-    return 0;
+    const int64_t Kn = L.knot_count, NN = L.z_rows, GRN = L.gain_rows;
+    // bytes per instance of the instance-major arrays (q, r and qf count when absent too: they fix the chunk size)
+    const int64_t sA = Kn * n * n * 8, sB = Kn * n * m * 8, sR = Kn * m * m * 8, sq = Kn * n * 8, sr = Kn * m * 8,
+                  sQf = (int64_t)n * n * 8, sx = (int64_t)n * 8;
+    return lqrb_for_chunks(
+        h, batch, 0, {{A, sA}, {B, sB}, {Q, sA}, {R, sR}, {q, sq}, {r, sr}, {Qf, sQf}, {qf, sx}, {x0, sx}},
+        {{Z, NN * 8}, {K, (int64_t)(N - 1) * m * n * 8}, {kff, (int64_t)(N - 1) * m * 8}, {info, 4}},
+        [&](Lane lane, int64_t cb, const void *const *in, void *const *out) -> int32_t {
+            const int64_t ldb = lqrb_padded_batch(cb);
+            double *knots = (double *)lqrb_scratch(h, SCR_PACK_IN, (size_t)ldb * Kn * L.rows_per_knot * 8, lane.index);
+            double *term = (double *)lqrb_scratch(h, SCR_PACK_IN2, (size_t)ldb * L.term_rows * 8, lane.index);
+            double *Zp = (double *)lqrb_scratch(h, SCR_PACK_OUT, (size_t)ldb * NN * 8, lane.index);
+            double *gains = (double *)lqrb_scratch(h, SCR_GAINS, (size_t)ldb * GRN * 8, lane.index);
+            if (!knots || !term || !Zp || !gains) return 1000 + (int)cudaErrorMemoryAllocation;
+            const double *const *a = (const double *const *)in;
+            int32_t rc = riccati_pack_on(h, n, m, N, cb, flags, a[0], a[1], a[2], a[3], a[4], a[5], a[6], a[7], a[8],
+                                         knots, term, lane.stream);
+            if (rc) return rc;
+            rc = riccati_solve_on(h, n, m, N, cb, flags, knots, term, Zp, gains, (int32_t *)out[3], lane);
+            if (rc) return rc;
+            return riccati_unpack_on(h, n, m, N, cb, Zp, gains, (double *)out[0], (double *)out[1], (double *)out[2],
+                                     lane.stream);
+        });
 }
 
 // ------------------------------------------------------------------ rollout -------------------
@@ -643,32 +575,22 @@ extern "C" int32_t lqrb_rollout_f64(lqrb_handle_t h, int32_t n, int32_t m, int32
     LQRB_CUDA(h, cudaSetDevice(h->device));
     const int lti = (flags & LQRB_FLAG_LTI) ? 1 : 0;
     const int64_t Kn = lti ? 1 : N - 1;
-    const bool dev = lqrb_is_device_ptr(A);
-    const double *dA = A, *dB = B, *dx0 = x0, *dU = U;
-    double *dX = X;
-    if (!dev) {
-        const size_t tot = (size_t)batch * (Kn * n * n + Kn * n * m + n + (N - 1) * m + (size_t)N * n) * 8;
-        double *buf = (double *)lqrb_scratch(h, SCR_STAGE_A, tot);
-        if (!buf) return 1000 + (int)cudaErrorMemoryAllocation;
-        double *a = buf, *b = a + batch * Kn * n * n, *x = b + batch * Kn * n * m, *u = x + batch * n;
-        dX = u + batch * (int64_t)(N - 1) * m;
-        LQRB_CUDA(h, cudaMemcpyAsync(a, A, (size_t)batch * Kn * n * n * 8, cudaMemcpyHostToDevice, h->stream));
-        LQRB_CUDA(h, cudaMemcpyAsync(b, B, (size_t)batch * Kn * n * m * 8, cudaMemcpyHostToDevice, h->stream));
-        LQRB_CUDA(h, cudaMemcpyAsync(x, x0, (size_t)batch * n * 8, cudaMemcpyHostToDevice, h->stream));
-        LQRB_CUDA(h, cudaMemcpyAsync(u, U, (size_t)batch * (N - 1) * m * 8, cudaMemcpyHostToDevice, h->stream));
-        dA = a; dB = b; dx0 = x; dU = u;
-    }
-    if (n <= 32) {
-        rollout_warp_kernel<<<(unsigned)((batch + 3) / 4), 128, 0, h->stream>>>(dA, dB, dx0, dU, dX, n, m, N, lti, batch);
-        h->kernel_name = "rollout_warp";
-    } else {
-        rollout_kernel<<<(unsigned)((batch + 127) / 128), 128, 0, h->stream>>>(dA, dB, dx0, dU, dX, n, m, N, lti, batch);
-        h->kernel_name = "rollout_tpi";
-    }
-    LQRB_LAUNCH_CHECK(h, "rollout_kernel");
-    if (!dev) {
-        LQRB_CUDA(h, cudaMemcpyAsync(X, dX, (size_t)batch * N * n * 8, cudaMemcpyDeviceToHost, h->stream));
-        LQRB_CUDA(h, cudaStreamSynchronize(h->stream));
-    }
-    return 0;
+    return lqrb_for_chunks(
+        h, batch, batch, {{A, Kn * n * n * 8}, {B, Kn * n * m * 8}, {x0, (int64_t)n * 8}, {U, (int64_t)(N - 1) * m * 8}},
+        {{X, (int64_t)N * n * 8}},
+        [&](Lane lane, int64_t cb, const void *const *in, void *const *out) -> int32_t {
+            const double *const *a = (const double *const *)in;
+            double *dX = (double *)out[0];
+            if (n <= 32) {
+                rollout_warp_kernel<<<(unsigned)((cb + 3) / 4), 128, 0, lane.stream>>>(a[0], a[1], a[2], a[3], dX, n, m,
+                                                                                       N, lti, cb);
+                h->kernel_name = "rollout_warp";
+            } else {
+                rollout_kernel<<<(unsigned)((cb + 127) / 128), 128, 0, lane.stream>>>(a[0], a[1], a[2], a[3], dX, n, m,
+                                                                                      N, lti, cb);
+                h->kernel_name = "rollout_tpi";
+            }
+            LQRB_LAUNCH_CHECK(h, "rollout_kernel");
+            return 0;
+        });
 }

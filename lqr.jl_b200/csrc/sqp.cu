@@ -849,8 +849,6 @@ extern "C" int32_t lqrb_sqp_dubins_f64(lqrb_handle_t h, int64_t batch, const lqr
     p[0] = n;
     p[N - 1] = n;
     const int64_t drows = lqrb_kkt_data_rows(n, m, N, p.data(), LQRB_HESS_DIAG, 0);
-    const bool dev = lqrb_is_device_ptr(Z);
-    cudaStream_t s = h->stream;
 
     // fused (default): the KKT kernel linearises each knot on the fly; sqp_fused = 0 keeps the three-kernel
     // path (linearise -> packed data -> generic KKT solve) that it is tested against
@@ -868,124 +866,103 @@ extern "C" int32_t lqrb_sqp_dubins_f64(lqrb_handle_t h, int64_t batch, const lqr
     double *Zp = buf, *dz = Zp + ldb * NN, *dzh = dz + ldb * NN, *mult = dzh + ldb * NN, *multh = mult + ldb * P,
            *multk = multh + ldb * P, *x0p = multk + ldb * P, *xfp = x0p + ldb * n, *stats = xfp + ldb * n;
 
-    // stage the instance-major inputs and pack them
-    const double *dZ = Z, *dx0 = x0, *dxf = xf;
-    double *stage = nullptr;
-    if (!dev) {
-        stage = (double *)lqrb_scratch(h, SCR_STAGE_A, (size_t)batch * (NN + 2 * n) * 8 + (size_t)batch * 24);
-        if (!stage) return 1000 + (int)cudaErrorMemoryAllocation;
-        LQRB_CUDA(h, cudaMemcpyAsync(stage, Z, (size_t)batch * NN * 8, cudaMemcpyHostToDevice, s));
-        LQRB_CUDA(h, cudaMemcpyAsync(stage + batch * NN, x0, (size_t)batch * n * 8, cudaMemcpyHostToDevice, s));
-        LQRB_CUDA(h, cudaMemcpyAsync(stage + batch * (NN + n), xf, (size_t)batch * n * 8, cudaMemcpyHostToDevice, s));
-        dZ = stage;
-        dx0 = stage + batch * NN;
-        dxf = stage + batch * (NN + n);
-    }
-    ArrayTable t = {};
-    t.ptr[0] = dZ; t.stride[0] = NN;
-    int32_t rc = lqrb_gather_pack(h, lqrb_identity_map(h, NN), t, batch, LQRB_TILE, Zp, s);
-    if (rc) return rc;
-    t.ptr[0] = dx0; t.stride[0] = n;
-    rc = lqrb_gather_pack(h, lqrb_identity_map(h, n), t, batch, LQRB_TILE, x0p, s);
-    if (rc) return rc;
-    t.ptr[0] = dxf;
-    rc = lqrb_gather_pack(h, lqrb_identity_map(h, n), t, batch, LQRB_TILE, xfp, s);
-    if (rc) return rc;
-    LQRB_CUDA(h, cudaMemsetAsync(multk, 0, (size_t)ldb * P * 8, s));
-
-    const Opts o{N, opts->dt, opts->q_diag, opts->r_diag, opts->qf_diag};
-    const unsigned grid = (unsigned)((batch + 63) / 64);
-    stats_init_kernel<<<grid, 64, 0, s>>>(stats, batch);
-    LQRB_LAUNCH_CHECK(h, "stats_init_kernel");
+    // Z is updated in place; the scratch above belongs to lane 0, where a call in one chunk runs
     int64_t solves = 0;
-    int hc[2];
-    for (int it = 0; it < opts->iters; ++it) {
-        // update! + convergence check (:126-137)
-        if (fused) {
-            // update! + convergence check + _solve! + line-search stage 0 in one kernel
-            LQRB_CUDA(h, cudaMemsetAsync(counters, 0, 8, s));
-            // the cp.async ring measured SLOWER than the L2 prefetch (config 4: 23.9 vs 18.7 ms, same box): option only
-            if (h->opt("sqp_prefetch", 0))
-                dubins_sqp_step_pf_kernel<<<grid, 64, 0, s>>>(Zp, x0p, xfp, multk, data, frec, dz, dinfo, stats, o, batch,
-                                                                 opts->eps_p, opts->eps_d, opts->line_search ? 0 : 1, counters);
-            else
-                dubins_sqp_step_kernel<<<grid, 64, 0, s>>>(Zp, x0p, xfp, multk, data, frec, dz, dinfo, stats, o, batch,
-                                                                  opts->eps_p, opts->eps_d, opts->line_search ? 0 : 1, counters);
-            h->kernel_name = "dubins_sqp_step<3,2,p=3/0/3,hess=2>";
-            LQRB_LAUNCH_CHECK(h, "dubins_sqp_step_kernel");
-        } else {
-            dubins_linearize_kernel<true><<<grid, 64, 0, s>>>(Zp, x0p, xfp, multk, data, stats, o, batch, 1, opts->eps_p, opts->eps_d);
-            LQRB_LAUNCH_CHECK(h, "dubins_linearize_kernel");
-            // _solve! (:143)
-            rc = lqrb_kkt_solve_packed_f64(h, n, m, N, batch, p.data(), LQRB_HESS_DIAG, 0, 0, data, dz, mult, nullptr, dinfo);
+    const int32_t rc = lqrb_for_chunks(
+        h, batch, batch, {{Z, NN * 8}, {x0, n * 8}, {xf, n * 8}}, {{Z, NN * 8}, {feas_p, 8}, {feas_d, 8}, {iters_done, 4}},
+        [&](Lane lane, int64_t, const void *const *in, void *const *out) -> int32_t {
+            const cudaStream_t s = lane.stream;
+            ArrayTable t = {};
+            t.ptr[0] = (const double *)in[0]; t.stride[0] = NN;
+            int32_t rc = lqrb_gather_pack(h, lqrb_identity_map(h, NN), t, batch, LQRB_TILE, Zp, s);
             if (rc) return rc;
-        }
-        solves += batch;
-        // line search (:146; spec src/sqp.jl:72-94)
-        if (!fused) {
-            LQRB_CUDA(h, cudaMemsetAsync(counters, 0, 8, s));
-            dubins_linesearch_kernel<false><<<grid, 64, 0, s>>>(Zp, dz, nullptr, mult, multk, x0p, xfp, data, stats, o, batch, 0,
-                                                                opts->line_search ? 0 : 1, counters);
-            LQRB_LAUNCH_CHECK(h, "dubins_linesearch_kernel");
-        }
-        if (!opts->line_search) continue;
-        LQRB_CUDA(h, cudaMemcpyAsync(hc, counters, 8, cudaMemcpyDeviceToHost, s));
-        LQRB_CUDA(h, cudaStreamSynchronize(s));
-        if (hc[0] == 0) continue;
-        // second-order correction: same chain with Ginv=false on c(x+dx) (:254-273)
-        if (fused) {
-            dubins_kkt_fused_kernel<true><<<grid, 64, 0, s>>>(Zp, x0p, xfp, data, frec, dzh, multh, dinfo, o, batch);
-            LQRB_LAUNCH_CHECK(h, "dubins_kkt_fused_kernel");
-        } else {
-            rc = lqrb_kkt_solve_packed_f64(h, n, m, N, batch, p.data(), LQRB_HESS_DIAG, 0, LQRB_FLAG_SOC, data, dzh, multh,
-                                           nullptr, dinfo);
+            t.ptr[0] = (const double *)in[1]; t.stride[0] = n;
+            rc = lqrb_gather_pack(h, lqrb_identity_map(h, n), t, batch, LQRB_TILE, x0p, s);
             if (rc) return rc;
-        }
-        solves += batch;
-        int pending = hc[0];
-        // trial 1 = the SOC step; trials 2..10 = the reference's back-tracking iterations i = 2..10 (alpha = rho^1..rho^9,
-        // src/sqp.jl:76-92)
-        for (int trial = 1; trial < 11 && pending > 0; ++trial) {
-            LQRB_CUDA(h, cudaMemsetAsync(counters, 0, 8, s));
-            if (fused)
-                dubins_linesearch_kernel<true><<<grid, 64, 0, s>>>(Zp, dz, dzh, mult, multk, x0p, xfp, data, stats, o, batch,
-                                                                   trial == 1 ? 1 : 2, 0, counters);
-            else
-                dubins_linesearch_kernel<false><<<grid, 64, 0, s>>>(Zp, dz, dzh, mult, multk, x0p, xfp, data, stats, o, batch,
-                                                                    trial == 1 ? 1 : 2, 0, counters);
-            LQRB_LAUNCH_CHECK(h, "dubins_linesearch_kernel");
-            LQRB_CUDA(h, cudaMemcpyAsync(hc, counters, 8, cudaMemcpyDeviceToHost, s));
-            LQRB_CUDA(h, cudaStreamSynchronize(s));
-            pending = hc[1];
-        }
-    }
-    // final feasibility numbers at the returned iterate
-    dubins_linearize_kernel<false><<<grid, 64, 0, s>>>(Zp, x0p, xfp, multk, nullptr, stats, o, batch, 0, opts->eps_p, opts->eps_d);
-    LQRB_LAUNCH_CHECK(h, "dubins_linearize_kernel");
+            t.ptr[0] = (const double *)in[2];
+            rc = lqrb_gather_pack(h, lqrb_identity_map(h, n), t, batch, LQRB_TILE, xfp, s);
+            if (rc) return rc;
+            LQRB_CUDA(h, cudaMemsetAsync(multk, 0, (size_t)ldb * P * 8, s));
 
-    // export
-    double *oZ = Z, *ofp = feas_p, *ofd = feas_d;
-    int32_t *oit = iters_done;
-    if (!dev) {
-        oZ = stage;
-        ofp = stage + batch * NN;
-        ofd = ofp + batch;
-        oit = (int32_t *)(ofd + batch);
-    }
-    ArrayTableOut to = {};
-    to.ptr[0] = oZ; to.stride[0] = NN;
-    rc = lqrb_scatter_unpack(h, lqrb_identity_map(h, NN), to, batch, LQRB_TILE, Zp, s);
+            const Opts o{N, opts->dt, opts->q_diag, opts->r_diag, opts->qf_diag};
+            const unsigned grid = (unsigned)((batch + 63) / 64);
+            stats_init_kernel<<<grid, 64, 0, s>>>(stats, batch);
+            LQRB_LAUNCH_CHECK(h, "stats_init_kernel");
+            int hc[2];
+            for (int it = 0; it < opts->iters; ++it) {
+                // update! + convergence check (:126-137)
+                if (fused) {
+                    // update! + convergence check + _solve! + line-search stage 0 in one kernel
+                    LQRB_CUDA(h, cudaMemsetAsync(counters, 0, 8, s));
+                    // the cp.async ring measured SLOWER than the L2 prefetch (config 4: 23.9 vs 18.7 ms, same box): option only
+                    if (h->opt("sqp_prefetch", 0))
+                        dubins_sqp_step_pf_kernel<<<grid, 64, 0, s>>>(Zp, x0p, xfp, multk, data, frec, dz, dinfo, stats, o, batch,
+                                                                         opts->eps_p, opts->eps_d, opts->line_search ? 0 : 1, counters);
+                    else
+                        dubins_sqp_step_kernel<<<grid, 64, 0, s>>>(Zp, x0p, xfp, multk, data, frec, dz, dinfo, stats, o, batch,
+                                                                          opts->eps_p, opts->eps_d, opts->line_search ? 0 : 1, counters);
+                    h->kernel_name = "dubins_sqp_step<3,2,p=3/0/3,hess=2>";
+                    LQRB_LAUNCH_CHECK(h, "dubins_sqp_step_kernel");
+                } else {
+                    dubins_linearize_kernel<true><<<grid, 64, 0, s>>>(Zp, x0p, xfp, multk, data, stats, o, batch, 1, opts->eps_p, opts->eps_d);
+                    LQRB_LAUNCH_CHECK(h, "dubins_linearize_kernel");
+                    // _solve! (:143)
+                    rc = lqrb_kkt_solve_packed_on(h, n, m, N, batch, p.data(), LQRB_HESS_DIAG, 0, 0, data, dz, mult, nullptr, dinfo, lane);
+                    if (rc) return rc;
+                }
+                solves += batch;
+                // line search (:146; spec src/sqp.jl:72-94)
+                if (!fused) {
+                    LQRB_CUDA(h, cudaMemsetAsync(counters, 0, 8, s));
+                    dubins_linesearch_kernel<false><<<grid, 64, 0, s>>>(Zp, dz, nullptr, mult, multk, x0p, xfp, data, stats, o, batch, 0,
+                                                                        opts->line_search ? 0 : 1, counters);
+                    LQRB_LAUNCH_CHECK(h, "dubins_linesearch_kernel");
+                }
+                if (!opts->line_search) continue;
+                LQRB_CUDA(h, cudaMemcpyAsync(hc, counters, 8, cudaMemcpyDeviceToHost, s));
+                LQRB_CUDA(h, cudaStreamSynchronize(s));
+                if (hc[0] == 0) continue;
+                // second-order correction: same chain with Ginv=false on c(x+dx) (:254-273)
+                if (fused) {
+                    dubins_kkt_fused_kernel<true><<<grid, 64, 0, s>>>(Zp, x0p, xfp, data, frec, dzh, multh, dinfo, o, batch);
+                    LQRB_LAUNCH_CHECK(h, "dubins_kkt_fused_kernel");
+                } else {
+                    rc = lqrb_kkt_solve_packed_on(h, n, m, N, batch, p.data(), LQRB_HESS_DIAG, 0, LQRB_FLAG_SOC, data, dzh, multh,
+                                                  nullptr, dinfo, lane);
+                    if (rc) return rc;
+                }
+                solves += batch;
+                int pending = hc[0];
+                // trial 1 = the SOC step; trials 2..10 = the reference's back-tracking iterations i = 2..10 (alpha = rho^1..rho^9,
+                // src/sqp.jl:76-92)
+                for (int trial = 1; trial < 11 && pending > 0; ++trial) {
+                    LQRB_CUDA(h, cudaMemsetAsync(counters, 0, 8, s));
+                    if (fused)
+                        dubins_linesearch_kernel<true><<<grid, 64, 0, s>>>(Zp, dz, dzh, mult, multk, x0p, xfp, data, stats, o, batch,
+                                                                           trial == 1 ? 1 : 2, 0, counters);
+                    else
+                        dubins_linesearch_kernel<false><<<grid, 64, 0, s>>>(Zp, dz, dzh, mult, multk, x0p, xfp, data, stats, o, batch,
+                                                                            trial == 1 ? 1 : 2, 0, counters);
+                    LQRB_LAUNCH_CHECK(h, "dubins_linesearch_kernel");
+                    LQRB_CUDA(h, cudaMemcpyAsync(hc, counters, 8, cudaMemcpyDeviceToHost, s));
+                    LQRB_CUDA(h, cudaStreamSynchronize(s));
+                    pending = hc[1];
+                }
+            }
+            // final feasibility numbers at the returned iterate
+            dubins_linearize_kernel<false><<<grid, 64, 0, s>>>(Zp, x0p, xfp, multk, nullptr, stats, o, batch, 0, opts->eps_p, opts->eps_d);
+            LQRB_LAUNCH_CHECK(h, "dubins_linearize_kernel");
+
+            // export
+            ArrayTableOut to = {};
+            to.ptr[0] = (double *)out[0]; to.stride[0] = NN;
+            rc = lqrb_scatter_unpack(h, lqrb_identity_map(h, NN), to, batch, LQRB_TILE, Zp, s);
+            if (rc) return rc;
+            stats_export_kernel<<<grid, 64, 0, s>>>(stats, (double *)out[1], (double *)out[2], (int32_t *)out[3], batch);
+            LQRB_LAUNCH_CHECK(h, "stats_export_kernel");
+            return 0;
+        });
     if (rc) return rc;
-    stats_export_kernel<<<grid, 64, 0, s>>>(stats, (feas_p || !dev) ? ofp : nullptr, (feas_d || !dev) ? ofd : nullptr,
-                                            (iters_done || !dev) ? oit : nullptr, batch);
-    LQRB_LAUNCH_CHECK(h, "stats_export_kernel");
-    if (!dev) {
-        LQRB_CUDA(h, cudaMemcpyAsync(Z, oZ, (size_t)batch * NN * 8, cudaMemcpyDeviceToHost, s));
-        if (feas_p) LQRB_CUDA(h, cudaMemcpyAsync(feas_p, ofp, (size_t)batch * 8, cudaMemcpyDeviceToHost, s));
-        if (feas_d) LQRB_CUDA(h, cudaMemcpyAsync(feas_d, ofd, (size_t)batch * 8, cudaMemcpyDeviceToHost, s));
-        if (iters_done) LQRB_CUDA(h, cudaMemcpyAsync(iters_done, oit, (size_t)batch * 4, cudaMemcpyDeviceToHost, s));
-        LQRB_CUDA(h, cudaStreamSynchronize(s));
-    }
     if (kkt_solves) *kkt_solves = solves;
     return 0;
 }
