@@ -163,8 +163,10 @@ template <int n, int m>
 static int32_t launch_dmma(lqrb_context *h, int N, int64_t batch, int lti, const double *knots,
                            const double *term, double *Z, double *gains, int32_t *info,
                            cudaStream_t s) {
-    // 3 stages x 4 warps: 34 KB per CTA -> 6 CTAs = 24 warps per SM (<= 85 registers per thread)
-    constexpr int STAGES = 3, WARPS = 4, MINB = 6;
+    // 3 stages x 4 warps: 34 KB per CTA -> 6 CTAs = 24 warps per SM (<= 85 registers per thread).  m >= 2 takes 5
+    // CTAs = 20 warps (<= 102 registers): the LDL' of the control block needs more live values, and at 85 registers
+    // it spilled in the knot loop (5a-R +6 %); with 5 CTAs nothing spills and 5a-R is as fast as before.
+    constexpr int STAGES = 3, WARPS = 4, MINB = m == 1 ? 6 : 5;
     const size_t smem = rdmma::riccati_dmma_warp_smem(rdmma::Map<n, m>::F, STAGES) * WARPS;
     auto kern = rdmma::riccati_dmma_kernel<n, m, STAGES, WARPS, MINB>;
     LQRB_CUDA(h, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));

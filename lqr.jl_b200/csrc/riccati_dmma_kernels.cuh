@@ -91,8 +91,11 @@ struct Map {
     __host__ __device__ static constexpr int kperm(int s, int q) { return s == 0 ? 2 * q : s == 1 ? 2 * q + 1 : 8 + q; }
 };
 
-// per-warp shared memory: STAGES knot records | 184 doubles of staging (backward: control block with
-// duplicated rows/columns; forward: [x;u] double buffer + one knot of gains) | STAGES mbarriers
+// per-warp shared memory: STAGES knot records | 184 doubles of staging (backward: control block, the
+// lanes' right-hand sides and a zero row, laid out below; forward: [x;u] double buffer + one knot of gains)
+// | STAGES mbarriers.  The backward layout keeps row stride 8: Qd uses 4 of its 8 rows and gud 4 of its 8
+// entries.  Packing it tighter would save 40 doubles per warp and change nothing else: registers, not
+// shared memory, limit the CTAs per SM.
 #define RDMMA_AUX 184
 __host__ __device__ inline size_t riccati_dmma_warp_smem(int F, int stages) {
     return ((size_t)stages * F * 8 + RDMMA_AUX * 8 + (size_t)stages * 8 + 15) / 16 * 16;
@@ -111,7 +114,8 @@ __device__ __forceinline__ double fast_rcp(double x) {
 // The same seed (20 bits, measured: tools/ubench/rcp_test.cu) with ONE third-order step r (1 + e + e^2),
 // e = 1 - x r: three dependent FMAs instead of four, within one ulp of the correctly rounded quotient.  For the
 // serial 8 x 8 pivot chains of the CTA kernels, where the reciprocal is on the critical path of the whole CTA
-// (5b-K: -2 %; no gain, or a small loss, in the warp-level kernels, which keep fast_rcp).
+// (5b-K: -2 %), and for the m dependent pivots of riccati_dmma's control block (5a-R: about 1 % against
+// fast_rcp).  The other warp-level kernels keep fast_rcp: no gain there, or a small loss.
 __device__ __forceinline__ double fast_rcp3(double x) {
     double r;
     asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(r) : "d"(x));
@@ -120,62 +124,44 @@ __device__ __forceinline__ double fast_rcp3(double x) {
     return fma(r, t, r);
 }
 
-// Row 0 of the inverse of the SPD m x m control block a (upper triangle read) by 2 x 2 block elimination:
-// two dependent reciprocals instead of four dependent rsqrt.  Each quad lane q calls this on the block
-// cyclically permuted by q, so "row 0" is its own row q and nothing has to be selected afterwards.
-// info: index of the first non-positive Cholesky pivot (pivots: a00, detA/a00, s00, detS/s00), potrf
-// semantics; meaningful for the unpermuted lane q = 0.
+// Row q of the inverse of the SPD m x m control block a (upper triangle read), factored as L D L' in the
+// natural pivot order: L y = e_q, then L' x = D^-1 y.  Every quad lane factors the same block in the same
+// order, so the m rows the quad applies to [Mux | gu] belong to one factorisation.  That is what keeps the
+// gains within a small factor of the reference's chol_solve! when two cheap actuators act almost alike:
+// the right-hand sides then lie along the large eigenvectors of Muu, and only rows of one factorisation
+// cancel the huge entries of its inverse.  The former form (each lane's row by 2 x 2 adjugate/determinant
+// blocks of the block cyclically shifted by its own control) reached relative errors of 17 where the
+// reference order's error is 3e-9 (n = 12, m = 4, tests/test_gpu_riccati_conditioning.py).
+// Pivots d_j are potrf's squared Cholesky pivots; only their reciprocals (fast_rcp3) enter the result.
+// info: index of the first non-positive pivot (potrf semantics), the same in every lane.
 template <int m>
-__device__ __forceinline__ int spd_inv_row0(const double (&a)[4][4], double (&mi)[4]) {
+__device__ __forceinline__ int spd_inv_row(double (&a)[4][4], int q, double (&mi)[4]) {
     int info = 0;
-    if constexpr (m == 1) {
-        if (!(a[0][0] > 0.0)) info = 1;
-        mi[0] = fast_rcp(a[0][0]);
-    } else {
-        const double detA = fma(a[0][0], a[1][1], -a[0][1] * a[0][1]);
-        if (!(a[0][0] > 0.0)) info = 1;
-        else if (!(detA > 0.0)) info = 2;
-        const double rA = fast_rcp(detA);
-        const double i00 = a[1][1] * rA, i01 = -a[0][1] * rA, i11 = a[0][0] * rA;
-        if constexpr (m == 2) {
-            mi[0] = i00;
-            mi[1] = i01;
-        } else {
-            constexpr int r = m - 2;
-            double X[2][2], S[2][2];
+    double l[4][4], r[4];  // l[i][j] = a(j)[j][i] / d_j for i > j: the multipliers of pivot j; r[j] = 1 / d_j
+    SM_UNROLL
+    for (int j = 0; j < m; ++j) {
+        if (info == 0 && !(a[j][j] > 0.0)) info = j + 1;
+        r[j] = fast_rcp3(a[j][j]);
+        SM_UNROLL
+        for (int i = j + 1; i < m; ++i) l[i][j] = a[j][i] * r[j];
+        SM_UNROLL
+        for (int i = j + 1; i < m; ++i)
             SM_UNROLL
-            for (int j = 0; j < r; ++j) {
-                X[0][j] = fma(i00, a[0][2 + j], i01 * a[1][2 + j]);
-                X[1][j] = fma(i01, a[0][2 + j], i11 * a[1][2 + j]);
-            }
-            SM_UNROLL
-            for (int i = 0; i < r; ++i)
-                SM_UNROLL
-                for (int j = i; j < r; ++j)
-                    S[i][j] = a[2 + i][2 + j] - fma(a[0][2 + i], X[0][j], a[1][2 + i] * X[1][j]);
-            double y0, y1 = 0.0;
-            if constexpr (r == 1) {
-                if (info == 0 && !(S[0][0] > 0.0)) info = 3;
-                y0 = -X[0][0] * fast_rcp(S[0][0]);
-            } else {
-                const double detS = fma(S[0][0], S[1][1], -S[0][1] * S[0][1]);
-                if (info == 0 && !(S[0][0] > 0.0)) info = 3;
-                else if (info == 0 && !(detS > 0.0)) info = 4;
-                const double rS = fast_rcp(detS);
-                // -X[0][:] * S^-1,  S^-1 = rS * [S11 -S01; -S01 S00]
-                y0 = -rS * fma(X[0][0], S[1][1], -X[0][1] * S[0][1]);
-                y1 = -rS * fma(X[0][1], S[0][0], -X[0][0] * S[0][1]);
-            }
-            double m00 = fma(-y0, X[0][0], i00), m01 = fma(-y0, X[1][0], i01);
-            if constexpr (r == 2) {
-                m00 = fma(-y1, X[0][1], m00);
-                m01 = fma(-y1, X[1][1], m01);
-            }
-            mi[0] = m00;
-            mi[1] = m01;
-            mi[2] = y0;
-            if constexpr (r == 2) mi[3] = y1;
-        }
+            for (int k = i; k < m; ++k) a[i][k] = fma(-l[i][j], a[j][k], a[i][k]);
+    }
+    SM_UNROLL
+    for (int i = 0; i < m; ++i) {  // L y = e_q
+        double s = q == i ? 1.0 : 0.0;
+        SM_UNROLL
+        for (int j = 0; j < i; ++j) s = fma(-l[i][j], mi[j], s);
+        mi[i] = s;
+    }
+    SM_UNROLL
+    for (int i = m - 1; i >= 0; --i) {  // L' x = D^-1 y
+        double s = mi[i] * r[i];
+        SM_UNROLL
+        for (int j = i + 1; j < m; ++j) s = fma(-l[j][i], mi[j], s);
+        mi[i] = s;
     }
     return info;
 }
@@ -198,7 +184,7 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
     double *buf = reinterpret_cast<double *>(wbase);             // STAGES records
     double *aux = buf + (size_t)STAGES * F;                      // RDMMA_AUX doubles
     uint64_t *full = reinterpret_cast<uint64_t *>(aux + RDMMA_AUX);  // STAGES mbarriers
-    // backward-pass staging (doubles): V0d[8][8] | Qd[8][8] | V1e[4][8] | gud[8] | G1e[4] | zero[8]
+    // backward-pass staging (doubles): V0d[8][8] | Qd[8][8] (4 rows used) | V1e[4][8] | gud[8] (4 used) | G1e[4] | zero[8]
     double *V0d = aux, *Qd = aux + 64, *V1e = aux + 128, *gud = aux + 160, *G1e = aux + 168, *zero = aux + 172;
     // forward-pass staging
     double *zs = aux, *gs = aux + 32;
@@ -244,10 +230,9 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
     // gain store offsets: K0 -> K[q, x_g]; K1 -> K[q, x_{8+g/2}] (g even) or kff[q] (g == 1)
     const int go0 = q < m ? q + m * g : -1;
     const int go1 = q < m ? (odd ? (g == 1 ? m * n + q : -1) : (HAS_X1 && 8 + g / 2 < n ? q + m * (8 + g / 2) : -1)) : -1;
-    // control-block staging: this lane's permuted read bases (cyclic shift by q: row 0 = control q)
-    const int qq = q < m ? q : 0;
-    const double *rQ = Qd + 9 * qq, *rgu = gud + qq, *rv0 = V0d + 8 * g + qq;
-    const double *rv1 = (!odd) ? V1e + 8 * (g >> 1) + qq : ((g == 1 && q < m) ? gud + qq : zero);
+    // control-block staging: every lane reads the whole block and its own two right-hand sides
+    const double *rv0 = V0d + 8 * g;
+    const double *rv1 = (!odd) ? V1e + 8 * (g >> 1) : ((g == 1 && q < m) ? gud : zero);
     const double *rt10 = g == 1 ? G1e + q : zero;
     // selection fragments of the transposing MMAs (scaled by 1/2 for the symmetrisation)
     const double hsel0 = g == 2 * q ? 0.5 : 0.0, hsel1 = g == 2 * q + 1 ? 0.5 : 0.0;
@@ -337,31 +322,22 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
             const double gh0 = T[0][1][1] + qr0;
             const double gh1 = T[1][1][1] + qr1;
 
-            // ---- stage the control columns (rows/columns duplicated with period m so that lane q reads
-            // the block cyclically shifted by q with immediate offsets)
+            // ---- stage the control columns
             if (q < m) {
                 V0d[8 * g + q] = M01[1];  // Mxu[x_g][u_q]
-                V0d[8 * g + q + m] = M01[1];
-                if (!odd) {
-                    V1e[8 * (g >> 1) + q] = M11[1];  // Mxu[x_{8+g/2}][u_q]
-                    V1e[8 * (g >> 1) + q + m] = M11[1];
-                } else if (su < m) {
-                    Qd[8 * su + q] = M11[1];  // Quu[su][q]
-                    Qd[8 * su + q + m] = M11[1];
-                    Qd[8 * (su + m) + q] = M11[1];
-                    Qd[8 * (su + m) + q + m] = M11[1];
-                }
+                if (!odd) V1e[8 * (g >> 1) + q] = M11[1];  // Mxu[x_{8+g/2}][u_q]
+                else if (su < m) Qd[8 * su + q] = M11[1];  // Quu[su][q]
             }
             if (q == 0) {
                 if (!odd) G1e[g >> 1] = gh1;
-                else if (su < m) { gud[su] = gh1; gud[su + m] = gh1; }
+                else if (su < m) gud[su] = gh1;
             }
             __syncwarp();
             double a[4][4], v0[4], v1[4];
             SM_UNROLL
             for (int s = 0; s < m; ++s)
                 SM_UNROLL
-                for (int t = s; t < m; ++t) a[s][t] = rQ[8 * s + t];
+                for (int t = s; t < m; ++t) a[s][t] = Qd[8 * s + t];
             SM_UNROLL
             for (int t = 0; t < m; ++t) {
                 v0[t] = rv0[t];
@@ -369,7 +345,7 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
             }
             const double t10 = rt10[0];
             double mi[4];
-            const int ci = spd_inv_row0<m>(a, mi);  // chol_solve! :28-31 (E^-1 applied by multiplication)
+            const int ci = spd_inv_row<m>(a, q, mi);  // chol_solve! :28-31 (E^-1 applied by multiplication)
             if (ci != 0 && st_all == 0) st_all = (steps - it) * 1000 + ci;
             // K[q][pos] = row q of Quu^-1 times [Qux | gu]   (K = E^-1 B'PA :41-43, kff in position 9)
             double K0 = 0.0, K1 = 0.0;
@@ -387,7 +363,7 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
             double S01[2] = {M01[0], q == 0 ? gh0 : 0.0};
             double S11[2] = {odd ? t10 : M11[0], (!odd && q == 0) ? gh1 : 0.0};
             const double nV0 = q < m ? -M01[1] : 0.0;
-            const double nV1 = q < m ? -v1[0] : 0.0;
+            const double nV1 = q < m ? -rv1[q] : 0.0;  // this lane's own control q
             mma884(S00[0], S00[1], nV0, K0);
             mma884(S01[0], S01[1], nV0, K1);
             mma884(S11[0], S11[1], nV1, K1);
