@@ -18,7 +18,10 @@
  *   - numerical failure never aborts a batch: per-instance `info[batch]` mirrors the potrf `info`
  *     the reference surfaces at src/cholesky_solve.jl:1-3:
  *         0 ok;  otherwise (knot+1)*1000 + stage*100 + (1-based pivot index),
- *         stage 0 = cost-Hessian / Riccati E block, 1 = Schur B block, 2 = Schur C block.
+ *         stage 0 = cost-Hessian / Riccati E block, 1 = Schur B block, 2 = Schur C block;
+ *     pivots count in the caller's numbering (a padded shape's codes are mapped back).  KKT: as in the
+ *     reference, which factors every H_k first, a Hessian failure at any knot takes precedence over a
+ *     Schur-block failure; otherwise the first failure in knot order is reported.
  *   - one handle per host thread / GPU, stream ordered, no global state (SURVEY §8b threading).
  *
  * Two data layouts

@@ -456,6 +456,16 @@ static void kkt_pad_plan(const lqrb_context *h, const KktShape &s, int n2, int m
     P->scr_b = (kkt_tuned_scratch_bytes(h, P->s2, P->z2, P->chunk) + 255) / 256 * 256;
 }
 
+// info codes of the padded shape -> the caller's z numbering.  The pad states sit between the caller's states and its
+// controls (zmap above), so a Hessian pivot (stage 0) above n2 is a control and moves down by n2 - n; the Schur blocks
+// list the caller's rows first and keep their numbers.
+__global__ void kkt_unpad_info_kernel(int32_t *info, int64_t cb, int n, int n2) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= cb) return;
+    const int32_t c = info[i], pivot = c % 1000;
+    if (c > 0 && pivot < 100 && pivot > n2) info[i] = c - (n2 - n);
+}
+
 static int32_t kkt_solve_padded(lqrb_context *h, const KktShape &s, int n2, int m2, int64_t batch, int flags,
                                 const double *data, double *scratch, double *dz, double *mult, double *res, int32_t *info,
                                 Lane lane, KktRecord *record) {
@@ -496,6 +506,10 @@ static int32_t kkt_solve_padded(lqrb_context *h, const KktShape &s, int n2, int 
         rc = kkt_solve_tuned(h, family, P.s2, cb, flags, data2, scr2, dz2, mult2, res ? res2 : nullptr,
                              info ? info + first : nullptr, lane, record);
         if (rc) return rc;
+        if (info) {
+            kkt_unpad_info_kernel<<<(unsigned)((cb + 255) / 256), 256, 0, st>>>(info + first, cb, s.n, n2);
+            LQRB_CUDA(h, cudaGetLastError());
+        }
         ArrayTableOut o = {};
         o.ptr[0] = dz + first * z.NN;
         o.stride[0] = z.NN;

@@ -110,7 +110,7 @@ __global__ void __launch_bounds__(THREADS) kkt_coop_kernel(KktCoopArgs a) {
         double *sb = a.scratch + inst * rec_rows;  // records by position: a list needs only its own slots
         double *zb = a.dz + ii * NN, *mb = a.mult + ii * mult_rows;
         double *rb = a.res ? a.res + ii * NN : nullptr;
-        int st_all = 0;
+        int st_all = 0, hcode = 0;  // first Schur-block failure, first Hessian failure
 
         // ======================= forward sweep =======================
         // phase 0: fused solve; 1: factor only (calculate_shur_factors! + cholesky!(U, F), blocks kept in `scratch`);
@@ -148,7 +148,7 @@ __global__ void __launch_bounds__(THREADS) kkt_coop_kernel(KktCoopArgs a) {
             }
             group_sync<G>();
             int st = factor_hessian<G>(Hf, dinv, w, a.hess, a.soc, t);
-            if (st && !st_all) st_all = (k + 1) * 1000 + st;
+            if (st && !hcode) hcode = (k + 1) * 1000 + st;
             // ---- W = H^-1 Y' (columns of D2', D1', C') and hg = H^-1 g
             if (fac) {
                 for (int e = t; e < w * p1; e += G) W2[e] = D2[(e / w) + (e % w) * n];
@@ -279,7 +279,8 @@ __global__ void __launch_bounds__(THREADS) kkt_coop_kernel(KktCoopArgs a) {
             }
             group_sync<G>();
         }
-        if (active && a.info && t == 0) a.info[ii] = st_all;
+        // the reference factors every H_k before any Schur block: a Hessian failure at any knot takes precedence
+        if (active && a.info && t == 0) a.info[ii] = hcode ? hcode : st_all;
         if (a.phase == 1) continue;  // factor only
 
         // ======================= backward sweep =======================

@@ -272,6 +272,14 @@ struct RecRows2 {
     static constexpr int oC = 0, ol = tri(p1), ROWS = ol + p1;
 };
 
+// The code a sweep reports, given the one so far and a later knot's: the first failure, except that a Hessian failure
+// (stage 0; pivots < 100 at these sizes) takes precedence over a Schur-block one, since the reference factors every H_k
+// before any Schur block (src/cholesky_solver.jl:166-182).
+__device__ __forceinline__ int kkt_first_failure(int st, int later) {
+    const bool hess = st != 0 && st % 1000 < 100, later_hess = later != 0 && later % 1000 < 100;
+    return (st == 0 || (later_hess && !hess)) ? later : st;
+}
+
 // ------------------------------------------------------------------ forward knot --------------
 template <int n, int mk, int p1, int ps, int p2, int HESS, bool SOC, int KS = 32>
 __device__ __forceinline__ int kkt_fwd_knot(const double *__restrict__ kp, double *__restrict__ rec,
@@ -527,13 +535,13 @@ __global__ void __launch_bounds__(THREADS, (n + m <= 5) ? 8 : 1)
         const int s2 = kkt_fwd_knot<n, m, n, PM, n, HESS, SOC>(
             db + ((int64_t)L::KF::ROWS + (int64_t)(k - 1) * L::KM::ROWS) * 32,
             sb + ((int64_t)L::RF::ROWS + (int64_t)(k - 1) * L::RM::ROWS) * 32, cy, k);
-        if (!st) st = s2;
+        st = kkt_first_failure(st, s2);
     }
     const int64_t dlast = (int64_t)L::KF::ROWS + (int64_t)(N - 2) * L::KM::ROWS;
     const int64_t rlast = (int64_t)L::RF::ROWS + (int64_t)(N - 2) * L::RM::ROWS;
     {
         const int s2 = kkt_fwd_knot<n, 0, n, PN, 0, HESS, SOC>(db + dlast * 32, sb + rlast * 32, cy, N - 1);
-        if (!st) st = s2;
+        st = kkt_first_failure(st, s2);
     }
     if (info) info[inst] = st;
 

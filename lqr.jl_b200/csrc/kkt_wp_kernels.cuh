@@ -432,7 +432,7 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
     issue(0, 0);
     if (N > 1) issue(1, 1);
 
-    int st_all = 0, lo = 0x7fffffff, hi = 0, spread = 0, hlo = 0x7fffffff, hhi = 0;
+    int st_all = 0, hcode = 0, lo = 0x7fffffff, hi = 0, spread = 0, hlo = 0x7fffffff, hhi = 0;
     Tile16 Cp;
     SM_UNROLL
     for (int rt = 0; rt < 2; ++rt)
@@ -447,7 +447,7 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
         mbar_wait(bars, 0);
         load_H(Hnext, buf + knot_shift(0), N == 1);
         const int bad = inv16<false, 4>(Hnext, g, q, hlo, hhi);
-        if (bad != 0) st_all = 1000 + PH::zmap(bad - 1) + 1;
+        if (bad != 0) hcode = 1000 + PH::zmap(bad - 1) + 1;
     }
 
     // ---------------- forward sweep: k = 0 .. N-1
@@ -564,7 +564,7 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
                 const int x = PH::xmap(bad - 1);
                 st_all = first ? 1000 + 100 + x + 1 : k * 1000 + 200 + x + 1;
             }
-            if (badh != 0 && st_all == 0) st_all = (k + 2) * 1000 + PH::zmap(badh - 1) + 1;
+            if (badh != 0 && hcode == 0) hcode = (k + 2) * 1000 + PH::zmap(badh - 1) + 1;
             if (lo > 0 && hi >= lo) spread = max(spread, hi - lo);
         }
         Tile16 Zm;
@@ -731,7 +731,8 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
         }
     }
     if (lane == 0) {
-        if (info) info[inst] = st_all;
+        // the reference factors every H_k before any Schur block: a Hessian failure at any knot takes precedence
+        if (info) info[inst] = hcode != 0 ? hcode : st_all;
         cinfo[inst] = spread >> 20;  // log2 of the worst pivot ratio of any Sigma_k
     }
     __syncwarp();
