@@ -6,45 +6,49 @@
 #include "riccati_dmma_kernels.cuh"
 #include "riccati_cta_kernels.cuh"
 
-// ------------------------------------------------------------------ size classes --------------
-// thread-per-instance instantiations (registers only).  Everything else -> cooperative kernel.
-#define RICCATI_TPI_SIZES(X) \
-    X(2, 1) X(3, 2) X(4, 1) X(4, 2) X(6, 3) X(2, 2) X(3, 1) X(3, 3) X(4, 3) X(5, 1) X(5, 2) X(5, 3) X(6, 1) X(6, 2)
+// ------------------------------------------------------------------ routing -------------------
+// The sizes with a kernel of their own, by family: Tpi thread per instance (registers only), Dmma warp per instance on
+// the FP64 tensor cores (n in {8,12}, m <= 4, even record length), Cta CTA per instance on the tensor cores (large
+// state).  The Dmma and Cta entries, in this order, are also the padding targets.
+#define RICCATI_SIZES(X)                                                                                              \
+    X(Tpi, 2, 1) X(Tpi, 3, 2) X(Tpi, 4, 1) X(Tpi, 4, 2) X(Tpi, 6, 3) X(Tpi, 2, 2) X(Tpi, 3, 1) X(Tpi, 3, 3)           \
+    X(Tpi, 4, 3) X(Tpi, 5, 1) X(Tpi, 5, 2) X(Tpi, 5, 3) X(Tpi, 6, 1) X(Tpi, 6, 2)                                     \
+    X(Dmma, 8, 1) X(Dmma, 8, 2) X(Dmma, 8, 3) X(Dmma, 8, 4) X(Dmma, 12, 1) X(Dmma, 12, 2) X(Dmma, 12, 3)              \
+    X(Dmma, 12, 4)                                                                                                    \
+    X(Cta, 16, 8) X(Cta, 16, 16) X(Cta, 24, 8) X(Cta, 24, 16) X(Cta, 32, 8) X(Cta, 32, 16) X(Cta, 48, 16) X(Cta, 64, 16)
 
-static bool riccati_has_tpi(int n, int m) {
-#define X(N_, M_) \
-    if (n == N_ && m == M_) return true;
-    RICCATI_TPI_SIZES(X)
+namespace {
+enum class RiccatiFamily { Tpi, Dmma, Cta, Pad, Coop };
+struct RiccatiRoute {
+    RiccatiFamily family;
+    int n2 = 0, m2 = 0;  // Pad: the tuned size class
+};
+}  // namespace
+
+// Which kernel family solves (n, m): the only reader of the options that steer the choice.
+//   riccati_variant = 2: the cooperative kernel for every shape (the tests' reference); any other value: the default.
+//   riccati_pad = 0: a size without a kernel of its own goes to the cooperative kernel instead of being padded.
+// The tensor-core kernels and the padded path read the packed records with 16-byte loads: misaligned data goes to
+// riccati_tpi or riccati_coop.
+static RiccatiRoute riccati_route(const lqrb_context *h, int n, int m, bool data_aligned) {
+    if (h->opt("riccati_variant", 0) == 2) return {RiccatiFamily::Coop};
+    RiccatiFamily own = RiccatiFamily::Coop;
+#define X(F_, N_, M_) \
+    if (n == N_ && m == M_) own = RiccatiFamily::F_;
+    RICCATI_SIZES(X)
 #undef X
-    return false;
-}
-
-// warp-per-instance FP64 tensor-core (DMMA) instantiations: n in {8,12}, m <= 4, even record length
-#define RICCATI_DMMA_SIZES(X) X(8, 1) X(8, 2) X(8, 3) X(8, 4) X(12, 1) X(12, 2) X(12, 3) X(12, 4)
-
-static bool riccati_has_dmma(int n, int m) {
-#define X(N_, M_) \
-    if (n == N_ && m == M_) return true;
-    RICCATI_DMMA_SIZES(X)
+    if (own == RiccatiFamily::Tpi || (data_aligned && own != RiccatiFamily::Coop)) return {own};
+    if (data_aligned && h->opt("riccati_pad", 1) != 0) {
+#define X(F_, N_, M_) \
+    if (RiccatiFamily::F_ != RiccatiFamily::Tpi && n <= N_ && m <= M_) return {RiccatiFamily::Pad, N_, M_};
+        RICCATI_SIZES(X)
 #undef X
-    return false;
-}
-
-// CTA-per-instance FP64 tensor-core instantiations (large state)
-#define RICCATI_CTA_SIZES(X) X(16, 8) X(16, 16) X(24, 8) X(24, 16) X(32, 8) X(32, 16) X(48, 16) X(64, 16)
-
-static bool riccati_has_cta(int n, int m) {
-#define X(N_, M_) \
-    if (n == N_ && m == M_) return true;
-    RICCATI_CTA_SIZES(X)
-#undef X
-    return false;
+    }
+    return {RiccatiFamily::Coop};
 }
 
 int lqrb_riccati_tile(const lqrb_context *h, int n, int m) {
-    const int64_t force = h->opt("riccati_variant", 0);  // 2 = coop
-    if (force == 2) return 1;
-    return riccati_has_tpi(n, m) ? LQRB_TILE : 1;
+    return riccati_route(h, n, m, true).family == RiccatiFamily::Tpi ? LQRB_TILE : 1;
 }
 
 // ------------------------------------------------------------------ row maps ------------------
@@ -105,29 +109,18 @@ static int32_t check_dims(lqrb_context *h, int n, int m, int N, int64_t batch) {
 // Launch shapes.  The headline batch (65,536 = 2,048 warps) must fit in ONE wave: 148 SMs x 16 warps
 // = 2,368 resident warps needs <= 128 registers per thread (ncu, round 1: at 154 registers only 12
 // warps/SM fit -> 1.15 waves and a tail that ran at 1/7 occupancy).  Small sizes take the tight
-// bound; the register-heavy sizes keep the loose one.
-template <int n, int m, bool LTI, int THREADS, int MINB>
-static void launch_tpi_cfg(int N, int64_t batch, const double *knots, const double *term, double *Z,
-                           double *gains, int32_t *info, cudaStream_t s) {
-    const unsigned grid = (unsigned)((batch + THREADS - 1) / THREADS);
-    riccati_tpi_kernel<n, m, LTI, THREADS, MINB><<<grid, THREADS, 0, s>>>(knots, term, Z, gains, info, N, batch);
-}
-
+// bound (64 threads x 8 CTAs); the register-heavy sizes keep the loose one (128 x 1).
 template <int n, int m>
 static int32_t launch_tpi(lqrb_context *h, int N, int64_t batch, int lti, const double *knots,
                           const double *term, double *Z, double *gains, int32_t *info,
                           cudaStream_t s) {
     constexpr bool SMALL = (n * n + n * m) <= 20;
-    const bool tight = SMALL && h->opt("riccati_tpi_cfg", 0) != 1;
-    if (SMALL && tight) {
-        if (lti) launch_tpi_cfg<n, m, true, 64, 8>(N, batch, knots, term, Z, gains, info, s);
-        else launch_tpi_cfg<n, m, false, 64, 8>(N, batch, knots, term, Z, gains, info, s);
-    } else {
-        if (lti) launch_tpi_cfg<n, m, true, 128, 1>(N, batch, knots, term, Z, gains, info, s);
-        else launch_tpi_cfg<n, m, false, 128, 1>(N, batch, knots, term, Z, gains, info, s);
-    }
+    constexpr int THREADS = SMALL ? 64 : 128, MINB = SMALL ? 8 : 1;
+    const unsigned grid = (unsigned)((batch + THREADS - 1) / THREADS);
+    if (lti) riccati_tpi_kernel<n, m, true, THREADS, MINB><<<grid, THREADS, 0, s>>>(knots, term, Z, gains, info, N, batch);
+    else riccati_tpi_kernel<n, m, false, THREADS, MINB><<<grid, THREADS, 0, s>>>(knots, term, Z, gains, info, N, batch);
     char nm[64];
-    snprintf(nm, sizeof nm, "riccati_tpi<%d,%d>%s%s", n, m, lti ? "[lti]" : "", tight ? "[64x8]" : "[128x1]");
+    snprintf(nm, sizeof nm, "riccati_tpi<%d,%d>%s%s", n, m, lti ? "[lti]" : "", SMALL ? "[64x8]" : "[128x1]");
     h->kernel_name = nm;
     LQRB_LAUNCH_CHECK(h, "riccati_tpi_kernel");
     return 0;
@@ -193,21 +186,31 @@ static int32_t launch_cta(lqrb_context *h, int N, int64_t batch, int lti, const 
     return 0;
 }
 
+template <RiccatiFamily F, int n, int m>
+static int32_t launch_sized(lqrb_context *h, int N, int64_t batch, int lti, const double *knots, const double *term,
+                            double *Z, double *gains, int32_t *info, cudaStream_t s) {
+    if constexpr (F == RiccatiFamily::Tpi) return launch_tpi<n, m>(h, N, batch, lti, knots, term, Z, gains, info, s);
+    else if constexpr (F == RiccatiFamily::Dmma) return launch_dmma<n, m>(h, N, batch, lti, knots, term, Z, gains, info, s);
+    else return launch_cta<n, m>(h, N, batch, lti, knots, term, Z, gains, info, s);
+}
+
+// the kernel of a (family, n, m) entry of RICCATI_SIZES
+static int32_t launch_tuned(lqrb_context *h, RiccatiFamily family, int n, int m, int N, int64_t batch, int lti,
+                            const double *knots, const double *term, double *Z, double *gains, int32_t *info,
+                            cudaStream_t s) {
+#define X(F_, N_, M_)                                                     \
+    if (family == RiccatiFamily::F_ && n == N_ && m == M_)                \
+        return launch_sized<RiccatiFamily::F_, N_, M_>(h, N, batch, lti, knots, term, Z, gains, info, s);
+    RICCATI_SIZES(X)
+#undef X
+    return lqrb_fail(h, 1, "no tuned Riccati kernel for this size");
+}
+
 // ------------------------------------------------------------------ padding into a tuned size class ----
 // A size without a tensor-core kernel of its own (n = 7, 9..11, 13.., or m > 4 at n <= 12, ...) is embedded in the next
 // tuned size class (n2, m2): pad states with A = 0, B = 0, Q = Qf = I, x0 = 0 and pad controls with R = I stay exactly
 // zero and leave the original recursion untouched.  The packed arrays are expanded on the device, the tuned kernel runs,
 // Z and the gains are compacted back.
-static bool riccati_pad_target(const lqrb_context *h, int n, int m, int *n2, int *m2) {
-    if (h->opt("riccati_pad", 1) == 0 || h->opt("riccati_variant", 0) != 0) return false;
-    if (lqrb_riccati_tile(h, n, m) == LQRB_TILE || riccati_has_dmma(n, m) || riccati_has_cta(n, m)) return false;
-#define X(N_, M_) \
-    if (n <= N_ && m <= M_) { *n2 = N_; *m2 = M_; return true; }
-    RICCATI_DMMA_SIZES(X)
-    RICCATI_CTA_SIZES(X)
-#undef X
-    return false;
-}
 
 namespace {
 struct RiccatiPadMaps {
@@ -256,13 +259,14 @@ static RiccatiPadMaps riccati_pad_maps(int n, int m, int N, int Kn, int n2, int 
     return M;
 }
 
-static int32_t riccati_solve_on(lqrb_context *h, int n, int m, int N, int64_t batch, int flags, const double *knots,
-                                const double *term, double *Z, double *gains, int32_t *info, Lane lane);
-
 static int32_t riccati_solve_padded(lqrb_context *h, int n, int m, int N, int n2, int m2, int64_t batch, int flags,
                                     const double *knots, const double *term, double *Z, double *gains, int32_t *info,
                                     Lane lane) {
-    const int Kn = (flags & LQRB_FLAG_LTI) ? 1 : N - 1;
+    const RiccatiFamily family = riccati_route(h, n2, m2, true).family;
+    if (family != RiccatiFamily::Dmma && family != RiccatiFamily::Cta)
+        return lqrb_fail(h, 1, "padded Riccati size has no tensor-core kernel");
+    const int lti = (flags & LQRB_FLAG_LTI) ? 1 : 0;
+    const int Kn = lti ? 1 : N - 1;
     const int64_t F = lqrb_riccati_knot_rows(n, m), F2 = lqrb_riccati_knot_rows(n2, m2);
     const int64_t TR = tri(n) + 2 * n, TR2 = tri(n2) + 2 * n2;
     const int64_t ZR = (int64_t)N * n + (int64_t)(N - 1) * m, ZR2 = (int64_t)N * n2 + (int64_t)(N - 1) * m2;
@@ -302,7 +306,8 @@ static int32_t riccati_solve_padded(lqrb_context *h, int n, int m, int N, int n2
         src.stride[0] = TR;
         rc = lqrb_gather_pack(h, mt, src, cb, 1, term2, lane.stream);
         if (rc) return rc;
-        rc = riccati_solve_on(h, n2, m2, N, cb, flags, knots2, term2, Z2, gains2, info ? info + first : nullptr, lane);
+        rc = launch_tuned(h, family, n2, m2, N, cb, lti, knots2, term2, Z2, gains2, info ? info + first : nullptr,
+                          lane.stream);
         if (rc) return rc;
         name = h->kernel_name;
         ArrayTableOut o = {};
@@ -325,34 +330,19 @@ static int32_t riccati_solve_on(lqrb_context *h, int n, int m, int N, int64_t ba
                                 const double *knots, const double *term, double *Z, double *gains,
                                 int32_t *info, Lane lane) {
     if (batch == 0) return 0;
-    {
-        int n2, m2;
-        if (((uintptr_t)knots & 15) == 0 && riccati_pad_target(h, n, m, &n2, &m2))
-            return riccati_solve_padded(h, n, m, N, n2, m2, batch, flags, knots, term, Z, gains, info, lane);
-    }
-    const cudaStream_t s = lane.stream;
+    const RiccatiRoute r = riccati_route(h, n, m, ((uintptr_t)knots & 15) == 0);
     const int lti = (flags & LQRB_FLAG_LTI) ? 1 : 0;
-    const int tile = lqrb_riccati_tile(h, n, m);
-    if (tile == LQRB_TILE) {
-#define X(N_, M_) \
-    if (n == N_ && m == M_) return launch_tpi<N_, M_>(h, N, batch, lti, knots, term, Z, gains, info, s);
-        RICCATI_TPI_SIZES(X)
-#undef X
+    switch (r.family) {
+    case RiccatiFamily::Pad:
+        return riccati_solve_padded(h, n, m, N, r.n2, r.m2, batch, flags, knots, term, Z, gains, info, lane);
+    case RiccatiFamily::Tpi:
+    case RiccatiFamily::Dmma:
+    case RiccatiFamily::Cta:
+        return launch_tuned(h, r.family, n, m, N, batch, lti, knots, term, Z, gains, info, lane.stream);
+    case RiccatiFamily::Coop:
+        break;
     }
-    // bulk copies need 16-byte aligned records
-    if (h->opt("riccati_variant", 0) != 2 && riccati_has_dmma(n, m) && ((uintptr_t)knots & 15) == 0) {
-#define X(N_, M_) \
-    if (n == N_ && m == M_) return launch_dmma<N_, M_>(h, N, batch, lti, knots, term, Z, gains, info, s);
-        RICCATI_DMMA_SIZES(X)
-#undef X
-    }
-    if (h->opt("riccati_variant", 0) != 2 && riccati_has_cta(n, m) && ((uintptr_t)knots & 15) == 0) {
-#define X(N_, M_) \
-    if (n == N_ && m == M_) return launch_cta<N_, M_>(h, N, batch, lti, knots, term, Z, gains, info, s);
-        RICCATI_CTA_SIZES(X)
-#undef X
-    }
-    return launch_coop(h, n, m, N, batch, lti, knots, term, Z, gains, info, s);
+    return launch_coop(h, n, m, N, batch, lti, knots, term, Z, gains, info, lane.stream);
 }
 
 extern "C" int32_t lqrb_riccati_solve_packed_f64(lqrb_handle_t h, int32_t n, int32_t m, int32_t N,

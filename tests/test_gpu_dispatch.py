@@ -1,5 +1,5 @@
-"""GPU: which KKT kernel family runs for a shape and the options (the routing table), and the conditioning record of a
-call whose tuned-kernel work is split into chunks."""
+"""GPU: which kernel family runs for a shape and the options, for both solvers (the KKT and the Riccati routing
+tables), and the conditioning record of a KKT call whose tuned-kernel work is split into chunks."""
 import numpy as np
 import pytest
 
@@ -145,6 +145,98 @@ def test_route(handle, oracle_mod, shape, opts, call, kern):
     dzo, lamo, infoo = oracle_mod.kkt_solve(prob)
     assert (info == 0).all() and (infoo == 0).all()
     assert np.linalg.norm(dz - dzo) <= 1e-9 * np.linalg.norm(dzo) and np.linalg.norm(lam - lamo) <= 1e-9 * np.linalg.norm(lamo)
+
+
+def _riccati_solve_packed(handle, prob, misaligned):
+    """riccati_pack -> riccati_solve_packed -> riccati_unpack on device buffers; `misaligned` puts the packed knots 8
+    bytes off 16-byte alignment."""
+    import torch
+    f = ops.riccati_flatten(prob)
+    n, m, N, b = f["n"], f["m"], f["N"], f["batch"]
+    flags = _lib.FLAG_LTI if f["lti"] else 0
+    L = _lib.riccati_layout(n, m, N, flags)
+    ldb = _lib.padded_batch(b)
+    names = ("A", "B", "Q", "R", "q", "r", "Qf", "qf", "x0")
+    dev = {k: torch.from_numpy(f[k]).cuda() for k in names}
+    z = lambda *s: torch.zeros(*s, dtype=torch.float64, device="cuda")  # noqa: E731
+    base = z(ldb * L.knot_count * L.rows_per_knot + 1)
+    knots = base[1:] if misaligned else base[:-1]
+    assert knots.data_ptr() % 16 == (8 if misaligned else 0)
+    term, Zp, gains = z(ldb * L.term_rows), z(ldb * L.z_rows), z(ldb * L.gain_rows)
+    Z, K, kff = z(b, L.z_rows), z(b, N - 1, n, m), z(b, N - 1, m)
+    info = torch.zeros(b, dtype=torch.int32, device="cuda")
+    handle.set_stream(torch.cuda.current_stream().cuda_stream)
+    try:
+        ops.riccati_pack(handle, n, m, N, b, flags, *[dev[k] for k in names], knots, term)
+        ops.riccati_solve_packed(handle, n, m, N, b, flags, knots, term, Zp, gains, info)
+        ops.riccati_unpack(handle, n, m, N, b, Zp, gains, Z, K, kff)
+        torch.cuda.synchronize()
+    finally:
+        handle.set_stream(None)
+    X, U = ops.split_primals(Z.cpu().numpy(), n, m, N)
+    return X, U, np.swapaxes(K.cpu().numpy(), -1, -2), kff.cpu().numpy(), info.cpu().numpy()
+
+
+# (shape, options, call) -> the kernel name the call reports.  call: "host" = lqrb_riccati_f64 on host buffers,
+# "packed" / "misaligned" = lqrb_riccati_solve_packed_f64 with 16-byte aligned / misaligned packed knots.
+RICCATI_ROUTES = [
+    # every family on its own shapes
+    (dict(n=4, m=1, N=30), {}, "host", "riccati_tpi<4,1>[64x8]"),
+    (dict(n=6, m=3, N=30), {}, "host", "riccati_tpi<6,3>[128x1]"),
+    (dict(n=4, m=1, N=30, lti=True), {}, "host", "riccati_tpi<4,1>[lti][64x8]"),
+    (dict(n=8, m=1, N=30), {}, "host", "riccati_dmma<8,1>"),
+    (dict(n=12, m=4, N=30), {}, "host", "riccati_dmma<12,4>"),
+    (dict(n=12, m=4, N=30, lti=True), {}, "host", "riccati_dmma<12,4>[lti]"),
+    (dict(n=16, m=16, N=12), {}, "host", "riccati_cta_dmma<16,16>"),
+    (dict(n=64, m=16, N=8), {}, "host", "riccati_cta_dmma<64,16>"),
+    # padding into each class
+    (dict(n=7, m=2, N=30), {}, "host", "riccati_dmma<8,2> <- (7,2) padded"),
+    (dict(n=5, m=4, N=30), {}, "host", "riccati_dmma<8,4> <- (5,4) padded"),
+    (dict(n=10, m=3, N=30), {}, "host", "riccati_dmma<12,3> <- (10,3) padded"),
+    (dict(n=7, m=7, N=20), {}, "host", "riccati_cta_dmma<16,8> <- (7,7) padded"),
+    (dict(n=13, m=2, N=20), {}, "host", "riccati_cta_dmma<16,8> <- (13,2) padded"),
+    (dict(n=40, m=12, N=8), {}, "host", "riccati_cta_dmma<48,16> <- (40,12) padded"),
+    # no padding target
+    (dict(n=65, m=16, N=6), {}, "host", "riccati_coop<G=256>(n=65,m=16)"),
+    # riccati_pad = 0
+    (dict(n=10, m=3, N=30), {"riccati_pad": 0}, "host", "riccati_coop<G=32>(n=10,m=3)"),
+    (dict(n=12, m=4, N=30), {"riccati_pad": 0}, "host", "riccati_dmma<12,4>"),
+    # riccati_variant = 2: the cooperative kernel everywhere; other values act as 0
+    (dict(n=4, m=1, N=30), {"riccati_variant": 2}, "host", "riccati_coop<G=32>(n=4,m=1)"),
+    (dict(n=12, m=4, N=30), {"riccati_variant": 2}, "host", "riccati_coop<G=32>(n=12,m=4)"),
+    (dict(n=64, m=16, N=8), {"riccati_variant": 2}, "host", "riccati_coop<G=256>(n=64,m=16)"),
+    (dict(n=10, m=3, N=30), {"riccati_variant": 2}, "host", "riccati_coop<G=32>(n=10,m=3)"),
+    (dict(n=10, m=3, N=30), {"riccati_variant": 1}, "host", "riccati_dmma<12,3> <- (10,3) padded"),
+    # the packed entry point, with aligned and misaligned data
+    (dict(n=4, m=1, N=30), {}, "misaligned", "riccati_tpi<4,1>[64x8]"),
+    (dict(n=12, m=4, N=30), {}, "misaligned", "riccati_coop<G=32>(n=12,m=4)"),
+    (dict(n=64, m=16, N=8), {}, "misaligned", "riccati_coop<G=256>(n=64,m=16)"),
+    (dict(n=10, m=3, N=30), {}, "misaligned", "riccati_coop<G=32>(n=10,m=3)"),
+    (dict(n=10, m=3, N=30), {}, "packed", "riccati_dmma<12,3> <- (10,3) padded"),
+]
+
+_RICCATI_DEFAULTS = {"riccati_variant": 0, "riccati_pad": 1}
+
+
+@pytest.mark.parametrize("shape,opts,call,kern", RICCATI_ROUTES)
+def test_riccati_route(handle, oracle_mod, shape, opts, call, kern):
+    n, m, N = shape["n"], shape["m"], shape["N"]
+    prob = problems.random_lqr_riccati(n, m, N, 3, seed=n + m + N, lti=shape.get("lti", False))
+    for k, v in opts.items():
+        handle.set_option(k, v)
+    try:
+        if call == "host":
+            out = ops.riccati_solve_problem(prob, handle=handle)
+        else:
+            out = _riccati_solve_packed(handle, prob, call == "misaligned")
+    finally:
+        for k in opts:
+            handle.set_option(k, _RICCATI_DEFAULTS[k])
+    assert handle.last_kernel == kern
+    ref = oracle_mod.riccati(prob)
+    assert (out[4] == 0).all() and (ref[4] == 0).all()
+    for got, want in zip(out[:4], ref[:4]):  # X, U, K, kff
+        assert np.linalg.norm(got - want) <= 1e-9 * np.linalg.norm(want)
 
 
 @pytest.mark.parametrize("b,opts", [(3600, {"scratch_budget_mb": 8}), (70, {"host_chunk": 32})])
