@@ -76,8 +76,29 @@ def gradient_flat(prob):
     return g
 
 
-def solve(Z0, x0, xf, o):
-    """Returns Z, feas_p, feas_d, iters, kkt_solves (per-instance bookkeeping like the device driver)."""
+# branch codes of the trace: which trial an instance accepted in one iteration
+BR_FROZEN, BR_REJECTED, BR_FULL, BR_SOC = -2, -1, 0, 1  # 2..10: back-tracking trial i, alpha = rho^(i-1)
+
+
+def _margin(lhs, rhs):
+    """Relative distance of a merit comparison from its threshold (NaN compares as 0: no margin)."""
+    with np.errstate(invalid="ignore"):
+        return np.nan_to_num(np.abs(lhs - rhs) / np.maximum(np.maximum(np.abs(lhs), np.abs(rhs)), 1e-300), nan=0.0)
+
+
+def solve(Z0, x0, xf, o, trace=False):
+    """Returns Z, feas_p, feas_d, iters, kkt_solves (per-instance bookkeeping like the device driver).
+
+    trace=True appends a dict of per-iteration arrays (the arithmetic is the same, Z is bit-identical):
+      Z          (iters, b, NN)  the iterate after iteration k + 1 (what a run with iters = k + 1 returns)
+      branch     (iters, b)      BR_FROZEN (converged before this iteration), BR_FULL (alpha = 1), BR_SOC,
+                                 2..10 (accepted at back-tracking trial i), BR_REJECTED (every trial rejected)
+      margin     (iters, b, 11)  relative margin of each merit comparison evaluated (alpha = 1, SOC, trials 2..10),
+                                 NaN where the instance did not evaluate it; 0 where a side is NaN
+      conv_margin (iters, b, 2)  relative margins of feas_p vs eps_p and feas_d vs eps_d in the convergence test
+      mu         (iters, b)      the merit penalty after its update
+      kkt_solves (iters,)        the running count of KKT solves, SOC solves included
+    """
     Z = Z0.copy()
     b = Z.shape[0]
     mu = np.ones(b)
@@ -85,54 +106,82 @@ def solve(Z0, x0, xf, o):
     iters = np.zeros(b, np.int32)
     lam = None
     solves = 0
+    tr = dict(Z=[], branch=[], margin=[], conv_margin=[], mu=[], kkt_solves=[])
     for _ in range(o["iters"]):
         prob = linearize(Z, x0, xf, o)
         c1, d, cN = constraints(Z, x0, xf, o)
         feas_p = np.maximum(np.abs(c1).max(1), np.maximum(np.abs(d).max((1, 2)), np.abs(cN).max(1)))
         feas_d = residual_norm(prob, lam)
+        if trace:
+            tr["conv_margin"].append(np.where(conv[:, None], np.nan, np.stack(
+                [_margin(feas_p, o["eps_p"]), _margin(feas_d, o["eps_d"])], -1)))
         conv |= (feas_p < o["eps_p"]) & (feas_d < o["eps_d"])
         dz, lam_new, info = oracle.kkt_solve(prob)
         solves += b
         act = ~conv
         lam = np.where(act[:, None], lam_new, lam if lam is not None else 0 * lam_new)
         iters[act] += 1
+        br = np.where(conv, BR_FROZEN, BR_REJECTED)
+        mg = np.full((b, 11), np.nan)
         if not o["line_search"]:
             Z[act] += dz[act]
-            continue
-        mu = np.where(act, np.maximum(mu, 1.1 * np.abs(lam_new).max(1)), mu)
-        g = gradient_flat(prob)
-        cn0 = c_norm1(Z, x0, xf, o)
-        phi0 = cost(Z, xf, o) + mu * cn0
-        dphi0 = (g * dz).sum(1) - mu * cn0
-        eta, rho = 1e-4, 0.5
-        done = conv.copy()
-        phi = lambda Zt: cost(Zt, xf, o) + mu * c_norm1(Zt, x0, xf, o)  # noqa: E731
-        ok = (phi(Z + dz) <= phi0 + eta * dphi0) & ~done
-        Z[ok] += dz[ok]
-        done |= ok
-        alpha = np.ones(b)
-        if (~done).any():
-            c1t, dt_, cNt = constraints(Z + dz, x0, xf, o)
-            prob2 = dict(prob)
-            p, Cs, cs = problems._init_goal_blocks(b, n, m, o["N"], c1t, cNt)
-            prob2.update(d=dt_, c=cs)
-            dzh, _, _ = oracle.kkt_solve(prob2, soc=True)
-            solves += b
-            ok = (phi(Z + dz + dzh) < phi0 + eta * dphi0) & ~done
-            Z[ok] += dz[ok] + dzh[ok]
+            br[act] = BR_FULL
+        else:
+            mu = np.where(act, np.maximum(mu, 1.1 * np.abs(lam_new).max(1)), mu)
+            g = gradient_flat(prob)
+            cn0 = c_norm1(Z, x0, xf, o)
+            phi0 = cost(Z, xf, o) + mu * cn0
+            dphi0 = (g * dz).sum(1) - mu * cn0
+            eta, rho = 1e-4, 0.5
+            done = conv.copy()
+            phi = lambda Zt: cost(Zt, xf, o) + mu * c_norm1(Zt, x0, xf, o)  # noqa: E731
+            lhs, rhs = phi(Z + dz), phi0 + eta * dphi0
+            if trace:
+                mg[~done, 0] = _margin(lhs, rhs)[~done]
+            ok = (lhs <= rhs) & ~done
+            Z[ok] += dz[ok]
             done |= ok
-            alpha[~done] = rho
-            for _trial in range(2, 11):  # the reference's i = 2..10 (src/sqp.jl:76-92): alpha = rho^1..rho^9
-                if done.all():
-                    break
-                ok = (phi(Z + alpha[:, None] * dz) <= phi0 + eta * alpha * dphi0) & ~done
-                Z[ok] += alpha[ok, None] * dz[ok]
+            br[ok] = BR_FULL
+            alpha = np.ones(b)
+            if (~done).any():
+                c1t, dt_, cNt = constraints(Z + dz, x0, xf, o)
+                prob2 = dict(prob)
+                p, Cs, cs = problems._init_goal_blocks(b, n, m, o["N"], c1t, cNt)
+                prob2.update(d=dt_, c=cs)
+                dzh, _, _ = oracle.kkt_solve(prob2, soc=True)
+                solves += b
+                lhs = phi(Z + dz + dzh)
+                if trace:
+                    mg[~done, 1] = _margin(lhs, rhs)[~done]
+                ok = (lhs < rhs) & ~done
+                Z[ok] += dz[ok] + dzh[ok]
                 done |= ok
-                alpha[~done] *= rho
+                br[ok] = BR_SOC
+                alpha[~done] = rho
+                for trial in range(2, 11):  # the reference's i = 2..10 (src/sqp.jl:76-92): alpha = rho^1..rho^9
+                    if done.all():
+                        break
+                    lhs, rhs_a = phi(Z + alpha[:, None] * dz), phi0 + eta * alpha * dphi0
+                    if trace:
+                        mg[~done, trial] = _margin(lhs, rhs_a)[~done]
+                    ok = (lhs <= rhs_a) & ~done
+                    Z[ok] += alpha[ok, None] * dz[ok]
+                    done |= ok
+                    br[ok] = trial
+                    alpha[~done] *= rho
+        if trace:
+            tr["Z"].append(Z.copy())
+            tr["branch"].append(br)
+            tr["margin"].append(mg)
+            tr["mu"].append(mu.copy())
+            tr["kkt_solves"].append(solves)
     prob = linearize(Z, x0, xf, o)
     c1, d, cN = constraints(Z, x0, xf, o)
     feas_p = np.maximum(np.abs(c1).max(1), np.maximum(np.abs(d).max((1, 2)), np.abs(cN).max(1)))
-    return Z, feas_p, residual_norm(prob, lam), iters, solves
+    out = (Z, feas_p, residual_norm(prob, lam), iters, solves)
+    if trace:
+        out += ({k: np.array(v) for k, v in tr.items()},)
+    return out
 
 
 def residual_norm(prob, lam):
@@ -187,6 +236,42 @@ def turn90_problem(batch, N=11, seed=2):
     body[:, :, :n], body[:, :, n:] = X[:, :-1], U
     Z[:, (N - 1) * (n + m):] = X[:, -1]
     return Z, x0, xf, o
+
+
+def hard_turn_problem(batch, N, tf, qf, z_sd, goal_scale, theta_sd, seed, keep=None):
+    """A turn90 problem made hard for the line search: horizon tf, terminal weight qf, goal position scaled by
+    goal_scale, goal heading + theta_sd * N(0,1), initial guess + z_sd * N(0,1).  keep: instance subset."""
+    Z0, x0, xf, o = turn90_problem(batch, N=N, seed=seed)
+    rng = np.random.default_rng(seed)
+    xf = xf * np.array([goal_scale, goal_scale, 1.0])
+    xf[:, 2] += theta_sd * rng.standard_normal(batch)
+    Z0 = Z0 + z_sd * rng.standard_normal(Z0.shape)
+    o = dict(o, dt=tf / (N - 1), qf_diag=qf)
+    if keep is not None:
+        Z0, x0, xf = Z0[keep], x0[keep], xf[keep]
+    return Z0, x0, xf, o
+
+
+def line_search_cases():
+    """Frozen inputs on which the line search takes every branch: name -> (Z0, x0, xf, options).
+
+    The first four reach the second-order correction and back-tracking trials 2..5 in hundreds of instance-iterations;
+    the short horizons N = 3, 4, 5 with batches 33, 65 and 1 are the edges of the device's prefetch ring and partial
+    warps and CTAs, and most of their instances converge (at different iterations) and freeze.  n3_far_start keeps
+    the 18 instances of its draw whose every merit comparison is at least 1e-7 (relative) from its threshold and whose
+    trajectory moves by less than 3e-12 under 1e-13 noise in the QP steps; they reach back-tracking trials 2..10, and
+    one of them (index 6 of the subset) rejects all ten trials in some iterations."""
+    far = [0, 5, 8, 16, 18, 20, 23, 25, 28, 30, 35, 38, 45, 47, 48, 55, 58, 63]
+    return {
+        "n11_far_goal": hard_turn_problem(128, 11, 3.0, 100.0, 1.0, 5.0, 3.0, seed=0),
+        "n21_short_tf": hard_turn_problem(128, 21, 1.0, 100.0, 1.0, 3.0, 2.0, seed=0),
+        "n6": hard_turn_problem(128, 6, 3.0, 100.0, 1.0, 2.0, 3.0, seed=0),
+        "n41_qf1000": hard_turn_problem(128, 41, 2.0, 1000.0, 2.0, 4.0, 3.0, seed=0),
+        "n3_b33": hard_turn_problem(33, 3, 3.0, 100.0, 0.5, 1.0, 0.0, seed=0),
+        "n4_b65": hard_turn_problem(65, 4, 3.0, 100.0, 0.5, 1.0, 0.0, seed=0),
+        "n5_b1": hard_turn_problem(1, 5, 3.0, 100.0, 1.0, 1.0, 1.0, seed=39),
+        "n3_far_start": hard_turn_problem(65, 3, 3.0, 100.0, 10.0, 1.0, 3.0, seed=2, keep=far),
+    }
 
 
 def slsqp_solution(Z0, x0, xf, o, i):
