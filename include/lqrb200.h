@@ -134,6 +134,25 @@ int32_t lqrb_riccati_f64(lqrb_handle_t handle, int32_t n, int32_t m, int32_t N, 
                          const double *qf, const double *x0, double *Z, double *K, double *kff,
                          int32_t *info);
 
+/* Gradient of a scalar loss l(Z) through lqrb_riccati_f64: given the inputs, that call's output Z and dZ = dl/dZ
+ * (same shape as Z), writes dl/d of every input.  The adjoint LQR (same A, B, Q, R, Qf, linear terms dZ, initial
+ * state 0) is solved by the same kernels as the forward solve, then one backward sweep forms the costates and the
+ * gradients (DESIGN §4.8).
+ *   inputs as in lqrb_riccati_f64 (x0 is not needed); Z[NN,batch], dZ[NN,batch]
+ *   outputs gA, gB, gQ, gR, gq, gr, gQf, gqf, gx0: the shape of their input (Kn = 1 under LQRB_FLAG_LTI: the sum over
+ *   the knots); any may be NULL, not all.  gq, gr, gqf are available with LQRB_FLAG_NO_AFFINE or NULL q, r, qf.
+ *   The kernels read only the upper triangle of Q, R, Qf: their gradients are returned as the symmetric matrices
+ *   (1/2)(x^ x' + x x^'); a finite-difference check perturbs (i,j) and (j,i) together.
+ *   info[batch] | NULL: the potrf info of the adjoint solve (the same matrices as the forward solve).  The gradients
+ *   of an instance with info != 0 carry no meaning.
+ * Host or device pointers, with the staged / device-resident rule of every entry point.                      */
+int32_t lqrb_riccati_grad_f64(lqrb_handle_t handle, int32_t n, int32_t m, int32_t N, int64_t batch,
+                              int32_t flags, const double *A, const double *B, const double *Q,
+                              const double *R, const double *q, const double *r, const double *Qf,
+                              const double *qf, const double *Z, const double *dZ, double *gA, double *gB,
+                              double *gQ, double *gR, double *gq, double *gr, double *gQf, double *gqf,
+                              double *gx0, int32_t *info);
+
 /* Device-resident split of the same call (all pointers are DEVICE pointers). */
 int32_t lqrb_riccati_pack_f64(lqrb_handle_t handle, int32_t n, int32_t m, int32_t N, int64_t batch,
                               int32_t flags, const double *A, const double *B, const double *Q,

@@ -68,6 +68,7 @@ _SIGS = {
     "lqrb_kkt_data_rows": (c_i64, [c_i32, c_i32, c_i32, c_vp, c_i32, c_i32]),
     "lqrb_kkt_knot_offset": (c_i64, [c_i32, c_i32, c_i32, c_vp, c_i32, c_i32, c_i32]),
     "lqrb_riccati_f64": (c_i32, [c_vp, c_i32, c_i32, c_i32, c_i64, c_i32] + [c_dp] * 12 + [c_vp]),
+    "lqrb_riccati_grad_f64": (c_i32, [c_vp, c_i32, c_i32, c_i32, c_i64, c_i32] + [c_dp] * 19 + [c_vp]),
     "lqrb_riccati_pack_f64": (c_i32, [c_vp, c_i32, c_i32, c_i32, c_i64, c_i32] + [c_dp] * 11),
     "lqrb_riccati_solve_packed_f64": (c_i32, [c_vp, c_i32, c_i32, c_i32, c_i64, c_i32] + [c_dp] * 4 + [c_vp]),
     "lqrb_riccati_tile_width": (c_i32, [c_vp, c_i32, c_i32]),

@@ -5,6 +5,7 @@
 #include "riccati_kernels.cuh"
 #include "riccati_dmma_kernels.cuh"
 #include "riccati_cta_kernels.cuh"
+#include "riccati_grad_kernels.cuh"
 
 // ------------------------------------------------------------------ routing -------------------
 // The sizes with a kernel of their own, by family: Tpi thread per instance (registers only), Dmma warp per instance on
@@ -77,6 +78,38 @@ static std::vector<RowMap> riccati_term_map(int n) {
         for (int i = 0; i <= j; ++i) map.push_back({6, i + j * n, 0.0});
     for (int e = 0; e < n; ++e) map.push_back({7, e, 0.0});
     for (int e = 0; e < n; ++e) map.push_back({8, e, 0.0});
+    return map;
+}
+
+// The adjoint problem of lqrb_riccati_grad_f64: the forward A, B, Q, R with q̂_k, r̂_k taken from dZ, always packed as
+// LTV (q̂ varies per knot; under LTI every knot points at record 0 of A, B, Q, R).
+// source array ids: 0 A, 1 B, 2 Q, 3 R, 4 dZ, 6 Qf
+static std::vector<RowMap> riccati_adjoint_knot_map(int n, int m, int N, int flags) {
+    const bool lti = (flags & LQRB_FLAG_LTI) != 0;
+    std::vector<RowMap> map;
+    map.reserve((size_t)(N - 1) * lqrb_riccati_knot_rows(n, m));
+    for (int k = 0; k < N - 1; ++k) {
+        const int kk = lti ? 0 : k, z = k * (n + m);
+        for (int e = 0; e < n * n; ++e) map.push_back({0, kk * n * n + e, 0.0});
+        for (int e = 0; e < n * m; ++e) map.push_back({1, kk * n * m + e, 0.0});
+        for (int j = 0; j < n; ++j)
+            for (int i = 0; i <= j; ++i) map.push_back({2, kk * n * n + i + j * n, 0.0});
+        for (int j = 0; j < m; ++j)
+            for (int i = 0; i <= j; ++i) map.push_back({3, kk * m * m + i + j * m, 0.0});
+        for (int e = 0; e < n; ++e) map.push_back({4, z + e, 0.0});
+        for (int e = 0; e < m; ++e) map.push_back({4, z + n + e, 0.0});
+        if (lqrb_riccati_knot_rows(n, m) > n * n + n * m + tri(n) + tri(m) + n + m) map.push_back({-1, 0, 0.0});  // padding
+    }
+    return map;
+}
+
+// Qf | q̂f = dZ[x_{N-1}] | x̂0 = 0
+static std::vector<RowMap> riccati_adjoint_term_map(int n, int m, int N) {
+    std::vector<RowMap> map;
+    for (int j = 0; j < n; ++j)
+        for (int i = 0; i <= j; ++i) map.push_back({6, i + j * n, 0.0});
+    for (int e = 0; e < n; ++e) map.push_back({4, (N - 1) * (n + m) + e, 0.0});
+    for (int e = 0; e < n; ++e) map.push_back({-1, 0, 0.0});
     return map;
 }
 
@@ -490,6 +523,123 @@ extern "C" int32_t lqrb_riccati_f64(lqrb_handle_t h, int32_t n, int32_t m, int32
             if (rc) return rc;
             return riccati_unpack_on(h, n, m, N, cb, Zp, gains, (double *)out[0], (double *)out[1], (double *)out[2],
                                      lane.stream);
+        });
+}
+
+// ------------------------------------------------------------------ gradient ------------------
+template <int G, int R>
+static int32_t launch_grad(lqrb_context *h, int n, int m, int N, int64_t batch, bool lti, const RiccatiGradArgs &a,
+                           cudaStream_t s) {
+    constexpr int THREADS = 128;
+    int threads = THREADS;
+    size_t smem = 0;
+    if (lti) {
+        // one accumulator slice per group, fewer groups per block when the slices are large
+        const size_t per = (size_t)(2 * n * n + n * m + m * m) * sizeof(double), cap = 227 * 1024;
+        if (per > cap) return lqrb_fail(h, -2, "n, m too large for the LTI gradient accumulators");
+        const int groups = (int)std::min<size_t>(THREADS / G, cap / per);
+        threads = groups * G;
+        smem = per * groups;
+    }
+    const int per_block = threads / G;
+    const unsigned grid = (unsigned)((batch + per_block - 1) / per_block);
+    if (lti) {
+        auto kern = riccati_grad_kernel<G, R, true>;
+        LQRB_CUDA(h, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        kern<<<grid, threads, smem, s>>>(a, n, m, N, batch);
+    } else {
+        riccati_grad_kernel<G, R, false><<<grid, threads, 0, s>>>(a, n, m, N, batch);
+    }
+    char nm[64];
+    snprintf(nm, sizeof nm, "riccati_grad<G=%d,R=%d>%s", G, R, lti ? "[lti]" : "");
+    h->kernel_name += std::string(" + ") + nm;
+    LQRB_LAUNCH_CHECK(h, "riccati_grad_kernel");
+    return 0;
+}
+
+// The solve accepts n <= 84 (riccati_coop_kernel's shared memory bounds the sizes without a tuned kernel), so three
+// rows per lane cover every size that reaches the sweep.
+static int32_t launch_grad_sized(lqrb_context *h, int n, int m, int N, int64_t batch, bool lti,
+                                 const RiccatiGradArgs &a, cudaStream_t s) {
+    if (n <= 4) return launch_grad<4, 1>(h, n, m, N, batch, lti, a, s);
+    if (n <= 8) return launch_grad<8, 1>(h, n, m, N, batch, lti, a, s);
+    if (n <= 16) return launch_grad<16, 1>(h, n, m, N, batch, lti, a, s);
+    if (n <= 32) return launch_grad<32, 1>(h, n, m, N, batch, lti, a, s);
+    if (n <= 64) return launch_grad<32, 2>(h, n, m, N, batch, lti, a, s);
+    if (n <= 96) return launch_grad<32, 3>(h, n, m, N, batch, lti, a, s);
+    return lqrb_fail(h, -2, "n too large for the Riccati gradient sweep");
+}
+
+// Gradient of ℓ(Z) through lqrb_riccati_f64 (DESIGN §4.8): the adjoint LQR (same A, B, Q, R, Qf; linear terms dZ;
+// x̂0 = 0) is packed and solved by the forward dispatch, its solution unpacked to Ẑ, and one backward sweep forms the
+// costates of both problems and every gradient.
+extern "C" int32_t lqrb_riccati_grad_f64(lqrb_handle_t h, int32_t n, int32_t m, int32_t N, int64_t batch,
+                                         int32_t flags, const double *A, const double *B, const double *Q,
+                                         const double *R, const double *q, const double *r, const double *Qf,
+                                         const double *qf, const double *Z, const double *dZ, double *gA, double *gB,
+                                         double *gQ, double *gR, double *gq, double *gr, double *gQf, double *gqf,
+                                         double *gx0, int32_t *info) {
+    int32_t rc = check_dims(h, n, m, N, batch);
+    if (rc) return rc;
+    if (flags & ~(LQRB_FLAG_LTI | LQRB_FLAG_NO_AFFINE)) return lqrb_fail(h, -6, "flags: only LTI and NO_AFFINE apply");
+    if (!A) return lqrb_fail(h, -7, "A is NULL");
+    if (!B) return lqrb_fail(h, -8, "B is NULL");
+    if (!Q) return lqrb_fail(h, -9, "Q is NULL");
+    if (!R) return lqrb_fail(h, -10, "R is NULL");
+    if (!Qf) return lqrb_fail(h, -13, "Qf is NULL");
+    if (!Z) return lqrb_fail(h, -15, "Z is NULL");
+    if (!dZ) return lqrb_fail(h, -16, "dZ is NULL");
+    if (!gA && !gB && !gQ && !gR && !gq && !gr && !gQf && !gqf && !gx0)
+        return lqrb_fail(h, -17, "every gradient output is NULL");
+    if (batch == 0) return 0;
+    LQRB_CUDA(h, cudaSetDevice(h->device));
+    if (flags & LQRB_FLAG_NO_AFFINE) q = r = qf = nullptr;
+
+    const bool lti = (flags & LQRB_FLAG_LTI) != 0;
+    lqrb_riccati_layout_t L;
+    lqrb_riccati_layout(n, m, N, 0, &L);  // the adjoint problem is always packed as LTV
+    const int64_t Kn = lti ? 1 : N - 1, NN = L.z_rows;
+    const int64_t sA = Kn * n * n * 8, sB = Kn * n * m * 8, sR = Kn * m * m * 8, sq = Kn * n * 8, sr = Kn * m * 8,
+                  sQf = (int64_t)n * n * 8, sx = (int64_t)n * 8;
+    return lqrb_for_chunks(
+        h, batch, 0,
+        {{A, sA}, {B, sB}, {Q, sA}, {R, sR}, {q, sq}, {r, sr}, {Qf, sQf}, {qf, sx}, {Z, NN * 8}, {dZ, NN * 8}},
+        {{gA, sA}, {gB, sB}, {gQ, sA}, {gR, sR}, {gq, sq}, {gr, sr}, {gQf, sQf}, {gqf, sx}, {gx0, sx}, {info, 4}},
+        [&](Lane lane, int64_t cb, const void *const *in, void *const *out) -> int32_t {
+            const int64_t ldb = lqrb_padded_batch(cb);
+            double *knots = (double *)lqrb_scratch(h, SCR_PACK_IN, (size_t)ldb * L.knot_count * L.rows_per_knot * 8,
+                                                   lane.index);
+            double *term = (double *)lqrb_scratch(h, SCR_PACK_IN2, (size_t)ldb * L.term_rows * 8, lane.index);
+            double *Zp = (double *)lqrb_scratch(h, SCR_PACK_OUT, (size_t)ldb * NN * 8, lane.index);
+            double *gains = (double *)lqrb_scratch(h, SCR_GAINS, (size_t)ldb * L.gain_rows * 8, lane.index);
+            double *Zh = (double *)lqrb_scratch(h, SCR_ADJOINT_Z, (size_t)cb * NN * 8, lane.index);
+            if (!knots || !term || !Zp || !gains || !Zh) return 1000 + (int)cudaErrorMemoryAllocation;
+            const double *const *a = (const double *const *)in;
+            const int tile = lqrb_riccati_tile(h, n, m);
+            ArrayTable t = {};
+            const double *ptrs[7] = {a[0], a[1], a[2], a[3], a[9], nullptr, a[6]};
+            const int64_t strides[7] = {sA / 8, sB / 8, sA / 8, sR / 8, NN, 0, sQf / 8};
+            for (int i = 0; i < 7; ++i) {
+                t.ptr[i] = ptrs[i];
+                t.stride[i] = strides[i];
+            }
+            DevMap km = lqrb_get_map(h, key("rak", n, m, N, lti ? 1 : 0), riccati_adjoint_knot_map(n, m, N, flags));
+            DevMap tm = lqrb_get_map(h, key("rat", n, m, N, 0), riccati_adjoint_term_map(n, m, N));
+            int32_t rc = lqrb_gather_pack(h, km, t, cb, tile, knots, lane.stream);
+            if (rc) return rc;
+            rc = lqrb_gather_pack(h, tm, t, cb, tile, term, lane.stream);
+            if (rc) return rc;
+            rc = riccati_solve_on(h, n, m, N, cb, 0, knots, term, Zp, gains, (int32_t *)out[9], lane);
+            if (rc) return rc;
+            ArrayTableOut o = {};
+            o.ptr[0] = Zh;
+            o.stride[0] = NN;
+            rc = lqrb_scatter_unpack(h, lqrb_identity_map(h, NN), o, cb, tile, Zp, lane.stream);
+            if (rc) return rc;
+            double *const *g = (double *const *)out;
+            const RiccatiGradArgs ga = {a[0], a[2], a[4], a[6], a[7], a[8], Zh, a[9],
+                                        g[0], g[1], g[2], g[3], g[4], g[5], g[6], g[7], g[8]};
+            return launch_grad_sized(h, n, m, N, cb, lti, ga, lane.stream);
         });
 }
 

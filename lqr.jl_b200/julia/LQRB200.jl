@@ -197,6 +197,28 @@ function rollout!(X::Array{Float64,3}, U::Array{Float64,3}, prob::LQRProblem, ha
     return X
 end
 
+"""riccati_grad!(G, prob, Z, dZ, handle): gradients of a loss l(Z) through solve!(sol, ::DPSolver, prob) from
+dZ = dl/dZ (NN×batch).  G is a NamedTuple (A, B, Q, R, q, r, Qf, qf, x0) of arrays shaped like the problem's (any may
+be `nothing`); returns the potrf info of the adjoint solve per instance."""
+function riccati_grad!(G::NamedTuple, prob::LQRProblem, Z::Matrix{Float64}, dZ::Matrix{Float64}, handle::Handle)
+    n, m, N = size(prob)
+    flags = islti(prob) ? FLAG_LTI : Int32(0)
+    info = zeros(Int32, batchsize(prob))
+    g(x) = x === nothing ? C_NULL : pointer(x)
+    GC.@preserve G prob Z dZ info begin
+        rc = ccall((:lqrb_riccati_grad_f64, lib), Int32,
+            (Ptr{Cvoid}, Int32, Int32, Int32, Int64, Int32, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+             Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+             Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+             Ptr{Float64}, Ptr{Int32}),
+            handle.ptr, n, m, N, batchsize(prob), flags, prob.A, prob.B, prob.Q, prob.R, ptr_or_null(prob.q),
+            ptr_or_null(prob.r), prob.Qf, ptr_or_null(prob.qf), Z, dZ, g(G.A), g(G.B), g(G.Q), g(G.R), g(G.q), g(G.r),
+            g(G.Qf), g(G.qf), g(G.x0), info)
+    end
+    check(handle, rc)
+    return info
+end
+
 # ------------------------------------------------------------------ LeastSquaresSolver (src/least_squares.jl)
 "LeastSquaresSolver(prob): the condensed (block-Toeplitz) form of the unconstrained LTI problem, src/least_squares.jl:1-59"
 struct LeastSquaresSolver
@@ -642,7 +664,7 @@ kkt_unpack!(h::Handle, n, m, N, batch, p::Vector{Int32}, hess_mode, explicit_d2,
          Ptr{Float64}, Ptr{Float64}),
         h.ptr, n, m, N, batch, p, hess_mode, explicit_d2, dzp, multp, resp, dz, mult, res))
 
-export Handle, LQRBError, LQRProblem, LQRSolution, DPSolver, LeastSquaresSolver, solve!, rollout!, num_vars, state, control,
+export Handle, LQRBError, LQRProblem, LQRSolution, DPSolver, LeastSquaresSolver, solve!, rollout!, riccati_grad!, num_vars, state, control,
        BlockCholesky, InvertedQuadratic, update_cost!, update_cholesky!, gradient,
        ConstraintBlock, ConstraintBlocks, dims, copy_blocks!, gen_con_inds,
        CholeskySolver, build_shur_factors, calculate_shur_factors!, forward_substitution!, backward_substitution!,

@@ -29,6 +29,14 @@ def riccati(h: Handle, n, m, N, batch, flags, A, B, Q, R, q, r, Qf, qf, x0, Z, K
            ptr(Qf), ptr(qf), ptr(x0), ptr(Z), ptr(K), ptr(kff), ptr(info))
 
 
+def riccati_grad(h: Handle, n, m, N, batch, flags, A, B, Q, R, q, r, Qf, qf, Z, dZ, gA=None, gB=None, gQ=None,
+                 gR=None, gq=None, gr=None, gQf=None, gqf=None, gx0=None, info=None):
+    """lqrb_riccati_grad_f64: gradients of l(Z) through lqrb_riccati_f64 from dZ = dl/dZ; buffers as riccati()."""
+    h.call("lqrb_riccati_grad_f64", n, m, N, batch, flags, ptr(A), ptr(B), ptr(Q), ptr(R), ptr(q), ptr(r), ptr(Qf),
+           ptr(qf), ptr(Z), ptr(dZ), ptr(gA), ptr(gB), ptr(gQ), ptr(gR), ptr(gq), ptr(gr), ptr(gQf), ptr(gqf), ptr(gx0),
+           ptr(info))
+
+
 def riccati_pack(h: Handle, n, m, N, batch, flags, A, B, Q, R, q, r, Qf, qf, x0, knots, term):
     h.call("lqrb_riccati_pack_f64", n, m, N, batch, flags, ptr(A), ptr(B), ptr(Q), ptr(R), ptr(q), ptr(r),
            ptr(Qf), ptr(qf), ptr(x0), ptr(knots), ptr(term))
@@ -211,6 +219,26 @@ def riccati_solve_problem(prob: dict, want_gains: bool = True, handle: Handle | 
             f["Qf"], f["qf"], f["x0"], Z, K, kff, info)
     X, U = split_primals(Z, n, m, N)
     return X, U, (np.swapaxes(K, -1, -2).copy() if want_gains else None), kff, info
+
+
+def riccati_grad_problem(prob: dict, Z, dZ, handle: Handle | None = None):
+    """Gradients of l(Z) through the solve of a Riccati problem dict, from host memory.  Z is the (b, NN) Primals
+    output of the solve and dZ = dl/dZ of the same shape.  Returns (grads, info): grads holds math-order arrays with
+    the shapes of the problem's A, B, Q, R, q, r, Qf, qf, x0 (keys likewise)."""
+    h = handle or default_handle()
+    f = prob if "batch" in prob else riccati_flatten(prob)
+    n, m, N, b = f["n"], f["m"], f["N"], f["batch"]
+    kn = (b,) if f["lti"] else (b, N - 1)
+    g = dict(A=np.zeros(kn + (n, n)), B=np.zeros(kn + (m, n)), Q=np.zeros(kn + (n, n)), R=np.zeros(kn + (m, m)),
+             q=np.zeros(kn + (n,)), r=np.zeros(kn + (m,)), Qf=np.zeros((b, n, n)), qf=np.zeros((b, n)),
+             x0=np.zeros((b, n)))
+    info = np.zeros(b, dtype=np.int32)
+    riccati_grad(h, n, m, N, b, _lib.FLAG_LTI if f["lti"] else 0, f["A"], f["B"], f["Q"], f["R"], f["q"], f["r"],
+                 f["Qf"], f["qf"], f64(Z), f64(dZ), g["A"], g["B"], g["Q"], g["R"], g["q"], g["r"], g["Qf"], g["qf"],
+                 g["x0"], info)
+    for k in ("A", "B", "Q", "R", "Qf"):  # column-major buffers -> math order
+        g[k] = np.ascontiguousarray(np.swapaxes(g[k], -1, -2))
+    return g, info
 
 
 def split_primals(Z, n, m, N):
