@@ -225,6 +225,29 @@ int32_t lqrb_kkt_solve_f64(lqrb_handle_t handle, int32_t n, int32_t m, int32_t N
                            const double *C, const double *c, double *dz, double *mult, double *res,
                            int32_t *info);
 
+/* Gradient of a scalar loss l(dz, mult) through lqrb_kkt_solve_f64: given the inputs, that call's outputs dz, mult and
+ * the cotangents dz_bar = dl/d dz, mult_bar = dl/d mult (same shapes), writes dl/d of every input.  The same KKT
+ * matrices are solved once more with g := dz_bar and [c; d] := mult_bar, by the same kernels as the forward solve; one
+ * kernel then forms every gradient as outer products of the two solutions (DESIGN §4.9).
+ *   inputs as in lqrb_kkt_solve_f64 (q, r, d, c are not needed); flags must be 0 (-8: LQRB_FLAG_SOC has no gradient);
+ *   dz_bar[NN,batch] | NULL, mult_bar[P,batch] | NULL (zero), not both NULL.
+ *   outputs gQ, gR, gHux, gq, gr, gA, gB, gd, gD2, gC, gc: the shape of their input (gD2, gC, gc: the same ragged
+ *   concatenations); any may be NULL, not all.  gHux needs LQRB_HESS_DENSE, gD2 an explicit D2, gC / gc sum(p) > 0.
+ *   The kernels read only the upper triangle of Q, R (LQRB_HESS_DIAG: the diagonal): their gradients are returned as
+ *   the symmetric matrices (1/2)(x^ x' + x x^'), under LQRB_HESS_DIAG only their diagonal (the rest is 0); a
+ *   finite-difference check perturbs (i,j) and (j,i) together.  gHux = u^ x' + u x^' (the solve reads Hux once).
+ *   info[batch] | NULL: the potrf info of the adjoint solve (the same matrices as the forward solve).  The gradients of
+ *   an instance with info != 0 carry no meaning.  The call leaves the kept factorisation (lqrb_kkt_factor_f64) and the
+ *   record of lqrb_kkt_last_condition as they were.
+ * Host or device pointers, with the staged / device-resident rule of every entry point.                          */
+int32_t lqrb_kkt_grad_f64(lqrb_handle_t handle, int32_t n, int32_t m, int32_t N, int64_t batch,
+                          const int32_t *p, int32_t hess_mode, int32_t flags,
+                          const double *Q, const double *R, const double *Hux, const double *A, const double *B,
+                          const double *D2, const double *C,
+                          const double *dz, const double *mult, const double *dz_bar, const double *mult_bar,
+                          double *gQ, double *gR, double *gHux, double *gq, double *gr, double *gA, double *gB,
+                          double *gd, double *gD2, double *gC, double *gc, int32_t *info);
+
 /* Device-resident split (DEVICE pointers; `data` has lqrb_kkt_data_rows() x ldb doubles). */
 int32_t lqrb_kkt_pack_f64(lqrb_handle_t handle, int32_t n, int32_t m, int32_t N, int64_t batch,
                           const int32_t *p, int32_t hess_mode, const double *Q, const double *R,

@@ -82,6 +82,7 @@ _SIGS = {
     "lqrb_block_cholesky_f64": (c_i32, [c_vp, c_i32, c_i32, c_i64, c_i32] + [c_dp] * 4 + [c_vp]),
     "lqrb_block_ldiv_f64": (c_i32, [c_vp, c_i32, c_i32, c_i64, c_i32, c_dp, c_i32, c_dp]),
     "lqrb_kkt_solve_f64": (c_i32, [c_vp, c_i32, c_i32, c_i32, c_i64, c_vp, c_i32, c_i32] + [c_dp] * 14 + [c_vp]),
+    "lqrb_kkt_grad_f64": (c_i32, [c_vp, c_i32, c_i32, c_i32, c_i64, c_vp, c_i32, c_i32] + [c_dp] * 22 + [c_vp]),
     "lqrb_kkt_pack_f64": (c_i32, [c_vp, c_i32, c_i32, c_i32, c_i64, c_vp, c_i32] + [c_dp] * 12),
     "lqrb_kkt_solve_packed_f64": (c_i32, [c_vp, c_i32, c_i32, c_i32, c_i64, c_vp, c_i32, c_i32, c_i32]
                                   + [c_dp] * 4 + [c_vp]),

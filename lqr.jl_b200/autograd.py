@@ -1,4 +1,4 @@
-"""Differentiable batched Riccati solve for torch (``lqr_b200.autograd``).
+"""Differentiable batched Riccati and constrained KKT solves for torch (``lqr_b200.autograd``).
 
 ``riccati_solve(A, B, Q, R, q, r, Qf, qf, x0, N=None) -> (X, U, info)`` solves the LTV-affine LQR of
 ``lqrb_riccati_f64`` on CUDA float64 tensors in math order and backpropagates through it with
@@ -15,6 +15,18 @@ non-symmetric inputs too.  ``info`` is the potrf info of the solve (0 = ok) and 
 of an instance with info != 0 carry no meaning.  The calls run on the current torch stream and do not synchronise;
 calls on different streams are ordered one after another (they share the device's handle).
 There is no CPU path: CPU tensors raise.
+
+``kkt_solve(Q, R, q, r, A, B, d, C, c, Hux=None, D2=None, hess_mode=HESS_BLOCKDIAG) -> (X, U, mult, info)`` solves the
+constrained KKT system of ``lqrb_kkt_solve_f64`` and backpropagates through it with ``lqrb_kkt_grad_f64``: one more
+solve of the same KKT matrices with the cotangents as right-hand side, then one kernel that forms the gradients.
+
+Shapes (math order, batch first):
+    Q (b, N, n, n)  R (b, N-1, m, m)  q (b, N, n)  r (b, N-1, m)  A (b, N-1, n, n)  B (b, N-1, n, m)  d (b, N-1, n)
+    C, c: lists of N tensors C_k (b, p_k, w_k), c_k (b, p_k) with w_k = n + m (w_N = n); p is read from their shapes
+    Hux (b, N-1, m, n) (LQRB_HESS_DENSE)   D2: None (D2_k = [-I 0]) or a list of N-1 tensors (b, n, w_k), k = 2..N
+    ->  X (b, N, n), U (b, N-1, m), mult (b, P) in the order [mu_1; lam_1; ...; mu_N], info (b,) int32
+Batch broadcasting, the symmetrisation of Q and R (under HESS_DIAG only their diagonals are read and receive gradient),
+``info``, streams and the CPU rule are as for ``riccati_solve``.
 """
 from __future__ import annotations
 
@@ -23,7 +35,7 @@ from torch.autograd.function import once_differentiable
 
 from . import _lib, ops
 
-__all__ = ["riccati_solve"]
+__all__ = ["riccati_solve", "kkt_solve"]
 
 
 def _cm(a):
@@ -120,3 +132,74 @@ def riccati_solve(A, B, Q, R, q, r, Qf, qf, x0, N: int | None = None):
         return t.expand((b,) + tuple(t.shape[1:])).contiguous()
     return _RiccatiSolve.apply(int(N), full(A), full(B), full(Q, True), full(R, True), full(q), full(r),
                                full(Qf, True), full(qf), full(x0))
+
+
+class _KktSolve(torch.autograd.Function):
+    """On the ABI's instance-major buffers (column-major blocks, ragged arrays concatenated): kkt_solve lays the
+    arguments out with differentiable torch operations, so the gradients of this function need no reshaping."""
+
+    @staticmethod
+    def forward(ctx, dims, p, Q, R, Hux, q, r, A, B, d, D2, C, c):
+        n, m, N, b, hess = dims
+        dz = torch.empty(b, _lib.num_vars(n, m, N), dtype=torch.float64, device=Q.device)
+        mult = torch.empty(b, _lib.num_cons(n, N, p), dtype=torch.float64, device=Q.device)
+        info = torch.empty(b, dtype=torch.int32, device=Q.device)
+        with torch.cuda.device(Q.device):
+            ops.kkt_solve(_handle(Q.device), n, m, N, b, p, hess, 0, Q, R, Hux, q, r, A, B, d, D2, C, c, dz, mult,
+                          None, info)
+        ctx.save_for_backward(*[a if a is not None else torch.empty(0) for a in (Q, R, Hux, A, B, D2, C)], dz, mult)
+        ctx.absent = (Hux is None, D2 is None)
+        ctx.shapes = [None if t is None else t.shape for t in (Q, R, Hux, q, r, A, B, d, D2, C, c)]
+        ctx.dims, ctx.p = dims, p
+        ctx.mark_non_differentiable(info)
+        return dz, mult, info
+
+    @staticmethod
+    @once_differentiable  # double backward is not provided: create_graph=True raises instead of returning constants
+    def backward(ctx, ddz, dmult, _dinfo):
+        n, m, N, b, hess = ctx.dims
+        Q, R, Hux, A, B, D2, C, dz, mult = ctx.saved_tensors
+        Hux, D2 = (None if gone else t for t, gone in zip((Hux, D2), ctx.absent))
+        rows = C.shape[1] > 0
+        # an absent input, Hux outside LQRB_HESS_DENSE and C, c without stage rows get no gradient
+        have = [s is not None for s in ctx.shapes]
+        have[2] = have[2] and hess == _lib.HESS_DENSE
+        have[9] = have[10] = rows
+        g = [dz.new_empty(s) if (w and h) else None for s, w, h in zip(ctx.shapes, ctx.needs_input_grad[2:], have)]
+        if all(x is None for x in g) or (ddz is None and dmult is None):
+            return (None,) * 13
+        with torch.cuda.device(dz.device):
+            ops.kkt_grad(_handle(dz.device), n, m, N, b, ctx.p, hess, 0, Q, R, Hux, A, B, D2, C if rows else None, dz,
+                         mult, ddz.contiguous() if ddz is not None else None,
+                         dmult.contiguous() if dmult is not None else None, *g)
+        return (None, None, *g)
+
+
+def kkt_solve(Q, R, q, r, A, B, d, C, c, Hux=None, D2=None, hess_mode=_lib.HESS_BLOCKDIAG):
+    """Differentiable batched constrained KKT solve; see the module docstring."""
+    C, c, D2 = list(C), list(c), (None if D2 is None else list(D2))
+    ts = [Q, R, q, r, A, B, d, *C, *c] + ([Hux] if Hux is not None else []) + (D2 or [])
+    for t in ts:
+        if not (t.is_cuda and t.dtype == torch.float64):
+            raise TypeError("kkt_solve takes CUDA float64 tensors (there is no CPU path)")
+    N, n, m = Q.shape[1], Q.shape[-1], R.shape[-1]
+    if len(C) != N or len(c) != N or (D2 is not None and len(D2) != N - 1):
+        raise ValueError("C and c need N blocks, D2 N-1")
+    p = [int(Ck.shape[-2]) for Ck in C]
+    b = max(t.shape[0] for t in ts)
+
+    def full(t, sym=False):
+        if sym:
+            t = 0.5 * (t + t.transpose(-1, -2))
+        return t.expand((b,) + tuple(t.shape[1:]))
+
+    def flat(blocks):  # per-knot math-order blocks -> the ABI's concatenation of column-major blocks
+        return torch.cat([_cm(full(x)).reshape(b, -1) for x in blocks], dim=1).contiguous()
+    dz, mult, info = _KktSolve.apply(
+        (n, m, N, b, int(hess_mode)), p, _cm(full(Q, True)), _cm(full(R, True)),
+        None if Hux is None else _cm(full(Hux)), full(q).contiguous(), full(r).contiguous(), _cm(full(A)),
+        _cm(full(B)), full(d).contiguous(), None if D2 is None else flat(D2), flat(C),
+        torch.cat([full(x) for x in c], dim=1).contiguous())
+    body = dz[:, :(N - 1) * (n + m)].view(b, N - 1, n + m)
+    X = torch.cat([body[:, :, :n], dz[:, None, (N - 1) * (n + m):]], dim=1)
+    return X, body[:, :, n:].contiguous(), mult, info

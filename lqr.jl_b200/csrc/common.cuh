@@ -56,7 +56,9 @@ enum ScratchSlot {
     SCR_REFINE,       // records of the instances re-solved by the Cholesky-based kernel (ill-conditioned blocks)
     SCR_REFINE_LIST,  // their indices
     SCR_RICCATI_PAD,  // Riccati problems embedded in a tuned size class: padded knots, term, Z, gains
-    SCR_ADJOINT_Z,    // lqrb_riccati_grad_f64: the adjoint solution, instance-major (read by the gradient sweep)
+    SCR_ADJOINT_Z,    // lqrb_riccati_grad_f64 / lqrb_kkt_grad_f64: the adjoint solution, instance-major (read by the
+                      // gradient kernels)
+    SCR_ADJOINT_MULT, // lqrb_kkt_grad_f64: the adjoint multipliers, instance-major
     SCR_COUNT
 };
 

@@ -3,6 +3,7 @@
 #include <cstdio>
 
 #include "kkt_dispatch.cuh"
+#include "kkt_grad_kernels.cuh"
 
 // ------------------------------------------------------------------ routing -------------------
 // Shapes each family has an instantiation for (kkt_dispatch.cuh) and whose stage pattern it handles.
@@ -730,6 +731,167 @@ extern "C" int32_t lqrb_kkt_solve_f64(lqrb_handle_t h, int32_t n, int32_t m, int
     if (rc) return rc;
     kkt_keep_record(h, record);
     return 0;
+}
+
+// ------------------------------------------------------------------ gradient ------------------
+// The adjoint problem of lqrb_kkt_grad_f64 (DESIGN §4.9): the forward matrices, with g taken from dz_bar (Primals
+// order) and d, c from mult_bar (order [mu_1; lam_1; ...; mu_N]).  Source ids as kkt_data_map with 3 = dz_bar and
+// 7 = mult_bar (4 and 10 unused); a NULL source packs zeros.
+static std::vector<RowMap> kkt_adjoint_data_map(const KktShape &s) {
+    const int n = s.n, m = s.m;
+    std::vector<int32_t> lam((size_t)s.N), mu_of_c;  // multiplier offset of lam_k | of each row of the concatenated c
+    int32_t off = 0;
+    for (int k = 0; k < s.N; ++k) {
+        for (int e = 0; e < s.p[k]; ++e) mu_of_c.push_back(off + e);
+        off += s.p[k];
+        lam[(size_t)k] = off;
+        if (k < s.N - 1) off += n;
+    }
+    std::vector<RowMap> map = kkt_data_map(s);
+    for (RowMap &r : map) {
+        const int32_t o = r.offset;
+        if (r.array == 3) r = RowMap{3, o / n * (n + m) + o % n, 0.0};  // q_k(i) -> x_k(i)
+        else if (r.array == 4) r = RowMap{3, o / m * (n + m) + n + o % m, 0.0};  // r_k(i) -> u_k(i)
+        else if (r.array == 7) r = RowMap{7, lam[(size_t)(o / n)] + o % n, 0.0};
+        else if (r.array == 10) r = RowMap{7, mu_of_c[(size_t)o], 0.0};
+    }
+    return map;
+}
+
+// per-knot offset tables of the gradient kernel (KktGradTables), built once per shape
+static int32_t kkt_grad_tables(lqrb_context *h, const KktShape &s, KktGradTables *t) {
+    const int n = s.n, m = s.m, N = s.N;
+    const std::string key = shape_key("kgrad", s);
+    auto it = h->blobs.find(key);
+    int32_t *d = nullptr;
+    if (it != h->blobs.end()) {
+        d = (int32_t *)it->second;
+    } else {
+        std::vector<int32_t> host(5 * (size_t)(N + 1), 0);
+        int32_t *mu = host.data(), *lam = mu + N + 1, *C = lam + N + 1, *c = C + N + 1, *D2 = c + N + 1;
+        for (int k = 0; k < N; ++k) {
+            const int w = n + (k < N - 1 ? m : 0);
+            lam[k] = mu[k] + s.p[k];
+            mu[k + 1] = lam[k] + (k < N - 1 ? n : 0);
+            C[k + 1] = C[k] + s.p[k] * w;
+            c[k + 1] = c[k] + s.p[k];
+            if (k > 0) D2[k + 1] = D2[k] + n * w;
+        }
+        lam[N] = mu[N];
+        LQRB_CUDA(h, cudaMalloc(&d, host.size() * sizeof(int32_t)));
+        LQRB_CUDA(h, cudaMemcpy(d, host.data(), host.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
+        LQRB_CUDA(h, cudaStreamSynchronize(cudaStreamLegacy));  // pageable source: wait for the staged DMA
+        h->blobs[key] = d;
+    }
+    *t = KktGradTables{d, d + (N + 1), d + 2 * (N + 1), d + 3 * (N + 1), d + 4 * (N + 1)};
+    return 0;
+}
+
+// Gradient of l(dz, mult) through lqrb_kkt_solve_f64 (DESIGN §4.9): the adjoint problem (same matrices, right-hand
+// side from the cotangents) is packed and solved by the forward dispatch, its solution unpacked to instance-major
+// scratch, and kkt_grad_kernel forms every requested gradient from the two solutions.  The adjoint solve's
+// conditioning record is dropped: lqrb_kkt_last_condition keeps describing the last forward solve.
+extern "C" int32_t lqrb_kkt_grad_f64(lqrb_handle_t h, int32_t n, int32_t m, int32_t N, int64_t batch,
+                                     const int32_t *p, int32_t hess_mode, int32_t flags, const double *Q,
+                                     const double *R, const double *Hux, const double *A, const double *B,
+                                     const double *D2, const double *C, const double *dz, const double *mult,
+                                     const double *dz_bar, const double *mult_bar, double *gQ, double *gR,
+                                     double *gHux, double *gq, double *gr, double *gA, double *gB, double *gd,
+                                     double *gD2, double *gC, double *gc, int32_t *info) {
+    int32_t rc = check_kkt(h, n, m, N, batch, p, hess_mode);
+    if (rc) return rc;
+    if (flags & LQRB_FLAG_SOC) return lqrb_fail(h, -8, "flags: the gradient of the second-order correction is not provided");
+    if (flags) return lqrb_fail(h, -8, "flags must be 0");
+    if (!Q) return lqrb_fail(h, -9, "Q is NULL");
+    if (!R) return lqrb_fail(h, -10, "R is NULL");
+    if (!A) return lqrb_fail(h, -12, "A is NULL");
+    if (!B) return lqrb_fail(h, -13, "B is NULL");
+    const KktShape s = make_shape(n, m, N, p, hess_mode, D2 != nullptr);
+    const KktSizes z = kkt_sizes(s);
+    if (z.sC > 0 && !C) return lqrb_fail(h, -15, "C is NULL but p has non-zero entries");
+    if (!dz) return lqrb_fail(h, -16, "dz is NULL");
+    if (!mult) return lqrb_fail(h, -17, "mult is NULL");
+    if (!dz_bar && !mult_bar) return lqrb_fail(h, -18, "dz_bar and mult_bar are both NULL");
+    double *const g[KG_COUNT] = {gQ, gR, gHux, gq, gr, gA, gB, gd, gD2, gC, gc};
+    if (std::all_of(g, g + KG_COUNT, [](double *x) { return x == nullptr; }))
+        return lqrb_fail(h, -20, "every gradient output is NULL");
+    if (gHux && hess_mode != LQRB_HESS_DENSE) return lqrb_fail(h, -22, "gHux needs LQRB_HESS_DENSE");
+    if (gD2 && !D2) return lqrb_fail(h, -28, "gD2 needs an explicit D2");
+    if (gC && z.sC == 0) return lqrb_fail(h, -29, "gC: p has no rows");
+    if (gc && z.sc == 0) return lqrb_fail(h, -30, "gc: p has no rows");
+    const int64_t K1 = N - 1;
+    const int64_t per[KG_COUNT] = {(int64_t)n * n * N, (int64_t)m * m * K1, (int64_t)m * n * K1, (int64_t)n * N,
+                                   (int64_t)m * K1,    (int64_t)n * n * K1, (int64_t)n * m * K1, (int64_t)n * K1,
+                                   z.sD2,              z.sC,                z.sc};
+    for (int o = 0; o < KG_COUNT; ++o)  // the kernel indexes an instance's elements in 31 bits
+        if (g[o] && per[o] > (1ll << 30)) return lqrb_fail(h, -2, "n, m, N too large for the gradient kernel");
+    if (batch == 0) return 0;
+    LQRB_CUDA(h, cudaSetDevice(h->device));
+
+    // inputs 0..10 in kkt_adjoint_data_map's source order, then the forward solution
+    const std::vector<HostArray> inputs = {
+        {Q, per[KG_Q] * 8},       {R, per[KG_R] * 8},           {Hux, Hux ? per[KG_HUX] * 8 : 0},
+        {dz_bar, z.NN * 8},       {nullptr, 0},                 {A, per[KG_A] * 8},
+        {B, per[KG_B] * 8},       {mult_bar, z.P * 8},          {D2, D2 ? z.sD2 * 8 : 0},
+        {C, z.sC * 8},            {nullptr, 0},                 {dz, z.NN * 8},
+        {mult, z.P * 8}};
+    std::vector<HostArray> outputs;
+    for (int o = 0; o < KG_COUNT; ++o) outputs.push_back({g[o], per[o] * 8});
+    outputs.push_back({info, 4});
+    KktGradTables tables;
+    rc = kkt_grad_tables(h, s, &tables);
+    if (rc) return rc;
+    const std::string mkey = shape_key("kadj", s);
+    auto mit = h->maps.find(mkey);
+    const DevMap amap = mit != h->maps.end() ? mit->second : lqrb_get_map(h, mkey, kkt_adjoint_data_map(s));
+    return lqrb_for_chunks(
+        h, batch, 0, inputs, outputs, [&](Lane lane, int64_t cb, const void *const *in, void *const *out) -> int32_t {
+            const int64_t ldb = lqrb_padded_batch(cb);
+            double *data = (double *)lqrb_scratch(h, SCR_PACK_IN, (size_t)ldb * z.data_rows * 8, lane.index);
+            double *dzp = (double *)lqrb_scratch(h, SCR_PACK_OUT, (size_t)ldb * z.NN * 8, lane.index);
+            double *mp = (double *)lqrb_scratch(h, SCR_PACK_OUT2, (size_t)ldb * z.P * 8, lane.index);
+            double *scr = (double *)lqrb_scratch(h, SCR_FACT, kkt_scratch_bytes(h, s, z, cb), lane.index);
+            double *zh = (double *)lqrb_scratch(h, SCR_ADJOINT_Z, (size_t)cb * z.NN * 8, lane.index);
+            double *mh = (double *)lqrb_scratch(h, SCR_ADJOINT_MULT, (size_t)cb * z.P * 8, lane.index);
+            if (!data || !dzp || !mp || !scr || !zh || !mh) return 1000 + (int)cudaErrorMemoryAllocation;
+            const int tile = lqrb_kkt_tile(h, n, m, N, p, hess_mode, s.d2x);
+            int32_t rc = lqrb_gather_pack(h, amap, kkt_array_table(inputs, in), cb, tile, data, lane.stream);
+            if (rc) return rc;
+            KktRecord record;
+            rc = kkt_solve_on(h, s, cb, 0, data, scr, dzp, mp, nullptr, (int32_t *)out[KG_COUNT], lane, &record);
+            if (rc) return rc;
+            rc = kkt_unpack_on(h, s, z, cb, dzp, mp, nullptr, zh, mh, nullptr, lane.stream);
+            if (rc) return rc;
+            KktGradArgs a = {};
+            a.z = (const double *)in[11];
+            a.mult = (const double *)in[12];
+            a.zh = zh;
+            a.multh = mh;
+            a.t = tables;
+            int64_t blocks = 0;
+            for (int o = 0; o < KG_COUNT; ++o) {
+                if (!out[o]) continue;
+                a.kind[a.nout] = o;
+                a.out[a.nout] = (double *)out[o];
+                a.per[a.nout] = kkt_grad_div((uint32_t)per[o]);
+                a.first_block[a.nout] = blocks;
+                blocks += (cb * per[o] + KKT_GRAD_THREADS * KKT_GRAD_PER_THREAD - 1) / (KKT_GRAD_THREADS * KKT_GRAD_PER_THREAD);
+                ++a.nout;
+            }
+            a.first_block[a.nout] = blocks;
+            a.n = kkt_grad_div((uint32_t)n);
+            a.m = kkt_grad_div((uint32_t)m);
+            a.nn = kkt_grad_div((uint32_t)(n * n));
+            a.mm = kkt_grad_div((uint32_t)(m * m));
+            a.nm = kkt_grad_div((uint32_t)(n * m));
+            a.NN = (int32_t)z.NN;
+            a.P = (int32_t)z.P;
+            a.diag = hess_mode == LQRB_HESS_DIAG;
+            kkt_grad_kernel<<<(unsigned)blocks, KKT_GRAD_THREADS, 0, lane.stream>>>(a, n, m, N, cb);
+            h->kernel_name += " + kkt_grad";
+            LQRB_LAUNCH_CHECK(h, "kkt_grad_kernel");
+            return 0;
+        });
 }
 
 

@@ -451,6 +451,30 @@ function _call_kkt!(s::CholeskySolver, flags::Int32)
     return s
 end
 
+"""kkt_grad!(G, solver, dZ̄, λ̄): gradients of a loss l(δZ, λ) through the last _solve!(solver) (δZ, λ as it left
+them) from dZ̄ = dl/dδZ (NN×batch) and λ̄ = dl/dλ (P×batch); either may be `nothing`, not both.  G is a NamedTuple
+(Q, R, Hux, q, r, A, B, d, D2, C, c) of arrays shaped like the solver's (any may be `nothing`); returns the potrf info
+of the adjoint solve per instance."""
+function kkt_grad!(G::NamedTuple, s::CholeskySolver, dZ̄::Union{Nothing,Matrix{Float64}},
+                   λ̄::Union{Nothing,Matrix{Float64}})
+    info = zeros(Int32, batchsize(s))
+    g(x) = x === nothing ? C_NULL : pointer(x)
+    GC.@preserve G s dZ̄ λ̄ info begin
+        rc = ccall((:lqrb_kkt_grad_f64, lib), Int32,
+            (Ptr{Cvoid}, Int32, Int32, Int32, Int64, Ptr{Int32}, Int32, Int32,
+             Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+             Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+             Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+             Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Int32}),
+            s.handle.ptr, s.n, s.m, s.N, batchsize(s), s.p, s.hess_mode, Int32(0),
+            s.Q, s.R, ptr_or_null(s.Hux), s.A, s.B, ptr_or_null(s.D2), s.C,
+            s.δZ, s.λ, g(dZ̄), g(λ̄),
+            g(G.Q), g(G.R), g(G.Hux), g(G.q), g(G.r), g(G.A), g(G.B), g(G.d), g(G.D2), g(G.C), g(G.c), info)
+    end
+    check(s.handle, rc)
+    return info
+end
+
 "_solve!(solver): src/cholesky_solver.jl:166-182 — the five steps in ONE fused kernel launch"
 _solve!(s::CholeskySolver) = (s.Ginv = true; _call_kkt!(s, Int32(0)))
 "second_order_correction!: src/cholesky_solver.jl:254-273 (the Ginv=false chain)"
@@ -664,7 +688,8 @@ kkt_unpack!(h::Handle, n, m, N, batch, p::Vector{Int32}, hess_mode, explicit_d2,
          Ptr{Float64}, Ptr{Float64}),
         h.ptr, n, m, N, batch, p, hess_mode, explicit_d2, dzp, multp, resp, dz, mult, res))
 
-export Handle, LQRBError, LQRProblem, LQRSolution, DPSolver, LeastSquaresSolver, solve!, rollout!, riccati_grad!, num_vars, state, control,
+export Handle, LQRBError, LQRProblem, LQRSolution, DPSolver, LeastSquaresSolver, solve!, rollout!, riccati_grad!, kkt_grad!, num_vars,
+       state, control,
        BlockCholesky, InvertedQuadratic, update_cost!, update_cholesky!, gradient,
        ConstraintBlock, ConstraintBlocks, dims, copy_blocks!, gen_con_inds,
        CholeskySolver, build_shur_factors, calculate_shur_factors!, forward_substitution!, backward_substitution!,

@@ -94,6 +94,17 @@ def kkt_solve(h: Handle, n, m, N, batch, p, hess_mode, flags, Q, R, Hux, q, r, A
            ptr(info))
 
 
+def kkt_grad(h: Handle, n, m, N, batch, p, hess_mode, flags, Q, R, Hux, A, B, D2, C, dz, mult, dz_bar, mult_bar,
+             gQ=None, gR=None, gHux=None, gq=None, gr=None, gA=None, gB=None, gd=None, gD2=None, gC=None, gc=None,
+             info=None):
+    """lqrb_kkt_grad_f64: gradients of l(dz, mult) through lqrb_kkt_solve_f64 from the cotangents dz_bar, mult_bar;
+    buffers as kkt_solve()."""
+    p = _p32(p)
+    h.call("lqrb_kkt_grad_f64", n, m, N, batch, p.ctypes.data, hess_mode, flags, ptr(Q), ptr(R), ptr(Hux), ptr(A),
+           ptr(B), ptr(D2), ptr(C), ptr(dz), ptr(mult), ptr(dz_bar), ptr(mult_bar), ptr(gQ), ptr(gR), ptr(gHux),
+           ptr(gq), ptr(gr), ptr(gA), ptr(gB), ptr(gd), ptr(gD2), ptr(gC), ptr(gc), ptr(info))
+
+
 def kkt_pack(h: Handle, n, m, N, batch, p, hess_mode, Q, R, Hux, q, r, A, B, d, D2, C, c, data):
     p = _p32(p)
     h.call("lqrb_kkt_pack_f64", n, m, N, batch, p.ctypes.data, hess_mode, ptr(Q), ptr(R), ptr(Hux), ptr(q),
@@ -195,6 +206,39 @@ def kkt_solve_problem(prob: dict, soc: bool = False, want_res: bool = False, han
     kkt_solve(h, n, m, N, b, f["p"], f["hess_mode"], _lib.FLAG_SOC if soc else 0, f["Q"], f["R"], f["Hux"],
               f["q"], f["r"], f["A"], f["B"], f["d"], f["D2"], f["C"], f["c"], dz, mult, res, info)
     return (dz, mult, info, res) if want_res else (dz, mult, info)
+
+
+def kkt_grad_problem(prob: dict, dz, mult, dz_bar, mult_bar, handle: Handle | None = None):
+    """Gradients of l(dz, mult) through the solve of a math-order KKT problem dict, from host memory.  dz (b, NN) and
+    mult (b, P) are the outputs of the solve, dz_bar and mult_bar the cotangents of the same shapes (either may be
+    None).  Returns (grads, info): grads holds math-order arrays with the shapes of the problem's Q, R, Hux, q, r, A,
+    B, d, D2, C, c (keys likewise; D2, C, c are per-knot lists, Hux and D2 None where the problem has none)."""
+    h = handle or default_handle()
+    f = kkt_flatten(prob)
+    n, m, N, b, p, mode = f["n"], f["m"], f["N"], f["batch"], f["p"], f["hess_mode"]
+    dense = mode == _lib.HESS_DENSE
+    g = dict(Q=np.zeros((b, N, n, n)), R=np.zeros((b, N - 1, m, m)), Hux=np.zeros((b, N - 1, n, m)) if dense else None,
+             q=np.zeros((b, N, n)), r=np.zeros((b, N - 1, m)), A=np.zeros((b, N - 1, n, n)),
+             B=np.zeros((b, N - 1, m, n)), d=np.zeros((b, N - 1, n)),
+             D2=np.zeros_like(f["D2"]) if f["D2"] is not None else None,
+             C=np.zeros_like(f["C"]) if f["C"].shape[1] else None, c=np.zeros_like(f["c"]) if f["c"].shape[1] else None)
+    info = np.zeros(b, dtype=np.int32)
+    kkt_grad(h, n, m, N, b, p, mode, 0, f["Q"], f["R"], f["Hux"], f["A"], f["B"], f["D2"], f["C"], f64(dz), f64(mult),
+             f64(dz_bar), f64(mult_bar), g["Q"], g["R"], g["Hux"], g["q"], g["r"], g["A"], g["B"], g["d"], g["D2"],
+             g["C"], g["c"], info)
+    for k in ("Q", "R", "Hux", "A", "B"):  # column-major buffers -> math order
+        if g[k] is not None:
+            g[k] = np.ascontiguousarray(np.swapaxes(g[k], -1, -2))
+    ws = [n + (m if k < N - 1 else 0) for k in range(N)]
+    if g["D2"] is not None:  # blocks n x w_k, k = 2..N
+        cuts = np.cumsum([n * w for w in ws[1:]])[:-1]
+        g["D2"] = [np.swapaxes(x.reshape(b, w, n), -1, -2).copy() for x, w in zip(np.split(g["D2"], cuts, axis=1), ws[1:])]
+    Cf = g["C"] if g["C"] is not None else np.zeros((b, 0))
+    cf = g["c"] if g["c"] is not None else np.zeros((b, 0))
+    Cs = np.split(Cf, np.cumsum([int(pk) * w for pk, w in zip(p, ws)])[:-1], axis=1)
+    g["C"] = [np.swapaxes(x.reshape(b, w, int(pk)), -1, -2).copy() for x, w, pk in zip(Cs, ws, p)]
+    g["c"] = [x.copy() for x in np.split(cf, np.cumsum(p)[:-1], axis=1)]
+    return g, info
 
 
 def riccati_flatten(prob: dict) -> dict:
