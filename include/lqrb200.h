@@ -153,6 +153,25 @@ int32_t lqrb_riccati_grad_f64(lqrb_handle_t handle, int32_t n, int32_t m, int32_
                               double *gQ, double *gR, double *gq, double *gr, double *gQf, double *gqf,
                               double *gx0, int32_t *info);
 
+/* Gradient of a scalar loss l(Z, K, kff) through lqrb_riccati_f64, the policy outputs included: given the inputs,
+ * that call's Z and the cotangents dZ = dl/dZ, dK = dl/dK, dkff = dl/dkff, writes the total dl/d of every input.  The
+ * Z part is lqrb_riccati_grad_f64's; the gains part recomputes the recursion into a per-knot tape and runs its adjoint
+ * forward over the knots (DESIGN §4.10).
+ *   inputs and outputs as in lqrb_riccati_grad_f64; dK[m,n,N-1,batch], dkff[m,N-1,batch] in the layout of the forward
+ *   call's K, kff.  dZ, dK, dkff may each be NULL, not all three; Z is read only when dZ is given.  With dZ = NULL, gx0
+ *   is written as zeros (the gains do not depend on x0).  With dK = dkff = NULL the result is bitwise that of
+ *   lqrb_riccati_grad_f64.
+ *   info[batch] | NULL: 0, or the forward solve's code for the first failed factorisation.
+ *   Error codes: -6 flags other than LTI / NO_AFFINE; -7..-10, -13 A, B, Q, R or Qf NULL; -15 Z NULL while dZ is
+ *   given; -16 every cotangent NULL; -19 every output NULL; shapes the solve rejects with the solve's code.
+ * Host or device pointers, with the staged / device-resident rule of every entry point.                      */
+int32_t lqrb_riccati_grad_gains_f64(lqrb_handle_t handle, int32_t n, int32_t m, int32_t N, int64_t batch,
+                                    int32_t flags, const double *A, const double *B, const double *Q,
+                                    const double *R, const double *q, const double *r, const double *Qf,
+                                    const double *qf, const double *Z, const double *dZ, const double *dK,
+                                    const double *dkff, double *gA, double *gB, double *gQ, double *gR, double *gq,
+                                    double *gr, double *gQf, double *gqf, double *gx0, int32_t *info);
+
 /* Device-resident split of the same call (all pointers are DEVICE pointers). */
 int32_t lqrb_riccati_pack_f64(lqrb_handle_t handle, int32_t n, int32_t m, int32_t N, int64_t batch,
                               int32_t flags, const double *A, const double *B, const double *Q,

@@ -3,7 +3,9 @@
 ``riccati_solve(A, B, Q, R, q, r, Qf, qf, x0, N=None) -> (X, U, info)`` solves the LTV-affine LQR of
 ``lqrb_riccati_f64`` on CUDA float64 tensors in math order and backpropagates through it with
 ``lqrb_riccati_grad_f64``: the adjoint of an LQR is another LQR with the same matrices, so the backward pass is one
-more solve on the same kernels plus one sweep that forms the gradients.
+more solve on the same kernels plus one sweep that forms the gradients.  With ``gains=True`` it returns
+``(X, U, K, kff, info)``, the policy u_k = -K_k x_k - kff_k included (K (b, N-1, m, n), kff (b, N-1, m)), and
+backpropagates through all four outputs with ``lqrb_riccati_grad_gains_f64``.
 
 Shapes (math order, batch first):
     LTV:  A (b, N-1, n, n)  B (b, N-1, n, m)  Q (b, N-1, n, n)  R (b, N-1, m, m)  q (b, N-1, n)  r (b, N-1, m)
@@ -66,49 +68,63 @@ def _handle(device: torch.device) -> _lib.Handle:
 
 class _RiccatiSolve(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, N, A, B, Q, R, q, r, Qf, qf, x0):
+    def forward(ctx, N, A, B, Q, R, q, r, Qf, qf, x0, gains=False):
         b, n, m = x0.shape[0], A.shape[-1], B.shape[-1]
         flags = _lib.FLAG_LTI if A.dim() == 3 else 0
         args = [_cm(A), _cm(B), _cm(Q), _cm(R), q, r, _cm(Qf), qf]
         Z = torch.empty(b, _lib.num_vars(n, m, N), dtype=torch.float64, device=x0.device)
         info = torch.empty(b, dtype=torch.int32, device=x0.device)
+        K = torch.empty(b, N - 1, n, m, dtype=torch.float64, device=x0.device) if gains else None  # column-major m x n
+        kff = torch.empty(b, N - 1, m, dtype=torch.float64, device=x0.device) if gains else None
         with torch.cuda.device(x0.device):
-            ops.riccati(_handle(x0.device), n, m, N, b, flags, *args, x0, Z, None, None, info)
+            ops.riccati(_handle(x0.device), n, m, N, b, flags, *args, x0, Z, K, kff, info)
         ctx.save_for_backward(*[a if a is not None else torch.empty(0) for a in args], Z)
         ctx.has_affine = (q is not None, r is not None, qf is not None)
         ctx.dims = (n, m, N, b, flags)
+        ctx.gains = gains
         ctx.mark_non_differentiable(info)
         body = Z[:, :(N - 1) * (n + m)].view(b, N - 1, n + m)
         X = torch.cat([body[:, :, :n], Z[:, None, (N - 1) * (n + m):]], dim=1)
+        if gains:
+            ctx.set_materialize_grads(False)  # an unused output's cotangent stays None and costs no work
+            return X, body[:, :, n:].contiguous(), K.transpose(-1, -2), kff, info
         return X, body[:, :, n:].contiguous(), info
 
     @staticmethod
     @once_differentiable  # double backward is not provided: create_graph=True raises instead of returning constants
-    def backward(ctx, dX, dU, _dinfo):
+    def backward(ctx, dX, dU, *rest):
         n, m, N, b, flags = ctx.dims
         A, B, Q, R, q, r, Qf, qf, Z = ctx.saved_tensors
         q, r, qf = (a if has else None for a, has in zip((q, r, qf), ctx.has_affine))
-        dZ = torch.zeros_like(Z)
-        body = dZ[:, :(N - 1) * (n + m)].view(b, N - 1, n + m)
-        if dX is not None:
-            body[:, :, :n] = dX[:, :N - 1]
-            dZ[:, (N - 1) * (n + m):] = dX[:, N - 1]
-        if dU is not None:
-            body[:, :, n:] = dU
-        want = ctx.needs_input_grad[1:]
-        if not any(want):
-            return (None,) * 10
+        dK, dkff = rest[:2] if ctx.gains else (None, None)
+        want = ctx.needs_input_grad[1:10]
+        if not any(want) or (ctx.gains and dX is None and dU is None and dK is None and dkff is None):
+            return (None,) * 11
+        dZ = None
+        if not ctx.gains or dX is not None or dU is not None:
+            dZ = torch.zeros_like(Z)
+            body = dZ[:, :(N - 1) * (n + m)].view(b, N - 1, n + m)
+            if dX is not None:
+                body[:, :, :n] = dX[:, :N - 1]
+                dZ[:, (N - 1) * (n + m):] = dX[:, N - 1]
+            if dU is not None:
+                body[:, :, n:] = dU
         like = (A, B, Q, R, q, r, Qf, qf, Z.new_empty(b, n))  # an absent q, r, qf needs no gradient
         g = [torch.empty_like(t) if w else None for t, w in zip(like, want)]
         with torch.cuda.device(Z.device):
-            ops.riccati_grad(_handle(Z.device), n, m, N, b, flags, A, B, Q, R, q, r, Qf, qf, Z, dZ, *g)
+            if ctx.gains:
+                ops.riccati_grad_gains(_handle(Z.device), n, m, N, b, flags, A, B, Q, R, q, r, Qf, qf, Z, dZ,
+                                       None if dK is None else _cm(dK), None if dkff is None else dkff.contiguous(),
+                                       *g)
+            else:
+                ops.riccati_grad(_handle(Z.device), n, m, N, b, flags, A, B, Q, R, q, r, Qf, qf, Z, dZ, *g)
         for i in (0, 1, 2, 3, 6):  # column-major buffers -> math order
             if g[i] is not None:
                 g[i] = g[i].transpose(-1, -2)
-        return (None, *g)
+        return (None, *g, None)
 
 
-def riccati_solve(A, B, Q, R, q, r, Qf, qf, x0, N: int | None = None):
+def riccati_solve(A, B, Q, R, q, r, Qf, qf, x0, N: int | None = None, gains: bool = False):
     """Differentiable batched LQR solve; see the module docstring."""
     ts = [t for t in (A, B, Q, R, q, r, Qf, qf, x0) if t is not None]
     for t in ts:
@@ -131,7 +147,7 @@ def riccati_solve(A, B, Q, R, q, r, Qf, qf, x0, N: int | None = None):
             t = 0.5 * (t + t.transpose(-1, -2))
         return t.expand((b,) + tuple(t.shape[1:])).contiguous()
     return _RiccatiSolve.apply(int(N), full(A), full(B), full(Q, True), full(R, True), full(q), full(r),
-                               full(Qf, True), full(qf), full(x0))
+                               full(Qf, True), full(qf), full(x0), bool(gains))
 
 
 class _KktSolve(torch.autograd.Function):

@@ -59,6 +59,7 @@ enum ScratchSlot {
     SCR_ADJOINT_Z,    // lqrb_riccati_grad_f64 / lqrb_kkt_grad_f64: the adjoint solution, instance-major (read by the
                       // gradient kernels)
     SCR_ADJOINT_MULT, // lqrb_kkt_grad_f64: the adjoint multipliers, instance-major
+    SCR_GAIN_TAPE,    // lqrb_riccati_grad_gains_f64: P_{k+1}, p_{k+1}, K_k, kff_k and the factor of G_k per knot
     SCR_COUNT
 };
 

@@ -6,6 +6,7 @@
 #include "riccati_dmma_kernels.cuh"
 #include "riccati_cta_kernels.cuh"
 #include "riccati_grad_kernels.cuh"
+#include "riccati_gain_grad_kernels.cuh"
 
 // ------------------------------------------------------------------ routing -------------------
 // The sizes with a kernel of their own, by family: Tpi thread per instance (registers only), Dmma warp per instance on
@@ -570,9 +571,52 @@ static int32_t launch_grad_sized(lqrb_context *h, int n, int m, int N, int64_t b
     return lqrb_fail(h, -2, "n too large for the Riccati gradient sweep");
 }
 
-// Gradient of ℓ(Z) through lqrb_riccati_f64 (DESIGN §4.8): the adjoint LQR (same A, B, Q, R, Qf; linear terms dZ;
-// x̂0 = 0) is packed and solved by the forward dispatch, its solution unpacked to Ẑ, and one backward sweep forms the
-// costates of both problems and every gradient.
+// Gradient of ℓ(Z) through lqrb_riccati_f64 for one chunk (DESIGN §4.8): the adjoint LQR (same A, B, Q, R, Qf; linear
+// terms dZ; x̂0 = 0) is packed and solved by the forward dispatch, its solution unpacked to Ẑ, and one backward sweep
+// forms the costates of both problems and every gradient.  `in` holds A, B, Q, R, q, r, Qf, qf, Z, dZ and `out` gA, gB,
+// gQ, gR, gq, gr, gQf, gqf, gx0, info, as chunk pointers of lqrb_for_chunks.
+static int32_t riccati_grad_chunk(lqrb_context *h, int n, int m, int N, int flags, Lane lane, int64_t cb,
+                                  const void *const *in, void *const *out) {
+    const bool lti = (flags & LQRB_FLAG_LTI) != 0;
+    lqrb_riccati_layout_t L;
+    lqrb_riccati_layout(n, m, N, 0, &L);  // the adjoint problem is always packed as LTV
+    const int64_t Kn = lti ? 1 : N - 1, NN = L.z_rows;
+    const int64_t sA = Kn * n * n, sB = Kn * n * m, sR = Kn * m * m, sQf = (int64_t)n * n;
+    const int64_t ldb = lqrb_padded_batch(cb);
+    double *knots = (double *)lqrb_scratch(h, SCR_PACK_IN, (size_t)ldb * L.knot_count * L.rows_per_knot * 8, lane.index);
+    double *term = (double *)lqrb_scratch(h, SCR_PACK_IN2, (size_t)ldb * L.term_rows * 8, lane.index);
+    double *Zp = (double *)lqrb_scratch(h, SCR_PACK_OUT, (size_t)ldb * NN * 8, lane.index);
+    double *gains = (double *)lqrb_scratch(h, SCR_GAINS, (size_t)ldb * L.gain_rows * 8, lane.index);
+    double *Zh = (double *)lqrb_scratch(h, SCR_ADJOINT_Z, (size_t)cb * NN * 8, lane.index);
+    if (!knots || !term || !Zp || !gains || !Zh) return 1000 + (int)cudaErrorMemoryAllocation;
+    const double *const *a = (const double *const *)in;
+    const int tile = lqrb_riccati_tile(h, n, m);
+    ArrayTable t = {};
+    const double *ptrs[7] = {a[0], a[1], a[2], a[3], a[9], nullptr, a[6]};
+    const int64_t strides[7] = {sA, sB, sA, sR, NN, 0, sQf};
+    for (int i = 0; i < 7; ++i) {
+        t.ptr[i] = ptrs[i];
+        t.stride[i] = strides[i];
+    }
+    DevMap km = lqrb_get_map(h, key("rak", n, m, N, lti ? 1 : 0), riccati_adjoint_knot_map(n, m, N, flags));
+    DevMap tm = lqrb_get_map(h, key("rat", n, m, N, 0), riccati_adjoint_term_map(n, m, N));
+    int32_t rc = lqrb_gather_pack(h, km, t, cb, tile, knots, lane.stream);
+    if (rc) return rc;
+    rc = lqrb_gather_pack(h, tm, t, cb, tile, term, lane.stream);
+    if (rc) return rc;
+    rc = riccati_solve_on(h, n, m, N, cb, 0, knots, term, Zp, gains, (int32_t *)out[9], lane);
+    if (rc) return rc;
+    ArrayTableOut o = {};
+    o.ptr[0] = Zh;
+    o.stride[0] = NN;
+    rc = lqrb_scatter_unpack(h, lqrb_identity_map(h, NN), o, cb, tile, Zp, lane.stream);
+    if (rc) return rc;
+    double *const *g = (double *const *)out;
+    const RiccatiGradArgs ga = {a[0], a[2], a[4], a[6], a[7], a[8], Zh, a[9],
+                                g[0], g[1], g[2], g[3], g[4], g[5], g[6], g[7], g[8]};
+    return launch_grad_sized(h, n, m, N, cb, lti, ga, lane.stream);
+}
+
 extern "C" int32_t lqrb_riccati_grad_f64(lqrb_handle_t h, int32_t n, int32_t m, int32_t N, int64_t batch,
                                          int32_t flags, const double *A, const double *B, const double *Q,
                                          const double *R, const double *q, const double *r, const double *Qf,
@@ -595,10 +639,7 @@ extern "C" int32_t lqrb_riccati_grad_f64(lqrb_handle_t h, int32_t n, int32_t m, 
     LQRB_CUDA(h, cudaSetDevice(h->device));
     if (flags & LQRB_FLAG_NO_AFFINE) q = r = qf = nullptr;
 
-    const bool lti = (flags & LQRB_FLAG_LTI) != 0;
-    lqrb_riccati_layout_t L;
-    lqrb_riccati_layout(n, m, N, 0, &L);  // the adjoint problem is always packed as LTV
-    const int64_t Kn = lti ? 1 : N - 1, NN = L.z_rows;
+    const int64_t Kn = (flags & LQRB_FLAG_LTI) ? 1 : N - 1, NN = lqrb_num_vars(n, m, N);
     const int64_t sA = Kn * n * n * 8, sB = Kn * n * m * 8, sR = Kn * m * m * 8, sq = Kn * n * 8, sr = Kn * m * 8,
                   sQf = (int64_t)n * n * 8, sx = (int64_t)n * 8;
     return lqrb_for_chunks(
@@ -606,40 +647,126 @@ extern "C" int32_t lqrb_riccati_grad_f64(lqrb_handle_t h, int32_t n, int32_t m, 
         {{A, sA}, {B, sB}, {Q, sA}, {R, sR}, {q, sq}, {r, sr}, {Qf, sQf}, {qf, sx}, {Z, NN * 8}, {dZ, NN * 8}},
         {{gA, sA}, {gB, sB}, {gQ, sA}, {gR, sR}, {gq, sq}, {gr, sr}, {gQf, sQf}, {gqf, sx}, {gx0, sx}, {info, 4}},
         [&](Lane lane, int64_t cb, const void *const *in, void *const *out) -> int32_t {
-            const int64_t ldb = lqrb_padded_batch(cb);
-            double *knots = (double *)lqrb_scratch(h, SCR_PACK_IN, (size_t)ldb * L.knot_count * L.rows_per_knot * 8,
-                                                   lane.index);
-            double *term = (double *)lqrb_scratch(h, SCR_PACK_IN2, (size_t)ldb * L.term_rows * 8, lane.index);
-            double *Zp = (double *)lqrb_scratch(h, SCR_PACK_OUT, (size_t)ldb * NN * 8, lane.index);
-            double *gains = (double *)lqrb_scratch(h, SCR_GAINS, (size_t)ldb * L.gain_rows * 8, lane.index);
-            double *Zh = (double *)lqrb_scratch(h, SCR_ADJOINT_Z, (size_t)cb * NN * 8, lane.index);
-            if (!knots || !term || !Zp || !gains || !Zh) return 1000 + (int)cudaErrorMemoryAllocation;
-            const double *const *a = (const double *const *)in;
-            const int tile = lqrb_riccati_tile(h, n, m);
-            ArrayTable t = {};
-            const double *ptrs[7] = {a[0], a[1], a[2], a[3], a[9], nullptr, a[6]};
-            const int64_t strides[7] = {sA / 8, sB / 8, sA / 8, sR / 8, NN, 0, sQf / 8};
-            for (int i = 0; i < 7; ++i) {
-                t.ptr[i] = ptrs[i];
-                t.stride[i] = strides[i];
+            return riccati_grad_chunk(h, n, m, N, flags, lane, cb, in, out);
+        });
+}
+
+// ------------------------------------------------------------------ gradient through the gains -----
+// Instances per block of riccati_gain_grad_kernel<G>: up to 128 threads, as many groups as their shared-memory slices
+// allow, in whole warps; 0 when one warp's groups do not fit.
+static int gain_grad_groups(int G, int n, int m) {
+    const size_t per = (size_t)gain_grad_smem_doubles(n, m) * sizeof(double), cap = 227 * 1024;
+    const int whole = 32 / G;  // groups per warp
+    const int groups = (int)std::min<size_t>(128 / G, cap / per) / whole * whole;
+    return groups;
+}
+
+template <int G, int R>
+static int32_t launch_gain_grad(lqrb_context *h, int n, int m, int N, int64_t batch, bool lti,
+                                const RiccatiGainGradArgs &a, cudaStream_t s) {
+    const int groups = gain_grad_groups(G, n, m);
+    if (groups == 0) return lqrb_fail(h, -2, "n, m too large for the gain gradient sweep");
+    const size_t smem = (size_t)gain_grad_smem_doubles(n, m) * sizeof(double) * groups;
+    const unsigned grid = (unsigned)((batch + groups - 1) / groups);
+    auto kern = lti ? riccati_gain_grad_kernel<G, R, true> : riccati_gain_grad_kernel<G, R, false>;
+    LQRB_CUDA(h, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kern<<<grid, groups * G, smem, s>>>(a, n, m, N, batch);
+    char nm[64];
+    snprintf(nm, sizeof nm, "riccati_gain_grad<G=%d,R=%d>%s", G, R, lti ? "[lti]" : "");
+    h->kernel_name = h->kernel_name.empty() ? std::string(nm) : h->kernel_name + " + " + nm;
+    LQRB_LAUNCH_CHECK(h, "riccati_gain_grad_kernel");
+    return 0;
+}
+
+// the lane configuration of riccati_grad_kernel (launch_grad_sized): lanes per instance and rows per lane
+static void gain_grad_lanes(int n, int *G, int *R) {
+    *G = n <= 4 ? 4 : n <= 8 ? 8 : n <= 16 ? 16 : 32;
+    *R = n <= 32 ? 1 : n <= 64 ? 2 : 3;
+}
+
+static int32_t launch_gain_grad_sized(lqrb_context *h, int n, int m, int N, int64_t batch, bool lti,
+                                      const RiccatiGainGradArgs &a, cudaStream_t s) {
+    if (n <= 4) return launch_gain_grad<4, 1>(h, n, m, N, batch, lti, a, s);
+    if (n <= 8) return launch_gain_grad<8, 1>(h, n, m, N, batch, lti, a, s);
+    if (n <= 16) return launch_gain_grad<16, 1>(h, n, m, N, batch, lti, a, s);
+    if (n <= 32) return launch_gain_grad<32, 1>(h, n, m, N, batch, lti, a, s);
+    if (n <= 64) return launch_gain_grad<32, 2>(h, n, m, N, batch, lti, a, s);
+    if (n <= 96) return launch_gain_grad<32, 3>(h, n, m, N, batch, lti, a, s);
+    return lqrb_fail(h, -2, "n too large for the gain gradient sweep");
+}
+
+// The code lqrb_riccati_f64 returns for a shape it cannot solve (0 when it can): only the cooperative kernel at
+// n + m > 24 has a size limit, its shared memory (launch_coop).
+static int32_t riccati_size_code(lqrb_context *h, int n, int m) {
+    if (riccati_route(h, n, m, true).family == RiccatiFamily::Coop && n + m > 24 &&
+        riccati_coop_smem_doubles(n, m) * sizeof(double) > 227 * 1024)
+        return lqrb_fail(h, -2, "n,m too large for the shared-memory Riccati kernel");
+    return 0;
+}
+
+// Gradient of ℓ(Z, K, kff) through lqrb_riccati_f64 (DESIGN §4.10): the Z part is lqrb_riccati_grad_f64's chunk body
+// (or zeroed outputs without dZ), then riccati_gain_grad_kernel recomputes the recursion into a per-knot tape and
+// adds the adjoint of the recursion driven by dK, dkff.
+extern "C" int32_t lqrb_riccati_grad_gains_f64(lqrb_handle_t h, int32_t n, int32_t m, int32_t N, int64_t batch,
+                                               int32_t flags, const double *A, const double *B, const double *Q,
+                                               const double *R, const double *q, const double *r, const double *Qf,
+                                               const double *qf, const double *Z, const double *dZ, const double *dK,
+                                               const double *dkff, double *gA, double *gB, double *gQ, double *gR,
+                                               double *gq, double *gr, double *gQf, double *gqf, double *gx0,
+                                               int32_t *info) {
+    int32_t rc = check_dims(h, n, m, N, batch);
+    if (rc) return rc;
+    if (flags & ~(LQRB_FLAG_LTI | LQRB_FLAG_NO_AFFINE)) return lqrb_fail(h, -6, "flags: only LTI and NO_AFFINE apply");
+    if (!A) return lqrb_fail(h, -7, "A is NULL");
+    if (!B) return lqrb_fail(h, -8, "B is NULL");
+    if (!Q) return lqrb_fail(h, -9, "Q is NULL");
+    if (!R) return lqrb_fail(h, -10, "R is NULL");
+    if (!Qf) return lqrb_fail(h, -13, "Qf is NULL");
+    if (dZ && !Z) return lqrb_fail(h, -15, "Z is NULL while dZ is given");
+    if (!dZ && !dK && !dkff) return lqrb_fail(h, -16, "every cotangent (dZ, dK, dkff) is NULL");
+    if (!gA && !gB && !gQ && !gR && !gq && !gr && !gQf && !gqf && !gx0)
+        return lqrb_fail(h, -19, "every gradient output is NULL");
+    if (batch == 0) return 0;
+    LQRB_CUDA(h, cudaSetDevice(h->device));
+    if (flags & LQRB_FLAG_NO_AFFINE) q = r = qf = nullptr;
+    if (!dZ) Z = nullptr;
+    if (!dZ && (rc = riccati_size_code(h, n, m))) return rc;
+
+    const bool lti = (flags & LQRB_FLAG_LTI) != 0;
+    const int64_t Kn = lti ? 1 : N - 1, NN = lqrb_num_vars(n, m, N);
+    const int64_t sA = Kn * n * n * 8, sB = Kn * n * m * 8, sR = Kn * m * m * 8, sq = Kn * n * 8, sr = Kn * m * 8,
+                  sQf = (int64_t)n * n * 8, sx = (int64_t)n * 8;
+    const int64_t sK = (int64_t)(N - 1) * m * n * 8, skff = (int64_t)(N - 1) * m * 8;
+    int G, Rr;
+    gain_grad_lanes(n, &G, &Rr);
+    const int groups = std::max(1, gain_grad_groups(G, n, m));
+    return lqrb_for_chunks(
+        h, batch, 0,
+        {{A, sA}, {B, sB}, {Q, sA}, {R, sR}, {q, sq}, {r, sr}, {Qf, sQf}, {qf, sx}, {Z, NN * 8}, {dZ, NN * 8},
+         {dK, sK}, {dkff, skff}},
+        {{gA, sA}, {gB, sB}, {gQ, sA}, {gR, sR}, {gq, sq}, {gr, sr}, {gQf, sQf}, {gqf, sx}, {gx0, sx}, {info, 4}},
+        [&](Lane lane, int64_t cb, const void *const *in, void *const *out) -> int32_t {
+            int32_t rc = 0;
+            h->kernel_name.clear();
+            if (dZ) {
+                rc = riccati_grad_chunk(h, n, m, N, flags, lane, cb, in, out);
+                if (rc) return rc;
+            } else {
+                const int64_t bytes[10] = {sA, sB, sA, sR, sq, sr, sQf, sx, sx, 4};
+                for (int i = 0; i < 10; ++i)
+                    if (out[i]) LQRB_CUDA(h, cudaMemsetAsync(out[i], 0, (size_t)(cb * bytes[i]), lane.stream));
             }
-            DevMap km = lqrb_get_map(h, key("rak", n, m, N, lti ? 1 : 0), riccati_adjoint_knot_map(n, m, N, flags));
-            DevMap tm = lqrb_get_map(h, key("rat", n, m, N, 0), riccati_adjoint_term_map(n, m, N));
-            int32_t rc = lqrb_gather_pack(h, km, t, cb, tile, knots, lane.stream);
-            if (rc) return rc;
-            rc = lqrb_gather_pack(h, tm, t, cb, tile, term, lane.stream);
-            if (rc) return rc;
-            rc = riccati_solve_on(h, n, m, N, cb, 0, knots, term, Zp, gains, (int32_t *)out[9], lane);
-            if (rc) return rc;
-            ArrayTableOut o = {};
-            o.ptr[0] = Zh;
-            o.stride[0] = NN;
-            rc = lqrb_scatter_unpack(h, lqrb_identity_map(h, NN), o, cb, tile, Zp, lane.stream);
-            if (rc) return rc;
+            if (!dK && !dkff) return 0;
+            const int64_t slots = round_up(cb, groups);  // groups past the batch write a slot of their own
+            double *tape = (double *)lqrb_scratch(h, SCR_GAIN_TAPE,
+                                                  (size_t)slots * (N - 1) * gain_grad_tape_doubles(n, m) * 8,
+                                                  lane.index);
+            if (!tape) return 1000 + (int)cudaErrorMemoryAllocation;
+            const double *const *a = (const double *const *)in;
             double *const *g = (double *const *)out;
-            const RiccatiGradArgs ga = {a[0], a[2], a[4], a[6], a[7], a[8], Zh, a[9],
-                                        g[0], g[1], g[2], g[3], g[4], g[5], g[6], g[7], g[8]};
-            return launch_grad_sized(h, n, m, N, cb, lti, ga, lane.stream);
+            const RiccatiGainGradArgs ga = {a[0], a[1], a[2], a[3], a[4], a[5], a[6], a[7], a[10], a[11], tape,
+                                            g[0], g[1], g[2], g[3], g[4], g[5], g[6], g[7], (int32_t *)out[9]};
+            return launch_gain_grad_sized(h, n, m, N, cb, lti, ga, lane.stream);
         });
 }
 

@@ -219,6 +219,31 @@ function riccati_grad!(G::NamedTuple, prob::LQRProblem, Z::Matrix{Float64}, dZ::
     return info
 end
 
+"""riccati_grad_gains!(G, prob, Z, dZ, dK, dkff, handle): gradients of a loss l(Z, K, kff) through
+solve!(sol, ::DPSolver, prob), the gains included, from dZ = dl/dZ (NN×batch), dK = dl/dK (m×n×(N-1)×batch) and
+dkff = dl/dkff (m×(N-1)×batch).  Any cotangent may be `nothing`, not all three (Z is read only with dZ).  G as in
+riccati_grad!; returns the info of the solve per instance."""
+function riccati_grad_gains!(G::NamedTuple, prob::LQRProblem, Z::Union{Nothing,Matrix{Float64}},
+                             dZ::Union{Nothing,Matrix{Float64}}, dK::Union{Nothing,Array{Float64,4}},
+                             dkff::Union{Nothing,Array{Float64,3}}, handle::Handle)
+    n, m, N = size(prob)
+    flags = islti(prob) ? FLAG_LTI : Int32(0)
+    info = zeros(Int32, batchsize(prob))
+    g(x) = x === nothing ? C_NULL : pointer(x)
+    GC.@preserve G prob Z dZ dK dkff info begin
+        rc = ccall((:lqrb_riccati_grad_gains_f64, lib), Int32,
+            (Ptr{Cvoid}, Int32, Int32, Int32, Int64, Int32, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+             Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+             Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+             Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Int32}),
+            handle.ptr, n, m, N, batchsize(prob), flags, prob.A, prob.B, prob.Q, prob.R, ptr_or_null(prob.q),
+            ptr_or_null(prob.r), prob.Qf, ptr_or_null(prob.qf), g(Z), g(dZ), g(dK), g(dkff), g(G.A), g(G.B), g(G.Q),
+            g(G.R), g(G.q), g(G.r), g(G.Qf), g(G.qf), g(G.x0), info)
+    end
+    check(handle, rc)
+    return info
+end
+
 # ------------------------------------------------------------------ LeastSquaresSolver (src/least_squares.jl)
 "LeastSquaresSolver(prob): the condensed (block-Toeplitz) form of the unconstrained LTI problem, src/least_squares.jl:1-59"
 struct LeastSquaresSolver
@@ -688,7 +713,7 @@ kkt_unpack!(h::Handle, n, m, N, batch, p::Vector{Int32}, hess_mode, explicit_d2,
          Ptr{Float64}, Ptr{Float64}),
         h.ptr, n, m, N, batch, p, hess_mode, explicit_d2, dzp, multp, resp, dz, mult, res))
 
-export Handle, LQRBError, LQRProblem, LQRSolution, DPSolver, LeastSquaresSolver, solve!, rollout!, riccati_grad!, kkt_grad!, num_vars,
+export Handle, LQRBError, LQRProblem, LQRSolution, DPSolver, LeastSquaresSolver, solve!, rollout!, riccati_grad!, riccati_grad_gains!, kkt_grad!, num_vars,
        state, control,
        BlockCholesky, InvertedQuadratic, update_cost!, update_cholesky!, gradient,
        ConstraintBlock, ConstraintBlocks, dims, copy_blocks!, gen_con_inds,
