@@ -612,7 +612,9 @@ static int32_t riccati_grad_chunk(lqrb_context *h, int n, int m, int N, int flag
     rc = lqrb_scatter_unpack(h, lqrb_identity_map(h, NN), o, cb, tile, Zp, lane.stream);
     if (rc) return rc;
     double *const *g = (double *const *)out;
-    const RiccatiGradArgs ga = {a[0], a[2], a[4], a[6], a[7], a[8], Zh, a[9],
+    // the sweep reads K_k from the adjoint solve's gains (the adjoint problem has the forward A, B, Q, R, Qf, so the
+    // same K_k), in the solve's packed layout: tiled for the thread-per-instance family, instance-major otherwise
+    const RiccatiGradArgs ga = {a[0], a[1], a[2], a[3], a[4], a[5], a[6], a[7], a[8], Zh, a[9], gains, tile,
                                 g[0], g[1], g[2], g[3], g[4], g[5], g[6], g[7], g[8]};
     return launch_grad_sized(h, n, m, N, cb, lti, ga, lane.stream);
 }

@@ -25,10 +25,11 @@ SHAPES = [("cartpole_ltv", 4, 1, 101, 65536, False), ("cartpole_lti", 4, 1, 101,
 
 
 def grad_kernel_bytes(n, m, N, batch, lti):
-    """what the sweep must move: reads A, Q, q per knot (Kn of them), Qf, qf, Z, Z^, dZ; writes every gradient"""
+    """what the sweep must move: reads A, B, Q, R, q, r per knot (Kn of them), K_k for every knot, Qf, qf, Z, Z^, dZ;
+    writes every gradient"""
     Kn = 1 if lti else N - 1
     NN = N * n + (N - 1) * m
-    reads = (N - 1) * (2 * n * n + n) + n * n + n + 3 * NN if not lti else 2 * n * n + n + n * n + n + 3 * NN
+    reads = Kn * (2 * n * n + n * m + m * m + n + m) + (N - 1) * m * n + n * n + n + 3 * NN
     writes = Kn * (2 * n * n + n * m + m * m + n + m) + n * n + 2 * n
     return 8 * batch * (reads + writes)
 
