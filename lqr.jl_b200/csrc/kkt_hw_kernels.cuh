@@ -643,7 +643,8 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
         } else {
             dp = 0.0;
         }
-        // exact symmetrisation: block transpose by shuffle (an antisymmetric residue is amplified by |A|^2 per knot)
+        // exact symmetrisation: block transpose by shuffle (keeps Cp, which the next knot inverts as an SPD block,
+        // exactly symmetric; on unstable A the averaging is not what keeps the sweep accurate, see DESIGN §2)
         SM_UNROLL
         for (int r = 0; r < bs; ++r)
             SM_UNROLL

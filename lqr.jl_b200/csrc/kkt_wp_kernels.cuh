@@ -579,7 +579,8 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
             if (lane < 16) vec[VV + lane] = xslot >= 0 ? rr : 0.0;
         }
         product<3, true>(Gm, Zm, T, -1.0);  // X = G - Z T_x' (upper tiles)
-        // Cp = symmetrised X (an antisymmetric rounding residue is amplified by |A|^2 per knot)
+        // Cp = symmetrised X: the diagonal tiles averaged with their transposes, tile (1,0) the transpose of tile (0,1)
+        // (the product forms upper tiles only); see DESIGN §2 for what the averaging does on unstable A
         Cp.v[0][0][0] = 0.5 * Gm.v[0][0][0];
         Cp.v[0][0][1] = 0.5 * Gm.v[0][0][1];
         transpose8(Cp.v[0][0], Gm.v[0][0], 0.5, g, q);

@@ -11,7 +11,8 @@ C_k z_k + c_k = 0 and lam_k of D1_k z_k + D2_{k+1} z_{k+1} + d_k = 0; hats likew
     dA_k = lam^_k x_k' + lam_k x^_k'            dB_k = lam^_k u_k' + lam_k u^_k'
     dC_k = mu^_k z_k' + mu_k z^_k'              dD2_{k+1} = lam^_k z_{k+1}' + lam_k z^_{k+1}'   (explicit D2)
 
-Both solves are the extended-precision refined solve, one instance at a time.  Everything is math order; the keys
+Both solves are the extended-precision refined solve, one instance at a time, unless ``sols`` gives them: a list of
+(z, mult, z^, nu^) per instance (for example from another solver, to measure what its error does to the gradient).  Everything is math order; the keys
 and shapes are those of the problem dict (D2, C, c: per-knot lists; Hux, D2: None where the problem has none).
 """
 from __future__ import annotations
@@ -21,8 +22,9 @@ import numpy as np
 from . import dense_kkt
 
 
-def kkt_grad(prob: dict, dz_bar=None, mult_bar=None):
-    """Gradients for every instance of a math-order KKT problem dict; dz_bar (b, NN), mult_bar (b, P), either None."""
+def kkt_grad(prob: dict, dz_bar=None, mult_bar=None, sols=None):
+    """Gradients for every instance of a math-order KKT problem dict; dz_bar (b, NN), mult_bar (b, P), either None;
+    sols: the forward and adjoint solutions per instance in place of the refined solves."""
     n, m, N = prob["n"], prob["m"], prob["N"]
     p = [int(x) for x in prob["p"]]
     mode = int(prob.get("hess_mode", 1))
@@ -37,9 +39,12 @@ def kkt_grad(prob: dict, dz_bar=None, mult_bar=None):
              d=np.zeros((b, N - 1, n)), D2=[np.zeros((b, n, ws[k])) for k in range(1, N)] if explicit else None,
              C=[np.zeros((b, p[k], ws[k])) for k in range(N)], c=[np.zeros((b, p[k])) for k in range(N)])
     for i in range(b):
-        H, gv, D, dv = dense_kkt.assemble(prob, i)
-        z, mult = dense_kkt.solve_refined(H, gv, D, dv)
-        zh, mh = dense_kkt.solve_refined(H, dzb[i], D, mb[i])
+        if sols is None:
+            H, gv, D, dv = dense_kkt.assemble(prob, i)
+            z, mult = dense_kkt.solve_refined(H, gv, D, dv)
+            zh, mh = dense_kkt.solve_refined(H, dzb[i], D, mb[i])
+        else:
+            z, mult, zh, mh = sols[i]
         zs = [z[k * (n + m):k * (n + m) + ws[k]] for k in range(N)]
         zhs = [zh[k * (n + m):k * (n + m) + ws[k]] for k in range(N)]
         mus, lams, muhs, lamhs, off = [], [], [], [], 0

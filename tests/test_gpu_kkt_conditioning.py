@@ -60,7 +60,7 @@ FAMILIES = [
 ]
 FAMILY_IDS = [f"{f[6].rstrip(',')}-{f[0]}x{f[1]}-ps{f[3]}-h{f[4]}" + (f"-{f[5]}" if f[5] else "") +
               ("-padded" if f[8] else "") + ("-" + ",".join(f[7]) if f[7] else "") for f in FAMILIES]
-DEFAULTS = {"kkt_variant": 0, "kkt_pad": 1}
+DEFAULTS = {"kkt_variant": 0, "kkt_pad": 1, "kkt_refine": 1}
 
 # c stops at 1e-4 and 1e-3: beyond, the refined solve no longer agrees with a 40-digit one (tests/test_oracle.py)
 PARALLEL = [(c, rs) for c in (1e-2, 1e-3, 1e-4) for rs in (1e-4, 1e-6, 1e-8)]
