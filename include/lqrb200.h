@@ -211,6 +211,38 @@ int32_t lqrb_lsq_solve_f64(lqrb_handle_t handle, int32_t n, int32_t m, int32_t N
                            const double *A, const double *B, const double *Q, const double *R,
                            const double *Qf, const double *x0, double *Z, int32_t *info);
 
+/* ---------------------------------------------------------------- DARE ---------------------- */
+/* The discrete algebraic Riccati equation of the infinite-horizon LQR,  P = Q + A'PA - A'PB (R + B'PB)^-1 B'PA,  its
+ * stabilising solution P and stationary gain K = (R + B'PB)^-1 B'PA (u = -K x, the sign of lqrb_riccati_f64), by the
+ * structured doubling algorithm: quadratic convergence, 7-10 doubling steps on the benchmark draws (DESIGN §4.11).
+ * P is the terminal cost Qf that makes a finite-horizon lqrb_riccati_f64 consistent with its stage cost.
+ *   A[n,n,batch] B[n,m,batch] Q[n,n,batch] R[m,m,batch] (instance-major, column-major; only the upper triangles of Q
+ *   and R are read), 1 <= n <= 64, 1 <= m <= n.
+ *   -> P[n,n,batch] (both triangles) | NULL, K[m,n,batch] | NULL (not both NULL), iters[batch] | NULL (doubling steps
+ *   taken), info[batch] | NULL.
+ *   Stopping rule: ||dH||_F <= 2^-52 ||H||_F for the increment dH of the last step, at most 64 steps.
+ *   info: 0 ok; 1 not converged within 64 steps (no stabilising solution, or a NaN / Inf input); 1000 + j R not positive
+ *   definite at pivot j; 2000 + j a zero pivot at column j of W = I + G_k H_k; 3000 + j R + B'PB not positive definite
+ *   at pivot j (formed when K is requested).  A failed instance's P and K are NaN; the other instances are not affected.
+ *   Error codes: -2 n, -3 m, -4 batch, -5..-8 A, B, Q, R NULL, -9 P and K both NULL.
+ * Host or device pointers, with the staged / device-resident rule of every entry point.                         */
+int32_t lqrb_dare_f64(lqrb_handle_t handle, int32_t n, int32_t m, int64_t batch, const double *A, const double *B,
+                      const double *Q, const double *R, double *P, double *K, int32_t *iters, int32_t *info);
+
+/* Gradient of a scalar loss l(P, K) through lqrb_dare_f64: given A, B, R, that call's P and the cotangents dP = dl/dP
+ * [n,n,batch], dK = dl/dK [m,n,batch] (either may be NULL, not both), writes dl/dA, dl/dB, dl/dQ, dl/dR in the shapes
+ * of the inputs (any may be NULL, not all).  K and R + B'PB are rebuilt from P (its upper triangle is read).  One
+ * Stein equation Y = Acl Y Acl' + S (Acl = A - BK) is solved by Smith doubling with the stopping rule of
+ * lqrb_dare_f64, the gradients are products of Y, P, K (DESIGN §4.11).  gQ and gR are returned as the symmetric
+ * matrices (Q and R enter through their upper triangles); a finite-difference check perturbs (i,j) and (j,i) together.
+ *   info: 0 ok; 1 the Stein doubling did not converge (rho(Acl) >= 1: P is not stabilising); 3000 + j R + B'PB not
+ *   positive definite at pivot j.  A failed instance's gradients are NaN.
+ *   Error codes: -2 n, -3 m, -4 batch, -5..-8 A, B, R, P NULL, -9 dP and dK both NULL, -11 every output NULL.
+ * Host or device pointers, with the staged / device-resident rule of every entry point.                         */
+int32_t lqrb_dare_grad_f64(lqrb_handle_t handle, int32_t n, int32_t m, int64_t batch, const double *A,
+                           const double *B, const double *R, const double *P, const double *dP, const double *dK,
+                           double *gA, double *gB, double *gQ, double *gR, int32_t *info);
+
 /* ---------------------------------------------------------------- BlockCholesky ------------- */
 /* Replaces cholesky!(chol, A, B[, C]) : src/block_cholesky.jl:55-91.  Instance-major:
  *   A[n,n,batch] B[m,m,batch] C[m,n,batch] (C NULL unless DENSE) -> M[(n+m),(n+m),batch]

@@ -79,6 +79,8 @@ _SIGS = {
     "lqrb_kkt_tile_width": (c_i32, [c_vp, c_i32, c_i32, c_i32, c_vp, c_i32, c_i32]),
     "lqrb_kkt_unpack_f64": (c_i32, [c_vp, c_i32, c_i32, c_i32, c_i64, c_vp, c_i32, c_i32] + [c_dp] * 6),
     "lqrb_rollout_f64": (c_i32, [c_vp, c_i32, c_i32, c_i32, c_i64, c_i32] + [c_dp] * 5),
+    "lqrb_dare_f64": (c_i32, [c_vp, c_i32, c_i32, c_i64] + [c_dp] * 6 + [c_vp, c_vp]),
+    "lqrb_dare_grad_f64": (c_i32, [c_vp, c_i32, c_i32, c_i64] + [c_dp] * 10 + [c_vp]),
     "lqrb_lsq_solve_f64": (c_i32, [c_vp, c_i32, c_i32, c_i32, c_i64] + [c_dp] * 7 + [c_vp]),
     "lqrb_block_cholesky_f64": (c_i32, [c_vp, c_i32, c_i32, c_i64, c_i32] + [c_dp] * 4 + [c_vp]),
     "lqrb_block_ldiv_f64": (c_i32, [c_vp, c_i32, c_i32, c_i64, c_i32, c_dp, c_i32, c_dp]),

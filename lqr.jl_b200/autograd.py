@@ -29,6 +29,15 @@ Shapes (math order, batch first):
     ->  X (b, N, n), U (b, N-1, m), mult (b, P) in the order [mu_1; lam_1; ...; mu_N], info (b,) int32
 Batch broadcasting, the symmetrisation of Q and R (under HESS_DIAG only their diagonals are read and receive gradient),
 ``info``, streams and the CPU rule are as for ``riccati_solve``.
+
+``dare_solve(A, B, Q, R) -> (P, K, info)`` solves the discrete algebraic Riccati equation of the infinite-horizon LQR
+with ``lqrb_dare_f64`` (structured doubling) and backpropagates through P and K with ``lqrb_dare_grad_f64`` (one Stein
+equation).  A (b, n, n), B (b, n, m), Q (b, n, n), R (b, m, m)  ->  P (b, n, n), K (b, m, n) with u = -K x, info (b,)
+int32 (0 ok, otherwise the codes of include/lqrb200.h; a failed instance's P, K and gradients are NaN).  Batch
+broadcasting, the symmetrisation of Q and R, streams and the CPU rule are as for ``riccati_solve``; a loss on P alone or
+K alone skips the other's cotangent.  ``riccati_solve(A, B, Q, R, q, r, Qf=P, qf, x0, N=N)`` with the same A, B, Q, R
+composes with it into a finite-horizon MPC layer whose terminal cost is the infinite-horizon cost-to-go: its gains are
+then K at every knot, and gradients flow through P into the stage-cost and dynamics arguments.
 """
 from __future__ import annotations
 
@@ -37,7 +46,7 @@ from torch.autograd.function import once_differentiable
 
 from . import _lib, ops
 
-__all__ = ["riccati_solve", "kkt_solve"]
+__all__ = ["riccati_solve", "kkt_solve", "dare_solve"]
 
 
 def _cm(a):
@@ -219,3 +228,48 @@ def kkt_solve(Q, R, q, r, A, B, d, C, c, Hux=None, D2=None, hess_mode=_lib.HESS_
     body = dz[:, :(N - 1) * (n + m)].view(b, N - 1, n + m)
     X = torch.cat([body[:, :, :n], dz[:, None, (N - 1) * (n + m):]], dim=1)
     return X, body[:, :, n:].contiguous(), mult, info
+
+
+class _DareSolve(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, A, B, Q, R):
+        b, n, m = A.shape[0], A.shape[-1], B.shape[-1]
+        Ac, Bc, Rc = _cm(A), _cm(B), _cm(R)
+        P = torch.empty(b, n, n, dtype=torch.float64, device=A.device)  # symmetric: either order
+        K = torch.empty(b, n, m, dtype=torch.float64, device=A.device)  # column-major m x n
+        info = torch.empty(b, dtype=torch.int32, device=A.device)
+        with torch.cuda.device(A.device):
+            ops.dare(_handle(A.device), n, m, b, Ac, Bc, _cm(Q), Rc, P, K, None, info)
+        ctx.save_for_backward(Ac, Bc, Rc, P)
+        ctx.dims = (n, m, b)
+        ctx.mark_non_differentiable(info)
+        ctx.set_materialize_grads(False)  # a loss on P alone or K alone passes no cotangent for the other
+        return P, K.transpose(-1, -2), info
+
+    @staticmethod
+    @once_differentiable  # double backward is not provided: create_graph=True raises instead of returning constants
+    def backward(ctx, dP, dK, _dinfo):
+        A, B, R, P = ctx.saved_tensors
+        n, m, b = ctx.dims
+        if (dP is None and dK is None) or not any(ctx.needs_input_grad):
+            return (None,) * 4
+        like = (A, B, P, R)  # gA, gB, gQ, gR: column-major buffers of the inputs' shapes
+        g = [torch.empty_like(t) if w else None for t, w in zip(like, ctx.needs_input_grad)]
+        with torch.cuda.device(A.device):
+            ops.dare_grad(_handle(A.device), n, m, b, A, B, R, P, None if dP is None else _cm(dP),
+                          None if dK is None else _cm(dK), *g)
+        return tuple(None if x is None else x.transpose(-1, -2) for x in g)
+
+
+def dare_solve(A, B, Q, R):
+    """Differentiable batched DARE solve; see the module docstring."""
+    for t in (A, B, Q, R):
+        if not (t.is_cuda and t.dtype == torch.float64):
+            raise TypeError("dare_solve takes CUDA float64 tensors (there is no CPU path)")
+    b = max(t.shape[0] for t in (A, B, Q, R))
+
+    def full(t, sym=False):
+        if sym:
+            t = 0.5 * (t + t.transpose(-1, -2))
+        return t.expand((b,) + tuple(t.shape[1:]))
+    return _DareSolve.apply(full(A), full(B), full(Q, True), full(R, True))

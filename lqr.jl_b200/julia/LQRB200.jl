@@ -244,6 +244,43 @@ function riccati_grad_gains!(G::NamedTuple, prob::LQRProblem, Z::Union{Nothing,M
     return info
 end
 
+"""dare!(P, K, A, B, Q, R, handle): stabilising solution P (n×n×batch) and stationary gain K (m×n×batch, u = -K x) of
+the discrete algebraic Riccati equation of A (n×n×batch), B (n×m×batch), Q (n×n×batch), R (m×m×batch) by structured
+doubling.  P or K may be `nothing`, not both.  Returns (info, iters) per instance (include/lqrb200.h codes)."""
+function dare!(P::Union{Nothing,Array{Float64,3}}, K::Union{Nothing,Array{Float64,3}}, A::Array{Float64,3},
+               B::Array{Float64,3}, Q::Array{Float64,3}, R::Array{Float64,3}, handle::Handle)
+    n, m, batch = size(A, 1), size(B, 2), size(A, 3)
+    info = zeros(Int32, batch)
+    iters = zeros(Int32, batch)
+    g(x) = x === nothing ? C_NULL : pointer(x)
+    GC.@preserve P K A B Q R info iters begin
+        rc = ccall((:lqrb_dare_f64, lib), Int32,
+            (Ptr{Cvoid}, Int32, Int32, Int64, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+             Ptr{Float64}, Ptr{Int32}, Ptr{Int32}),
+            handle.ptr, n, m, batch, A, B, Q, R, g(P), g(K), iters, info)
+    end
+    check(handle, rc)
+    return info, iters
+end
+
+"""dare_grad!(G, A, B, R, P, dP, dK, handle): gradients of a loss l(P, K) through dare! from dP = dl/dP (n×n×batch)
+and dK = dl/dK (m×n×batch), either may be `nothing`, not both.  G is a NamedTuple (A, B, Q, R) of arrays shaped like
+the inputs (any may be `nothing`); returns the info per instance."""
+function dare_grad!(G::NamedTuple, A::Array{Float64,3}, B::Array{Float64,3}, R::Array{Float64,3}, P::Array{Float64,3},
+                    dP::Union{Nothing,Array{Float64,3}}, dK::Union{Nothing,Array{Float64,3}}, handle::Handle)
+    n, m, batch = size(A, 1), size(B, 2), size(A, 3)
+    info = zeros(Int32, batch)
+    g(x) = x === nothing ? C_NULL : pointer(x)
+    GC.@preserve G A B R P dP dK info begin
+        rc = ccall((:lqrb_dare_grad_f64, lib), Int32,
+            (Ptr{Cvoid}, Int32, Int32, Int64, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+             Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Int32}),
+            handle.ptr, n, m, batch, A, B, R, P, g(dP), g(dK), g(G.A), g(G.B), g(G.Q), g(G.R), info)
+    end
+    check(handle, rc)
+    return info
+end
+
 # ------------------------------------------------------------------ LeastSquaresSolver (src/least_squares.jl)
 "LeastSquaresSolver(prob): the condensed (block-Toeplitz) form of the unconstrained LTI problem, src/least_squares.jl:1-59"
 struct LeastSquaresSolver
@@ -713,7 +750,7 @@ kkt_unpack!(h::Handle, n, m, N, batch, p::Vector{Int32}, hess_mode, explicit_d2,
          Ptr{Float64}, Ptr{Float64}),
         h.ptr, n, m, N, batch, p, hess_mode, explicit_d2, dzp, multp, resp, dz, mult, res))
 
-export Handle, LQRBError, LQRProblem, LQRSolution, DPSolver, LeastSquaresSolver, solve!, rollout!, riccati_grad!, riccati_grad_gains!, kkt_grad!, num_vars,
+export Handle, LQRBError, LQRProblem, LQRSolution, DPSolver, LeastSquaresSolver, solve!, rollout!, riccati_grad!, riccati_grad_gains!, dare!, dare_grad!, kkt_grad!, num_vars,
        state, control,
        BlockCholesky, InvertedQuadratic, update_cost!, update_cholesky!, gradient,
        ConstraintBlock, ConstraintBlocks, dims, copy_blocks!, gen_con_inds,

@@ -315,6 +315,44 @@ def riccati_grad_gains_problem(prob: dict, Z, dZ, dK, dkff, handle: Handle | Non
     return g, info
 
 
+def dare(h: Handle, n, m, batch, A, B, Q, R, P=None, K=None, iters=None, info=None):
+    """lqrb_dare_f64: stabilising solution P [n,n,batch] and gain K [m,n,batch] of the discrete algebraic Riccati
+    equation; instance-major column-major buffers, host or device."""
+    h.call("lqrb_dare_f64", n, m, batch, ptr(A), ptr(B), ptr(Q), ptr(R), ptr(P), ptr(K), ptr(iters), ptr(info))
+
+
+def dare_grad(h: Handle, n, m, batch, A, B, R, P, dP, dK, gA=None, gB=None, gQ=None, gR=None, info=None):
+    """lqrb_dare_grad_f64: gradients of l(P, K) through lqrb_dare_f64 from dP = dl/dP, dK = dl/dK (either may be
+    None, not both); buffers as dare()."""
+    h.call("lqrb_dare_grad_f64", n, m, batch, ptr(A), ptr(B), ptr(R), ptr(P), ptr(dP), ptr(dK), ptr(gA), ptr(gB),
+           ptr(gQ), ptr(gR), ptr(info))
+
+
+def dare_problem(prob: dict, handle: Handle | None = None):
+    """Solve the DARE of the math-order arrays A (b,n,n), B (b,n,m), Q (b,n,n), R (b,m,m) of a problem dict (an LTI
+    Riccati problem dict serves) from host memory.  Returns P (b,n,n), K (b,m,n), iters (b,), info (b,)."""
+    h = handle or default_handle()
+    A, B = np.asarray(prob["A"]), np.asarray(prob["B"])
+    b, n, m = A.shape[0], A.shape[-1], B.shape[-1]
+    P, K = np.zeros((b, n, n)), np.zeros((b, n, m))  # column-major buffers
+    iters, info = np.zeros(b, dtype=np.int32), np.zeros(b, dtype=np.int32)
+    dare(h, n, m, b, cm(A), cm(B), cm(prob["Q"]), cm(prob["R"]), P, K, iters, info)
+    return np.swapaxes(P, -1, -2).copy(), np.swapaxes(K, -1, -2).copy(), iters, info
+
+
+def dare_grad_problem(prob: dict, P, dP=None, dK=None, handle: Handle | None = None):
+    """Gradients of l(P, K) through dare_problem, from host memory: P (b,n,n) as it returned, dP = dl/dP (b,n,n),
+    dK = dl/dK (b,m,n) in math order (either may be None, not both).  Returns (grads, info): grads holds math-order
+    arrays A, B, Q, R with the shapes of the problem's."""
+    h = handle or default_handle()
+    A, B = np.asarray(prob["A"]), np.asarray(prob["B"])
+    b, n, m = A.shape[0], A.shape[-1], B.shape[-1]
+    g = dict(A=np.zeros((b, n, n)), B=np.zeros((b, m, n)), Q=np.zeros((b, n, n)), R=np.zeros((b, m, m)))
+    info = np.zeros(b, dtype=np.int32)
+    dare_grad(h, n, m, b, cm(A), cm(B), cm(prob["R"]), cm(P), cm(dP), cm(dK), g["A"], g["B"], g["Q"], g["R"], info)
+    return {k: np.ascontiguousarray(np.swapaxes(v, -1, -2)) for k, v in g.items()}, info
+
+
 def split_primals(Z, n, m, N):
     """Primals layout [x1;u1;...;xN] (src/lqr_problem.jl:46-73) -> X (b,N,n), U (b,N-1,m) copies."""
     b = Z.shape[0]
