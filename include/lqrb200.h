@@ -243,6 +243,65 @@ int32_t lqrb_dare_grad_f64(lqrb_handle_t handle, int32_t n, int32_t m, int64_t b
                            const double *B, const double *R, const double *P, const double *dP, const double *dK,
                            double *gA, double *gB, double *gQ, double *gR, int32_t *info);
 
+/* ---------------------------------------------------------------- box-constrained MPC (ADMM) - */
+/* Box-constrained LTI MPC by ADMM on a cached infinite-horizon Riccati factor (the algorithm of TinyMPC, Nguyen et al.,
+ * ICRA 2024; DESIGN §4.12).  Per instance, with x_1 = x0:
+ *     min  sum_{k=1}^{N-1} 1/2 (x_k - xref_k)'Q(x_k - xref_k) + 1/2 (u_k - uref_k)'R(u_k - uref_k)
+ *          + 1/2 (x_N - xref_N)'Qf(x_N - xref_N)
+ *     s.t. x_{k+1} = A x_k + B u_k,  umin_k <= u_k <= umax_k (k = 1..N-1),  xmin_k <= x_k <= xmax_k (k = 2..N)
+ * THE TERMINAL COST DEPENDS ON rho: Qf = Pt - rho I with Pt = DARE(A, B, Q + rho I, R + rho I) (Pt >= Q + rho I, so
+ * Qf >= Q).  With that Qf the finite-horizon gains of the rho-augmented problem equal the stationary K at every knot,
+ * so one cached factor serves every iteration and every horizon.
+ * Iteration (scaled duals; z, y, v, g start at 0 on a cold start):
+ *   1. qt_k = -Q xref_k - rho (v_k - g_k), rt_k = -R uref_k - rho (z_k - y_k), p_N = -Qf xref_N - rho (v_N - g_N);
+ *   2. for k = N-1..1: d_k = C1 (B'p_{k+1} + rt_k), p_k = qt_k + C2 p_{k+1} - K'rt_k   (C1 = (R + rho I + B'Pt B)^-1,
+ *      C2 = (A - BK)');
+ *   3. u_k = -K x_k - d_k, x_{k+1} = A x_k + B u_k;
+ *   4. z = clamp(u + y, umin, umax), v = clamp(x + g, xmin, xmax);   5. y += u - z, g += x - v;
+ *   6. r_pri = max(|u - z|_inf, |x - v|_inf), r_dual = rho max(|z - z_prev|_inf, |v - v_prev|_inf);
+ *   7. stop when r_pri <= eps_pri and r_dual <= eps_dual, or after max_iter iterations.
+ * The returned trajectory is the last primal iterate (x, u): dynamically exact, within r_pri of the bounds.
+ *
+ * lqrb_admm_cache_f64: the cache of (A, B, Q, R, rho).
+ *   A[n,n,batch] B[n,m,batch] Q[n,n,batch] R[m,m,batch] (only the upper triangles of Q and R are read), rho > 0 finite
+ *   (one value for the batch), 1 <= n <= 32, 1 <= m <= n.
+ *   -> cache[L,batch], L = 4n^2 + 2nm + 2m^2 + 1 doubles per instance, column-major blocks in this order:
+ *      A (n x n) | B (n x m) | Q (n x n) | R (m x m) | Qf (n x n) | K (m x n) | C1 (m x m) | C2 (n x n) | rho,
+ *      Q and R symmetric (from their upper triangles), K the DARE gain of the rho-augmented costs (u = -K x);
+ *      info[batch] | NULL: the codes of lqrb_dare_f64 for (A, B, Q + rho I, R + rho I): 0, 1, 1000 + j, 2000 + j,
+ *      3000 + j.  A failed instance's record is NaN (a solve on it reports info 2); the others are not affected.
+ *   Error codes: -2 n, -3 m, -4 batch, -5 rho, -6..-9 A, B, Q, R NULL, -10 cache NULL.
+ *
+ * lqrb_admm_solve_f64: the ADMM iterations, each instance to its own stopping point.
+ *   flags: 0 or LQRB_FLAG_WARM_START (start from `state` instead of zeros).
+ *   opts: max_iter >= 1, eps_pri >= 0, eps_dual >= 0 (eps = 0: exactly max_iter iterations).
+ *   cache[L,batch] from lqrb_admm_cache_f64 with the same n, m; x0[n,batch];
+ *   xref[n,N,batch] | NULL (0), uref[m,N-1,batch] | NULL (0), umin, umax[m,N-1,batch] | NULL (-inf, +inf),
+ *   xmin, xmax[n,N-1,batch] | NULL (-inf, +inf; knots 2..N).  Infinite bound entries are legal; a NaN anywhere is not.
+ *   state[2(N-1)(m+n),batch] | NULL, in/out, per instance [z (m,N-1); y (m,N-1); v (n,N-1); g (n,N-1)] (v, g at knots
+ *   2..N): read only under LQRB_FLAG_WARM_START, written whenever given (the receding-horizon loop passes it back).
+ *   -> Z[N*n+(N-1)*m,batch] (Primals order, as lqrb_riccati_f64), iters[batch] | NULL (iterations run),
+ *      res[2,batch] | NULL (r_pri, r_dual of the last iteration), info[batch] | NULL:
+ *      0 converged; 1 max_iter reached (the last iterate is written); 2 a NaN in the instance's inputs (cache record,
+ *      x0, references, bounds, warm-start state) or in an iterate; 3 an empty box (min > max) somewhere.  Under 2 and
+ *      3 the instance's Z, state and res are NaN.  The other instances of the batch are not affected.
+ *   Each instance's working set (2n^2 + 2nm + m^2 + (N-1)(6n + 6m) doubles) stays in shared memory for all
+ *   iterations; a shape where it exceeds 227 KB is rejected with -4 (N too long for this n, m).
+ *   Error codes: -2 n, -3 m, -4 N < 2 or the working set above, -5 batch, -6 flags (or WARM_START without state),
+ *   -7 opts NULL or out of range, -8 cache NULL, -9 x0 NULL, -17 Z NULL.
+ * Both: host or device pointers, with the staged / device-resident rule of every entry point.  Not differentiable. */
+#define LQRB_FLAG_WARM_START 8
+typedef struct {
+    int32_t max_iter;
+    double eps_pri, eps_dual;
+} lqrb_admm_options_t;
+int32_t lqrb_admm_cache_f64(lqrb_handle_t handle, int32_t n, int32_t m, int64_t batch, double rho, const double *A,
+                            const double *B, const double *Q, const double *R, double *cache, int32_t *info);
+int32_t lqrb_admm_solve_f64(lqrb_handle_t handle, int32_t n, int32_t m, int32_t N, int64_t batch, int32_t flags,
+                            const lqrb_admm_options_t *opts, const double *cache, const double *x0, const double *xref,
+                            const double *uref, const double *umin, const double *umax, const double *xmin,
+                            const double *xmax, double *state, double *Z, int32_t *iters, double *res, int32_t *info);
+
 /* ---------------------------------------------------------------- BlockCholesky ------------- */
 /* Replaces cholesky!(chol, A, B[, C]) : src/block_cholesky.jl:55-91.  Instance-major:
  *   A[n,n,batch] B[m,m,batch] C[m,n,batch] (C NULL unless DENSE) -> M[(n+m),(n+m),batch]

@@ -17,7 +17,7 @@ CSRC = os.path.join(_HERE, "csrc")
 HEADER = os.path.join(os.path.dirname(_HERE), "include", "lqrb200.h")
 
 HESS_DENSE, HESS_BLOCKDIAG, HESS_DIAG = 0, 1, 2
-FLAG_SOC, FLAG_LTI, FLAG_NO_AFFINE = 1, 2, 4
+FLAG_SOC, FLAG_LTI, FLAG_NO_AFFINE, FLAG_WARM_START = 1, 2, 4, 8
 TILE = 32
 
 _lib = None
@@ -38,6 +38,10 @@ class SqpOptions(C.Structure):
     _fields_ = [("N", c_i32), ("iters", c_i32), ("dt", C.c_double), ("q_diag", C.c_double),
                 ("r_diag", C.c_double), ("qf_diag", C.c_double), ("eps_p", C.c_double),
                 ("eps_d", C.c_double), ("line_search", c_i32)]
+
+
+class AdmmOptions(C.Structure):
+    _fields_ = [("max_iter", c_i32), ("eps_pri", C.c_double), ("eps_dual", C.c_double)]
 
 
 def build(force: bool = False, jobs: int = 8) -> str:
@@ -81,6 +85,9 @@ _SIGS = {
     "lqrb_rollout_f64": (c_i32, [c_vp, c_i32, c_i32, c_i32, c_i64, c_i32] + [c_dp] * 5),
     "lqrb_dare_f64": (c_i32, [c_vp, c_i32, c_i32, c_i64] + [c_dp] * 6 + [c_vp, c_vp]),
     "lqrb_dare_grad_f64": (c_i32, [c_vp, c_i32, c_i32, c_i64] + [c_dp] * 10 + [c_vp]),
+    "lqrb_admm_cache_f64": (c_i32, [c_vp, c_i32, c_i32, c_i64, C.c_double] + [c_dp] * 5 + [c_vp]),
+    "lqrb_admm_solve_f64": (c_i32, [c_vp, c_i32, c_i32, c_i32, c_i64, c_i32, C.POINTER(AdmmOptions)] + [c_dp] * 10
+                            + [c_vp, c_dp, c_vp]),
     "lqrb_lsq_solve_f64": (c_i32, [c_vp, c_i32, c_i32, c_i32, c_i64] + [c_dp] * 7 + [c_vp]),
     "lqrb_block_cholesky_f64": (c_i32, [c_vp, c_i32, c_i32, c_i64, c_i32] + [c_dp] * 4 + [c_vp]),
     "lqrb_block_ldiv_f64": (c_i32, [c_vp, c_i32, c_i32, c_i64, c_i32, c_dp, c_i32, c_dp]),

@@ -60,6 +60,7 @@ enum ScratchSlot {
                       // gradient kernels)
     SCR_ADJOINT_MULT, // lqrb_kkt_grad_f64: the adjoint multipliers, instance-major
     SCR_GAIN_TAPE,    // lqrb_riccati_grad_gains_f64: P_{k+1}, p_{k+1}, K_k, kff_k and the factor of G_k per knot
+    SCR_ADMM_CACHE,   // lqrb_admm_cache_f64: Q + rho I, R + rho I, and the DARE's P, K, info of a chunk
     SCR_COUNT
 };
 

@@ -1,7 +1,9 @@
-// dare.cu — host side of the batched discrete algebraic Riccati equation and its gradient (DESIGN §4.11).
+// dare.cu — host side of the batched discrete algebraic Riccati equation and its gradient (DESIGN §4.11), and of the
+// ADMM cache built on it (DESIGN §4.12).
+#include <cmath>
 #include <cstdio>
 
-#include "dare_kernels.cuh"
+#include "admm_kernels.cuh"
 
 namespace {
 // Launch shape of both kernels, as launch_coop (riccati.cu): a warp per instance, four instances per 128-thread
@@ -85,5 +87,51 @@ extern "C" int32_t lqrb_dare_grad_f64(lqrb_handle_t h, int32_t n, int32_t m, int
             return dare_launch(h, "dare_grad", dare_grad_kernel<32, 128>, dare_grad_kernel<256, 256>, per, n, cb,
                                lane.stream, a[0], a[1], a[2], a[3], a[4], a[5], g[0], g[1], g[2], g[3],
                                (int32_t *)out[4], n, m, cb);
+        });
+}
+
+extern "C" int32_t lqrb_admm_cache_f64(lqrb_handle_t h, int32_t n, int32_t m, int64_t batch, double rho,
+                                       const double *A, const double *B, const double *Q, const double *R,
+                                       double *cache, int32_t *info) {
+    if (!h) return -1;
+    if (n < 1 || n > 32) return lqrb_fail(h, -2, "n out of range [1,32]");
+    if (m < 1 || m > n) return lqrb_fail(h, -3, "m out of range [1,n]");
+    if (batch < 0) return lqrb_fail(h, -4, "batch must be >= 0");
+    if (!(rho > 0.0) || !std::isfinite(rho)) return lqrb_fail(h, -5, "rho must be finite and > 0");
+    if (!A) return lqrb_fail(h, -6, "A is NULL");
+    if (!B) return lqrb_fail(h, -7, "B is NULL");
+    if (!Q) return lqrb_fail(h, -8, "Q is NULL");
+    if (!R) return lqrb_fail(h, -9, "R is NULL");
+    if (!cache) return lqrb_fail(h, -10, "cache is NULL");
+    if (batch == 0) return 0;
+    LQRB_CUDA(h, cudaSetDevice(h->device));
+    const int64_t sA = (int64_t)n * n * 8, sB = (int64_t)n * m * 8, sR = (int64_t)m * m * 8;
+    const size_t per = dare_smem_doubles(n) * sizeof(double);
+    const size_t cache_smem = 4 * ((size_t)n * n + 2 * n * m + 2 * m * m) * sizeof(double);
+    return lqrb_for_chunks(
+        h, batch, 0, {{A, sA}, {B, sB}, {Q, sA}, {R, sR}}, {{cache, admm_cache_doubles(n, m) * 8}, {info, 4}},
+        [&](Lane lane, int64_t cb, const void *const *in, void *const *out) -> int32_t {
+            const double *const *a = (const double *const *)in;
+            // scratch: Q + rho I | R + rho I | P | K | DARE info
+            const size_t nd = (size_t)cb * (2 * n * n + m * m + n * m);
+            double *Qt = (double *)lqrb_scratch(h, SCR_ADMM_CACHE, nd * 8 + (size_t)cb * 4, lane.index);
+            if (!Qt) return 1000 + (int)cudaErrorMemoryAllocation;
+            double *Rt = Qt + cb * n * n, *P = Rt + cb * m * m, *K = P + cb * n * n;
+            int32_t *dinfo = (int32_t *)(K + cb * n * m);
+            const int64_t total = cb * (n * n + m * m);
+            admm_shift_kernel<<<(unsigned)std::min<int64_t>((total + 255) / 256, 4096), 256, 0, lane.stream>>>(
+                a[2], a[3], rho, Qt, Rt, n, m, cb);
+            LQRB_LAUNCH_CHECK(h, "admm_shift_kernel");
+            int32_t rc = dare_launch(h, "dare", dare_kernel<32, 128>, dare_kernel<256, 256>, per, n, cb, lane.stream,
+                                     a[0], a[1], (const double *)Qt, (const double *)Rt, P, K, (int32_t *)nullptr,
+                                     dinfo, n, m, cb);
+            if (rc) return rc;
+            LQRB_CUDA(h, cudaFuncSetAttribute(admm_cache_kernel<32, 128>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                              (int)cache_smem));
+            admm_cache_kernel<32, 128><<<(unsigned)((cb + 3) / 4), 128, cache_smem, lane.stream>>>(
+                a[0], a[1], a[2], a[3], Rt, P, K, dinfo, rho, (double *)out[0], (int32_t *)out[1], n, m, cb);
+            h->kernel_name = "admm_cache";
+            LQRB_LAUNCH_CHECK(h, "admm_cache_kernel");
+            return 0;
         });
 }

@@ -37,7 +37,7 @@ using LinearAlgebra
 const lib = get(ENV, "LQRB200_LIB", joinpath(@__DIR__, "..", "liblqrb200.so"))
 
 const HESS_DENSE, HESS_BLOCKDIAG, HESS_DIAG = Int32(0), Int32(1), Int32(2)
-const FLAG_SOC, FLAG_LTI, FLAG_NO_AFFINE = Int32(1), Int32(2), Int32(4)
+const FLAG_SOC, FLAG_LTI, FLAG_NO_AFFINE, FLAG_WARM_START = Int32(1), Int32(2), Int32(4), Int32(8)
 const DevPtr = Ptr{Float64}   # a device address (e.g. `pointer(::CuArray{Float64})` reinterpreted by the caller)
 
 struct LQRBError <: Exception
@@ -279,6 +279,58 @@ function dare_grad!(G::NamedTuple, A::Array{Float64,3}, B::Array{Float64,3}, R::
     end
     check(handle, rc)
     return info
+end
+
+"""admm_cache!(cache, A, B, Q, R, rho, handle): the cache of box-constrained MPC by ADMM (lqrb_admm_cache_f64) for
+A (n×n×batch), B (n×m×batch), Q (n×n×batch), R (m×m×batch) and rho > 0: cache is (4n²+2nm+2m²+1)×batch, per instance
+[A | B | Q | R | Qf | K | C1 | C2 | rho] with the terminal cost Qf = P̃ - rho I of the solve.  Returns the info per
+instance (the DARE's codes)."""
+function admm_cache!(cache::Matrix{Float64}, A::Array{Float64,3}, B::Array{Float64,3}, Q::Array{Float64,3},
+                     R::Array{Float64,3}, rho::Float64, handle::Handle)
+    n, m, batch = size(A, 1), size(B, 2), size(A, 3)
+    info = zeros(Int32, batch)
+    GC.@preserve cache A B Q R info begin
+        rc = ccall((:lqrb_admm_cache_f64, lib), Int32,
+            (Ptr{Cvoid}, Int32, Int32, Int64, Float64, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+             Ptr{Float64}, Ptr{Int32}),
+            handle.ptr, n, m, batch, rho, A, B, Q, R, cache, info)
+    end
+    check(handle, rc)
+    return info
+end
+
+"lqrb_admm_options_t"
+struct AdmmOptions
+    max_iter::Int32
+    eps_pri::Float64
+    eps_dual::Float64
+end
+
+"""admm_solve!(Z, cache, x0, bounds, handle; N, xref, uref, state, warm, max_iter, eps): box-constrained MPC by ADMM
+(lqrb_admm_solve_f64) on a cache from admm_cache!.  Z is (N n + (N-1) m)×batch in Primals order; bounds is a NamedTuple
+(umin, umax, xmin, xmax) of m×(N-1)×batch / n×(N-1)×batch arrays or `nothing` (±Inf); xref (n×N×batch), uref
+(m×(N-1)×batch) may be `nothing` (0); state (2(N-1)(m+n)×batch) is read when warm and written when given.  Returns
+(info, iters, res) per instance."""
+function admm_solve!(Z::Matrix{Float64}, cache::Matrix{Float64}, x0::Matrix{Float64}, bounds::NamedTuple,
+                     handle::Handle; N::Integer, m::Integer, xref=nothing, uref=nothing,
+                     state::Union{Nothing,Matrix{Float64}}=nothing, warm::Bool=false, max_iter::Integer=100,
+                     eps::Float64=1e-6)
+    n, batch = size(x0, 1), size(x0, 2)
+    info = zeros(Int32, batch)
+    iters = zeros(Int32, batch)
+    res = zeros(Float64, 2, batch)
+    opts = Ref(AdmmOptions(Int32(max_iter), eps, eps))
+    g(x) = x === nothing ? C_NULL : pointer(x)
+    GC.@preserve Z cache x0 bounds xref uref state info iters res opts begin
+        rc = ccall((:lqrb_admm_solve_f64, lib), Int32,
+            (Ptr{Cvoid}, Int32, Int32, Int32, Int64, Int32, Ref{AdmmOptions}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+             Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+             Ptr{Int32}, Ptr{Float64}, Ptr{Int32}),
+            handle.ptr, n, m, N, batch, warm ? FLAG_WARM_START : Int32(0), opts, cache, x0, g(xref), g(uref),
+            g(bounds.umin), g(bounds.umax), g(bounds.xmin), g(bounds.xmax), g(state), Z, iters, res, info)
+    end
+    check(handle, rc)
+    return info, iters, res
 end
 
 # ------------------------------------------------------------------ LeastSquaresSolver (src/least_squares.jl)
@@ -750,7 +802,7 @@ kkt_unpack!(h::Handle, n, m, N, batch, p::Vector{Int32}, hess_mode, explicit_d2,
          Ptr{Float64}, Ptr{Float64}),
         h.ptr, n, m, N, batch, p, hess_mode, explicit_d2, dzp, multp, resp, dz, mult, res))
 
-export Handle, LQRBError, LQRProblem, LQRSolution, DPSolver, LeastSquaresSolver, solve!, rollout!, riccati_grad!, riccati_grad_gains!, dare!, dare_grad!, kkt_grad!, num_vars,
+export Handle, LQRBError, LQRProblem, LQRSolution, DPSolver, LeastSquaresSolver, solve!, rollout!, riccati_grad!, riccati_grad_gains!, dare!, dare_grad!, admm_cache!, admm_solve!, kkt_grad!, num_vars,
        state, control,
        BlockCholesky, InvertedQuadratic, update_cost!, update_cholesky!, gradient,
        ConstraintBlock, ConstraintBlocks, dims, copy_blocks!, gen_con_inds,

@@ -3,6 +3,8 @@ memory, torch CUDA tensors for device memory) already in the ABI's layouts and f
 No arithmetic happens here."""
 from __future__ import annotations
 
+import math
+
 import numpy as np
 
 from . import _lib
@@ -351,6 +353,68 @@ def dare_grad_problem(prob: dict, P, dP=None, dK=None, handle: Handle | None = N
     info = np.zeros(b, dtype=np.int32)
     dare_grad(h, n, m, b, cm(A), cm(B), cm(prob["R"]), cm(P), cm(dP), cm(dK), g["A"], g["B"], g["Q"], g["R"], info)
     return {k: np.ascontiguousarray(np.swapaxes(v, -1, -2)) for k, v in g.items()}, info
+
+
+def admm_cache_doubles(n, m) -> int:
+    """doubles per instance of the lqrb_admm_cache_f64 record [A | B | Q | R | Qf | K | C1 | C2 | rho]"""
+    return 4 * n * n + 2 * n * m + 2 * m * m + 1
+
+
+def admm_cache_split(cache, n, m) -> dict:
+    """(b, L) cache records -> dict of math-order views A, B, Q, R, Qf, K, C1, C2 (b, rows, cols) and rho (b,)"""
+    out, o = {}, 0
+    for k, (r, c) in zip(("A", "B", "Q", "R", "Qf", "K", "C1", "C2"),
+                         ((n, n), (n, m), (n, n), (m, m), (n, n), (m, n), (m, m), (n, n))):
+        out[k] = cache[:, o:o + r * c].reshape(-1, c, r).swapaxes(-1, -2)
+        o += r * c
+    out["rho"] = cache[:, o]
+    return out
+
+
+def admm_cache(h: Handle, n, m, batch, rho, A, B, Q, R, cache, info=None):
+    """lqrb_admm_cache_f64: the ADMM cache of (A, B, Q, R, rho); instance-major column-major buffers, host or device."""
+    h.call("lqrb_admm_cache_f64", n, m, batch, float(rho), ptr(A), ptr(B), ptr(Q), ptr(R), ptr(cache), ptr(info))
+
+
+def admm_solve(h: Handle, n, m, N, batch, cache, x0, Z, xref=None, uref=None, umin=None, umax=None, xmin=None,
+               xmax=None, state=None, warm=False, max_iter=100, eps_pri=1e-6, eps_dual=1e-6, iters=None, res=None,
+               info=None):
+    """lqrb_admm_solve_f64: box-constrained MPC by ADMM on a cache from admm_cache(); buffers as in the header
+    (instance-major column-major, host or device); `state` is updated in place, read when `warm`."""
+    o = _lib.AdmmOptions(max_iter=int(max_iter), eps_pri=float(eps_pri), eps_dual=float(eps_dual))
+    import ctypes as C
+    h.call("lqrb_admm_solve_f64", n, m, N, batch, _lib.FLAG_WARM_START if warm else 0, C.byref(o), ptr(cache), ptr(x0),
+           ptr(xref), ptr(uref), ptr(umin), ptr(umax), ptr(xmin), ptr(xmax), ptr(state), ptr(Z), ptr(iters), ptr(res),
+           ptr(info))
+
+
+def admm_cache_problem(prob: dict, rho, handle: Handle | None = None):
+    """The ADMM cache of the math-order arrays A (b,n,n), B (b,n,m), Q (b,n,n), R (b,m,m) of a problem dict (an LTI
+    Riccati problem dict serves), from host memory.  Returns (cache (b, L), info (b,)); admm_cache_split() reads it."""
+    h = handle or default_handle()
+    A, B = np.asarray(prob["A"]), np.asarray(prob["B"])
+    b, n, m = A.shape[0], A.shape[-1], B.shape[-1]
+    cache = np.zeros((b, admm_cache_doubles(n, m)))
+    info = np.zeros(b, dtype=np.int32)
+    admm_cache(h, n, m, b, rho, cm(A), cm(B), cm(prob["Q"]), cm(prob["R"]), cache, info)
+    return cache, info
+
+
+def admm_solve_problem(cache, x0, N, xref=None, uref=None, umin=None, umax=None, xmin=None, xmax=None, state=None,
+                       warm=False, max_iter=100, eps_pri=1e-6, eps_dual=1e-6, handle: Handle | None = None):
+    """lqrb_admm_solve_f64 from host memory on math-order arrays: cache (b, L), x0 (b,n), xref (b,N,n), uref (b,N-1,m),
+    umin / umax (b,N-1,m), xmin / xmax (b,N-1,n), each optional; state (b, 2(N-1)(m+n)) is updated in place when given.
+    Returns X (b,N,n), U (b,N-1,m), iters (b,), res (b,2), info (b,)."""
+    h = handle or default_handle()
+    x0 = f64(x0)
+    b, n = x0.shape
+    m = (math.isqrt(n * n + 2 * (cache.shape[1] - 1 - 4 * n * n)) - n) // 2  # the root of 2m^2 + 2nm = L - 1 - 4n^2
+    Z = np.zeros((b, _lib.num_vars(n, m, N)))
+    iters, res, info = np.zeros(b, dtype=np.int32), np.zeros((b, 2)), np.zeros(b, dtype=np.int32)
+    admm_solve(h, n, m, N, b, f64(cache), x0, Z, f64(xref), f64(uref), f64(umin), f64(umax), f64(xmin), f64(xmax),
+               state, warm, max_iter, eps_pri, eps_dual, iters, res, info)
+    X, U = split_primals(Z, n, m, N)
+    return X, U, iters, res, info
 
 
 def split_primals(Z, n, m, N):
